@@ -26,6 +26,9 @@ and cfg5 at the same N, so that one driver invocation per N times every BASELINE
                installed in this image (Python 3.12, no network; SURVEY.md section 0). The stand-in is the torch-CPU
                (oneDNN/MKL) restatement of the same training step (oracle/unet_torch.py) on cfg1 = batch 8 of 256x256x3
                fp32, all host cores, thread count printed; the numpy/BLAS port is kept as a second key.
+ * `--dump-outputs DIR` (rank 0): after the K timed steps, what the last of them left for its caller, as .npy files
+               (see dump_outputs). Inputs and initial weights are seeded, so two builds of the project run with the
+               same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -371,6 +374,30 @@ class Harness:
         return ok[0] > 0.5
 
 
+DUMP_SAMPLE = 1 << 21   # values kept of a larger output: five files of at most 8 MB each stay under 64 MB
+
+
+def dump_outputs(eng, out_dir: str):
+    """Writes what the training step just run computed, as a caller reads it back: loss.npy (float64 [data loss, L2
+    loss]), logits.npy, grads.npy (flat trainable-gradient arena), weights.npy (flat fp32 weight arena after the
+    optimizer update) and, for batch norm, moving_stats.npy, all float32. An output of more than DUMP_SAMPLE values is
+    reduced to DUMP_SAMPLE of them at sorted positions drawn with a fixed seed from its length alone, so the same
+    positions are kept on every run (and grads / weights keep the same parameters)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    data, reg = eng.read_loss()
+    outputs = {"loss": np.array([data, reg], np.float64),
+               "logits": eng.logits.download(np.float32, (eng.logits.nbytes // 4,)),
+               "grads": eng.G.download(np.float32, (eng.n_train,)),
+               "weights": eng.W.download(np.float32, (eng.n_train,))}
+    if getattr(eng, "n_stats", 0) > 0:
+        outputs["moving_stats"] = eng.S.download(np.float32, (eng.n_stats,))
+    for name, a in outputs.items():
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def dp_check(h: Harness, eng, lr):
     """Correctness of the data-parallel step, carried in the bench line (N > 1).
     (1) every rank's fp32 weight arena has the same CRC-32C after the timed steps;
@@ -423,6 +450,8 @@ def run_b200(args):
     sampler = ClockSampler(h.local) if rank == 0 else None   # started before warm-up: nvidia-smi takes ~1 s to spin up
     eng, units, lr = h.engine(name, batch)
     ms, n_launch = h.time_steps(eng, lr, args.steps, warmup)
+    if args.dump_outputs and rank == 0:     # before the untimed steps below move the weights on
+        dump_outputs(eng, args.dump_outputs)
 
     # ---- roofline side measurement (2-D engines): the same K steps again with every tensor-core launch bracketed by
     # CUDA events on its stream and the filter-gradient side stream folded back into the compute stream, so that each
@@ -559,7 +588,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-other-configs", dest="no_other_configs", action="store_true")
     ap.add_argument("--no-numpy-port", dest="no_numpy_port", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)
