@@ -47,11 +47,6 @@ class NormDesc(C.Structure):
     ]
 
 
-class Pipe(C.Structure):
-    """bsl_pipe: image-slice flags between an HBM-bound pass and the tensor-core kernel that reads its output."""
-    _fields_ = [("flags", C.c_void_p), ("counters", C.c_void_p), ("slices", C.c_int), ("epoch", C.c_int)]
-
-
 class InputDesc(C.Structure):
     _fields_ = [("n", C.c_int), ("channels", C.c_int), ("src_h", C.c_int), ("src_w", C.c_int), ("out_h", C.c_int),
                 ("out_w", C.c_int), ("max_centers", C.c_int), ("noise_scale", C.c_float), ("min_std", C.c_float),

@@ -57,7 +57,7 @@ __device__ __forceinline__ float guide_at(int yy, int xx, const float* ctr, cons
 __global__ void input_stage_kernel(bsl_input_desc d, bsl_input_params p, const unsigned short* __restrict__ slices,
                                    const unsigned char* __restrict__ seg, float* __restrict__ images,
                                    int* __restrict__ labels, float* __restrict__ sp_guide) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long per = (long long)d.out_h * d.out_w;
   if (t >= per * d.n) return;

@@ -168,7 +168,7 @@ SplitPlan plan_split(bsl_ctx* ctx, int mn_tiles, int k_tiles) {
 
 __global__ void reduce_splits_kernel(const float* __restrict__ part, float* __restrict__ out, long long n,
                                      int splits) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * 4;
   if (i >= n) return;
   float4 acc = *reinterpret_cast<const float4*>(part + i);
@@ -181,7 +181,7 @@ __global__ void reduce_splits_kernel(const float* __restrict__ part, float* __re
 
 __global__ void reduce_splits_strided_kernel(const float* __restrict__ part, float* __restrict__ out, long long n,
                                              int splits, long long stride) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * 4;
   if (i >= n) return;
   float4 acc = *reinterpret_cast<const float4*>(part + i);
@@ -211,14 +211,6 @@ int reduce_splits(bsl_ctx* ctx, const float* part, float* out, long long n, int 
 
 
 // ------------------------------------------------------------------ second-generation (halo-tile) kernels
-// BSL_IGEMM_V1=1 forces the first-generation kernels everywhere (A/B timing, bisecting).
-bool force_v1() {
-  static const int v = [] {
-    const char* e = getenv("BSL_IGEMM_V1");
-    return e ? atoi(e) : 0;
-  }();
-  return v != 0;
-}
 
 template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool TMA_ST = false>
 int launch_halo_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, int grid,
@@ -258,8 +250,7 @@ int launch_halo_res_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b
 // activation stages. May lower nsub to 1 (the filter is no longer re-read per unit, so sharing it matters less).
 constexpr int CH_DYN_BUDGET = 232448 - 10 * 1024;   // 227 KB minus static shared memory (barriers, statistics)
 bool plan_resident(int bn, int ntaps, int cblocks, int* nsub, int* a_stages, int* smem) {
-  static const int off = getenv("BSL_B_RES") ? atoi(getenv("BSL_B_RES")) == 0 : 0;
-  if (off || bn > 128) return false;
+  if (bn > 128) return false;
   const int res = ntaps * cblocks * bn * 128;
   const int left = CH_DYN_BUDGET - 1024 - res;
   if (left <= 0) return false;
@@ -294,10 +285,6 @@ void replan_units(bsl_ctx* ctx, HaloPlan& p) {
   p.slots = cdiv(p.grid, p.n_ntiles);
 }
 
-bool pair_on() {
-  static const int on = getenv("BSL_PAIR") ? atoi(getenv("BSL_PAIR")) != 0 : 1;
-  return on;
-}
 // How many CTA pairs of the (one-CTA-per-SM) pair kernels the device holds AT ONCE. The kernels are persistent with a
 // static schedule, so a pair that had to wait for a second round would double the launch's time: a GPC with an odd number
 // of usable SMs hosts one pair fewer than sm_count / 2 suggests. Asked from the driver once (the widest configuration).
@@ -324,9 +311,7 @@ int max_pairs(bsl_ctx* ctx) {
     if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) n = 0;
   }
   (void)cudaGetLastError();
-  static const int env = getenv("BSL_MAX_PAIRS") ? atoi(getenv("BSL_MAX_PAIRS")) : 0;
   cached = std::max(0, std::min(n, ctx->sm_count / 2));
-  if (env > 0) cached = std::min(cached, env);
   return cached;
 }
 // CTA pairs run 128-wide tiles: per CTA a pair takes in half of every filter slice, so the narrower tile costs no more
@@ -335,8 +320,7 @@ int max_pairs(bsl_ctx* ctx) {
 // double-buffered. Measured on the wide cfg2 layers: -10 % against single CTAs with 256-wide tiles
 // (profiles/r02_ab_experiments.md). min_cols: fprop keeps its fused statistics for 128-column layers.
 bool pair_replan(bsl_ctx* ctx, HaloPlan& p, int ncols, int min_cols, int ntaps) {
-  static const int env_bn = getenv("BSL_HALO_BN") ? atoi(getenv("BSL_HALO_BN")) : 0;
-  if (!pair_on() || env_bn || ntaps != 9 || ncols % 128 || ncols < min_cols || p.n_sub_total % 4) return false;
+  if (ntaps != 9 || ncols % 128 || ncols < min_cols || p.n_sub_total % 4) return false;
   if (max_pairs(ctx) < 1) return false;
   p.bn = 128;
   p.nsub = 2;
@@ -344,12 +328,6 @@ bool pair_replan(bsl_ctx* ctx, HaloPlan& p, int ncols, int min_cols, int ntaps) 
   replan_units(ctx, p);
   p.pair = 1;
   return true;
-}
-
-// Which column-tile widths use the TMA-store epilogue (BSL_TMA_STORE: 0 none, 1 = 256-wide tiles, 2 = also 128).
-int tma_store_level() {
-  static const int v = getenv("BSL_TMA_STORE") ? atoi(getenv("BSL_TMA_STORE")) : 1;
-  return v;
 }
 
 // Output tensor map of the TMA-store epilogue: (c, x, y, image) with a 64-channel x 8 x 16 pixel box.
@@ -368,8 +346,8 @@ int out_map(bsl_ctx* ctx, const ConvHaloArgs& a, int w, int h, CUtensorMap* out)
 // works on two units of two sub-tiles and the same column tile). `b_half`: for a K-major filter (dgrad) the tensor map
 // whose box holds HALF the tile's rows; an MN-major filter (fprop) is loaded in 64-column blocks either way.
 bool pair_eligible(bsl_ctx* ctx, const ConvHaloArgs& a, int bn, int nsub) {
-  return pair_on() && max_pairs(ctx) >= 1 && (bn == 256 || bn == 128) && nsub == 2 && a.n_sub_total % 4 == 0 && a.ntaps == 9 && a.halo == 1 && !a.tap_table &&
-         a.wait_flags == nullptr && a.up_cpb == 0 && a.relu_mask == nullptr;
+  return max_pairs(ctx) >= 1 && (bn == 256 || bn == 128) && nsub == 2 && a.n_sub_total % 4 == 0 && a.ntaps == 9 && a.halo == 1 &&
+         !a.tap_table && a.up_cpb == 0;
 }
 template <int BN, bool B_MN>
 int launch_halo_pair(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, cudaStream_t stream,
@@ -393,16 +371,11 @@ int launch_halo_pair(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, c
 // which also frees room for activation stages. dgrad reads the HWIO filter K-major as it is; fprop gets a K-major copy
 // ([tap][cout][cin], a few hundred KB at most) written into the per-stream filter scratch right before the launch --
 // an MN-major filter would have to be split into 32-column halves, which the 128-byte swizzle cannot express.
-bool pair_res_on() {
-  static const int on = getenv("BSL_PAIR_RES") ? atoi(getenv("BSL_PAIR_RES")) != 0 : 1;
-  return pair_on() && on;
-}
 bool plan_resident_pair(bsl_ctx* ctx, int bn, int ntaps, int cblocks, int n_sub_total, int* nsub, int* a_stages, int* smem) {
   // one-block reductions (K = 64) stay with single CTAs: their units are so short that the epilogue, not the tensor pipe,
   // sets the pace once the MMAs get faster (measured: 64 -> 64 fprop 0.298 -> 0.314 ms, dgrad unchanged), while
   // 128 -> 64 fprop gained 19 % and 128 -> 64 dgrad 25 % (profiles/r02_ab_experiments.md)
-  static const int min_cb = getenv("BSL_PAIR_RES_MIN_CB") ? atoi(getenv("BSL_PAIR_RES_MIN_CB")) : 2;
-  if (!pair_res_on() || (bn != 64 && bn != 128) || ntaps != 9 || cblocks < min_cb || max_pairs(ctx) < 1) return false;
+  if ((bn != 64 && bn != 128) || ntaps != 9 || cblocks < 2 || max_pairs(ctx) < 1) return false;
   const int res = ntaps * cblocks * (bn / 2) * 128;
   const int left = CH_DYN_BUDGET - 1024 - res;
   if (left <= 0) return false;
@@ -451,7 +424,7 @@ int launch_halo_res_pair(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, c
 // HWIO [taps][cin][cout] -> [taps][cout][cin] (bf16), the K-major filter of the forward pass of a CTA pair.
 __global__ void filter_kmajor_kernel(const __nv_bfloat16* __restrict__ w, __nv_bfloat16* __restrict__ o, int cin, int cout,
                                      int total) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;   // output index: (tap, co, ci)
   if (i >= total) return;
   const int ci = i % cin, t = i / cin;
@@ -463,20 +436,17 @@ template <bool B_MN, bool STATS, bool SCATTER>
 int launch_halo(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args,
                 int grid, cudaStream_t stream, const CUtensorMap* b_half = nullptr) {
   if constexpr (!STATS && !SCATTER) {
-    const int lvl = tma_store_level();
     if (pair_eligible(ctx, args, bn, nsub) && (B_MN || b_half != nullptr)) {
       CUtensorMap o;
       if (out_map(ctx, args, args.vw, args.vh, &o) == 0)
         return bn == 256 ? launch_halo_pair<256, B_MN>(ctx, a, B_MN ? b : *b_half, args, stream, o)
                          : launch_halo_pair<128, B_MN>(ctx, a, B_MN ? b : *b_half, args, stream, o);
     }
-    if (args.relu_mask == nullptr && ((bn == 256 && lvl >= 1) || (bn == 128 && lvl >= 2))) {
+    if (bn == 256) {   // TMA-store epilogue of the 256-wide tiles (DESIGN.md 3.6)
       CUtensorMap o;
       if (out_map(ctx, args, args.vw, args.vh, &o) == 0) {
-        if (bn == 256 && nsub == 2) return launch_halo_one<256, 2, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
-        if (bn == 256 && nsub == 1) return launch_halo_one<256, 1, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
-        if (bn == 128 && nsub == 2) return launch_halo_one<128, 2, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
-        if (bn == 128 && nsub == 1) return launch_halo_one<128, 1, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
+        if (nsub == 2) return launch_halo_one<256, 2, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
+        if (nsub == 1) return launch_halo_one<256, 1, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
       }
     }
   }
@@ -495,27 +465,19 @@ int launch_halo(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, const CUte
 // Ragged extents: a grid that the tile does not divide runs with ceil(extent / tile) tiles -- TMA zero-fills the reads
 // past the edge (SAME padding already relies on it), the epilogue masks the stores and the statistics of pixels outside
 // the image (ConvHaloArgs::vw / vh), the filter-gradient kernels need nothing (zero dy rows contribute zero). Taken when
-// the padded grid holds at most 2x the pixels; BSL_HALO_RAGGED=0 restores the exact-multiple rule.
-bool ragged_on() {
-  static const bool on = !(getenv("BSL_HALO_RAGGED") && atoi(getenv("BSL_HALO_RAGGED")) == 0);
-  return on;
-}
+// the padded grid holds at most 2x the pixels.
 bool tiles_ok(int w, int h, int tw, int th) {
   if (w % tw == 0 && h % th == 0) return true;
-  if (!ragged_on() || w < 1 || h < 1) return false;
+  if (w < 1 || h < 1) return false;
   return (long long)cdiv(w, tw) * tw * cdiv(h, th) * th <= 2LL * w * h;
 }
-bool halo_eligible(int w, int h) { return !force_v1() && tiles_ok(w, h, 8, 16); }
+bool halo_eligible(int w, int h) { return tiles_ok(w, h, 8, 16); }
 
 HaloPlan plan_halo(bsl_ctx* ctx, int w, int h, int n, int ncols) {
   HaloPlan p = {};
   p.n_sub_total = cdiv(w, 8) * cdiv(h, 16) * n;
   p.bn = ncols % 256 == 0 ? 256 : (ncols % 128 == 0 ? 128 : 64);
   p.nsub = p.n_sub_total % 2 == 0 ? 2 : 1;
-  static const int env_bn = getenv("BSL_HALO_BN") ? atoi(getenv("BSL_HALO_BN")) : 0;      // tuning overrides
-  static const int env_nsub = getenv("BSL_HALO_NSUB") ? atoi(getenv("BSL_HALO_NSUB")) : 0;
-  if (env_bn && ncols % env_bn == 0) p.bn = env_bn;
-  if (env_nsub == 1) p.nsub = 1;
   p.n_ntiles = ncols / p.bn;
   p.n_units = cdiv(p.n_sub_total, p.nsub) * p.n_ntiles;
   int g = std::min(p.n_units, ctx->sm_count);
@@ -523,17 +485,6 @@ HaloPlan plan_halo(bsl_ctx* ctx, int w, int h, int n, int ncols) {
   p.grid = std::max(g, 1);
   p.slots = cdiv(p.grid, p.n_ntiles);
   return p;
-}
-
-// Attaches the image-slice flags a tensor-core kernel waits on (bsl_pipe, include/bsl_b200.h) to the kernel arguments.
-int attach_wait(bsl_ctx* ctx, ConvHaloArgs& a, const bsl_pipe* wait, int n) {
-  if (!wait) return BSL_OK;
-  if (!wait->flags || wait->slices < 1 || wait->slices > 64 || n % wait->slices)
-    return bsl_fail(ctx, BSL_EINVAL, "pipe: slices=%d must divide n=%d and be <= 64", wait->slices, n);
-  a.wait_flags = wait->flags;
-  a.wait_epoch = wait->epoch;
-  a.wait_imgs = n / wait->slices;
-  return BSL_OK;
 }
 
 void halo_common(ConvHaloArgs& a, const HaloPlan& p, int w, int h, int n) {
@@ -545,10 +496,6 @@ void halo_common(ConvHaloArgs& a, const HaloPlan& p, int w, int h, int n) {
   a.n_sub_total = p.n_sub_total;
   a.n_units = p.n_units;
   a.n_ntiles = p.n_ntiles;
-  static const int narrow = getenv("BSL_NARROW_STORE") ? atoi(getenv("BSL_NARROW_STORE")) : 0;
-  a.narrow_store = narrow;
-  static const int slow_issue = getenv("BSL_SLOW_ISSUE") ? atoi(getenv("BSL_SLOW_ISSUE")) : 0;
-  a.slow_issue = slow_issue;
   a.dbg = g_dbg_waits;
   a.kd = 1;        // 2-D: every image is its own one-slice "volume" (tensor map dims (c, w, h, n, 1))
   a.depth = n;
@@ -559,130 +506,26 @@ struct WgradPlan {
 };
 
 bool wgrad_halo_eligible(const bsl_conv2d_desc* d) {
-  return !force_v1() && d->kh == 3 && d->kw == 3 && tiles_ok(d->w, d->h, WG_TW, WG_TH);
+  return d->kh == 3 && d->kw == 3 && tiles_ok(d->w, d->h, WG_TW, WG_TH);
 }
 
-// ---- wide wgrad (wgrad_halo2_kernel): split counts for the two CTA classes, chosen by simulating the hardware's
-// in-order block dispatch onto the SMs (one CTA per SM: 216 KB of shared memory each).
-struct Wgrad2Plan {
+// ---- wide wgrad (wgrad_halo3_kernel): 3x3 layers whose output channels come in 128-wide blocks. Split counts for the
+// two CTA classes are chosen by simulating the hardware's in-order block dispatch onto the SMs.
+struct WideWgradPlan {
   int k_tiles, splits_a, per_a, splits_b, per_b;
-  size_t ws_floats;
 };
 
-bool wgrad2_eligible(const bsl_conv2d_desc* d) {
-  static const int off = getenv("BSL_WGRAD_V2") ? atoi(getenv("BSL_WGRAD_V2")) == 0 : 0;
-  return !off && !force_v1() && d->kh == 3 && d->kw == 3 && tiles_ok(d->w, d->h, WG_TW, WG_TH) && d->cout % 128 == 0;
+bool wgrad_wide_eligible(const bsl_conv2d_desc* d) {
+  return d->kh == 3 && d->kw == 3 && tiles_ok(d->w, d->h, WG_TW, WG_TH) && d->cout % 128 == 0;
 }
 
-Wgrad2Plan plan_wgrad2_core(bsl_ctx* ctx, int k, int mn, size_t per_tap) {
-  Wgrad2Plan best = {};
-  const int sms = ctx->sm_count;
-  const double fixed = 6.0;  // prologue + epilogue of a CTA, in units of one (tile, accumulator) step
-  static const double tb_tile = getenv("BSL_WG2_TB") ? atof(getenv("BSL_WG2_TB")) : 1.0;   // class-b cost of a pixel tile
-  double best_t = 1e300;
-  const int max_a = std::max(1, std::min(k / 2, (2 * sms) / mn + 2));
-  std::vector<double> free_at(sms);
-  for (int na = 1; na <= max_a; ++na) {
-    const int per_a = cdiv(k, na), sa = cdiv(k, per_a);
-    if (sa != na) continue;
-    const int nb_hi = tb_tile > 1.0 ? na + 2 : std::min(na, na / 2 + 2);   // class b has half the MMA work per tile
-    for (int nb2 = std::max(1, na / 2 - 1); nb2 <= nb_hi; ++nb2) {
-      const int per_b = cdiv(k, nb2), sb = cdiv(k, per_b);
-      if (sb != nb2) continue;
-      const double ta = 2.0 * per_a + fixed, tb = tb_tile * per_b + fixed;
-      // in-order dispatch: all class-a CTAs, then class-b, each to the SM that frees up first
-      std::fill(free_at.begin(), free_at.end(), 0.0);
-      const long long ja = (long long)mn * sa, jb = (long long)mn * sb;
-      double makespan = 0;
-      for (long long j = 0; j < ja + jb; ++j) {
-        int arg = 0;
-        for (int m = 1; m < sms; ++m)
-          if (free_at[m] < free_at[arg]) arg = m;
-        free_at[arg] += j < ja ? ta : tb;
-        makespan = std::max(makespan, free_at[arg]);
-      }
-      makespan += 0.02 * (sa + sb);  // a little pressure towards fewer partials to reduce afterwards
-      if (makespan < best_t) {
-        best_t = makespan;
-        best = {k, sa, per_a, sb, per_b, 0};
-      }
-    }
-  }
-  best.ws_floats = ((size_t)(best.splits_a > 1 ? best.splits_a * 6 : 0) + (size_t)(best.splits_b > 1 ? best.splits_b * 3 : 0)) *
-                   per_tap;
-  return best;
-}
-
-Wgrad2Plan plan_wgrad2(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
-  return plan_wgrad2_core(ctx, cdiv(d->w, WG_TW) * cdiv(d->h, WG_TH) * d->n, (d->cin / 64) * (d->cout / 128),
-                          (size_t)d->cin * d->cout);
-}
-
-const Wgrad2Plan& cached_wgrad2(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
-  static std::mutex mu;
-  static std::unordered_map<unsigned long long, Wgrad2Plan> cache;
-  const unsigned long long key = ((unsigned long long)d->n << 48) ^ ((unsigned long long)d->h << 36) ^
-                                 ((unsigned long long)d->w << 24) ^ ((unsigned long long)d->cin << 12) ^ d->cout;
-  std::lock_guard<std::mutex> g(mu);
-  auto it = cache.find(key);
-  if (it == cache.end()) it = cache.emplace(key, plan_wgrad2(ctx, d)).first;
-  return it->second;
-}
-
-int conv2d_wgrad2(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* dy, float* dw, void* workspace,
-                  size_t workspace_bytes, cudaStream_t stream) {
-  const Wgrad2Plan& p = cached_wgrad2(ctx, d);
-  if (p.ws_floats * sizeof(float) > workspace_bytes || (p.ws_floats && !workspace))
-    return bsl_fail(ctx, BSL_EWORKSPACE, "conv2d_wgrad: workspace %zu < %zu", workspace_bytes, p.ws_floats * sizeof(float));
-  const int xbox[4] = {WG_TW + 2, WG_TH + 2, 1, 1}, ybox[4] = {WG_TW, WG_TH, 1, 1};
-  CUtensorMap tx, ty;
-  int rc;
-  if ((rc = nhwc_map(ctx, x, d->cin, d->w, d->h, d->n, d->x_ld, xbox, &tx))) return rc;
-  if ((rc = nhwc_map(ctx, dy, d->cout, d->w, d->h, d->n, d->y_ld, ybox, &ty))) return rc;
-  const long long per_tap = (long long)d->cin * d->cout;
-  float* ws = reinterpret_cast<float*>(workspace);
-  WgradHalo2Args a = {};
-  a.ntile_w = cdiv(d->w, WG_TW);
-  a.ntile_h = cdiv(d->h, WG_TH);
-  a.n = d->n;
-  a.k_tiles_total = p.k_tiles;
-  a.splits_a = p.splits_a;
-  a.per_a = p.per_a;
-  a.splits_b = p.splits_b;
-  a.per_b = p.per_b;
-  a.cin = d->cin;
-  a.cout = d->cout;
-  a.out_a = p.splits_a > 1 ? ws : dw;
-  a.out_b = p.splits_b > 1 ? ws + (p.splits_a > 1 ? (long long)p.splits_a * 6 * per_tap : 0) : dw + 6 * per_tap;
-  a.kd = 1;
-  a.depth = d->n;
-  a.dbg = g_dbg_waits;
-  a.status = ctx->d_status;
-  static bool configured = false;
-  if (!configured) {
-    BSL_CUDA(ctx, cudaFuncSetAttribute(wgrad_halo2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG2_SMEM_BYTES));
-    configured = true;
-  }
-  bsl_launch(wgrad_halo2_kernel, dim3(dim3(d->cin / 64, d->cout / 128, p.splits_a + p.splits_b)), dim3(WG_THREADS), WG2_SMEM_BYTES, stream, 
-      tx, ty, a);
-  BSL_LAUNCH_CHECK(ctx, "wgrad_halo2_kernel launch");
-  if (p.splits_a > 1 && (rc = reduce_splits(ctx, a.out_a, dw, 6 * per_tap, p.splits_a, stream))) return rc;
-  if (p.splits_b > 1 && (rc = reduce_splits(ctx, a.out_b, dw + 6 * per_tap, 3 * per_tap, p.splits_b, stream))) return rc;
-  return BSL_OK;
-}
-
-// ---- wide wgrad, third generation (wgrad_halo3_kernel): every CTA fills two accumulators per pixel tile. Costs per
-// pixel tile in units of 384 tensor cycles, from the per-CTA cycle counters (tools/gpu_conv_bench.py --ops wgrad --waits).
-bool wgrad3_on() {
-  static const int on = getenv("BSL_WGRAD_V3") ? atoi(getenv("BSL_WGRAD_V3")) != 0 : 1;
-  return on;
-}
-
-Wgrad2Plan plan_wgrad3_core(bsl_ctx* ctx, int k, int ncb, int nnbk, size_t per_tap) {
-  static const double cost_a = getenv("BSL_WG3_TA") ? atof(getenv("BSL_WG3_TA")) : 2.0;
-  static const double cost_b2 = getenv("BSL_WG3_TB2") ? atof(getenv("BSL_WG3_TB2")) : 2.1;   // two input blocks
-  static const double cost_b1 = getenv("BSL_WG3_TB1") ? atof(getenv("BSL_WG3_TB1")) : 1.4;   // lone last input block
-  Wgrad2Plan best = {};
+// Every CTA fills two accumulators per pixel tile. Costs per pixel tile in units of 384 tensor cycles, from the per-CTA
+// cycle counters (tools/gpu_conv_bench.py --ops wgrad --waits).
+WideWgradPlan plan_wgrad3_core(bsl_ctx* ctx, int k, int ncb, int nnbk) {
+  const double cost_a = 2.0;
+  const double cost_b2 = 2.1;   // two input blocks
+  const double cost_b1 = 1.4;   // lone last input block
+  WideWgradPlan best = {};
   const int sms = ctx->sm_count;
   const double fixed = 6.0;   // prologue + epilogue of a CTA
   const int ncb_b = cdiv(ncb, 2);
@@ -716,7 +559,7 @@ Wgrad2Plan plan_wgrad3_core(bsl_ctx* ctx, int k, int ncb, int nnbk, size_t per_t
       makespan += 0.02 * (sa + sb);   // a little pressure towards fewer partials to reduce afterwards
       if (makespan < best_t) {
         best_t = makespan;
-        best = {k, sa, per_a, sb, per_b, 0};
+        best = {k, sa, per_a, sb, per_b};
       }
     }
   }
@@ -725,12 +568,12 @@ Wgrad2Plan plan_wgrad3_core(bsl_ctx* ctx, int k, int ncb, int nnbk, size_t per_t
 
 // Launch + reduction of the partials; shared by the 2-D layers (kd = 1, depth = n) and UNet3D's stride-1 layers.
 // Partials are [split][kd][taps][cin][cout]; a class with a single split writes its rows of dW directly when kd == 1.
-size_t wgrad3_ws_bytes(const Wgrad2Plan& q, int kd, size_t per_tap) {
+size_t wgrad3_ws_bytes(const WideWgradPlan& q, int kd, size_t per_tap) {
   const bool direct_a = q.splits_a == 1 && kd == 1, direct_b = q.splits_b == 1 && kd == 1;
   return ((direct_a ? 0 : (size_t)q.splits_a * 6) + (direct_b ? 0 : (size_t)q.splits_b * 3)) * kd * per_tap * sizeof(float);
 }
 
-int launch_wgrad3(bsl_ctx* ctx, const Wgrad2Plan& q, const CUtensorMap& txa, const CUtensorMap& txb, const CUtensorMap& ty,
+int launch_wgrad3(bsl_ctx* ctx, const WideWgradPlan& q, const CUtensorMap& txa, const CUtensorMap& txb, const CUtensorMap& ty,
                   int w, int h, int n_imgs, int cin, int cout, int kd, int depth, float* dw, void* workspace,
                   size_t workspace_bytes, cudaStream_t stream) {
   const long long per_tap = (long long)cin * cout;
@@ -760,11 +603,9 @@ int launch_wgrad3(bsl_ctx* ctx, const Wgrad2Plan& q, const CUtensorMap& txa, con
   a.depth = depth;
   a.dbg = g_dbg_waits;
   a.status = ctx->d_status;
-  static const int st_a = std::min(WG3_MAX_STAGES, std::max(2, getenv("BSL_WG3_STAGES_A") ? atoi(getenv("BSL_WG3_STAGES_A")) : WG3_STAGES_A));
-  static const int st_b = std::min(6, std::max(2, getenv("BSL_WG3_STAGES_B") ? atoi(getenv("BSL_WG3_STAGES_B")) : WG3_STAGES_B));
-  a.stages_a = st_a;
-  a.stages_b = st_b;
-  const int smem = wg3_smem_bytes(st_a, st_b);
+  a.stages_a = WG3_STAGES_A;
+  a.stages_b = WG3_STAGES_B;
+  constexpr int smem = wg3_smem_bytes(WG3_STAGES_A, WG3_STAGES_B);
   static bool configured = false;
   if (!configured) {
     BSL_CUDA(ctx, cudaFuncSetAttribute(wgrad_halo3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -785,22 +626,21 @@ int launch_wgrad3(bsl_ctx* ctx, const Wgrad2Plan& q, const CUtensorMap& txa, con
   return BSL_OK;
 }
 
-const Wgrad2Plan& cached_wgrad3(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
+const WideWgradPlan& cached_wgrad3(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
   static std::mutex mu;
-  static std::unordered_map<unsigned long long, Wgrad2Plan> cache;
+  static std::unordered_map<unsigned long long, WideWgradPlan> cache;
   const unsigned long long key = ((unsigned long long)d->n << 48) ^ ((unsigned long long)d->h << 36) ^
                                  ((unsigned long long)d->w << 24) ^ ((unsigned long long)d->cin << 12) ^ d->cout;
   std::lock_guard<std::mutex> g(mu);
   auto it = cache.find(key);
   if (it == cache.end())
-    it = cache.emplace(key, plan_wgrad3_core(ctx, cdiv(d->w, WG_TW) * cdiv(d->h, WG_TH) * d->n, d->cin / 64, d->cout / 128,
-                                             (size_t)d->cin * d->cout)).first;
+    it = cache.emplace(key, plan_wgrad3_core(ctx, cdiv(d->w, WG_TW) * cdiv(d->h, WG_TH) * d->n, d->cin / 64, d->cout / 128)).first;
   return it->second;
 }
 
 int conv2d_wgrad3(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* dy, float* dw, void* workspace,
                   size_t workspace_bytes, cudaStream_t stream) {
-  const Wgrad2Plan& p = cached_wgrad3(ctx, d);
+  const WideWgradPlan& p = cached_wgrad3(ctx, d);
   const int xbox_a[4] = {WG_TW + 2, WG_TH + 1, 1, 1}, xbox_b[4] = {WG_TW + 2, WG_TH, 1, 1}, ybox[4] = {WG_TW, WG_TH, 1, 1};
   CUtensorMap txa, txb, ty;
   int rc;
@@ -838,7 +678,6 @@ int bsl_debug_set(bsl_ctx* ctx, int key, int value) {
         g_dbg_waits = nullptr;
       }
       return BSL_OK;
-    case 4: bsl_pdl_set(value); return BSL_OK;   // programmatic dependent launch on / off (internal.h)
   }
   return bsl_fail(ctx, BSL_EINVAL, "debug_set: unknown key %d", key);
 }
@@ -904,14 +743,12 @@ static int launch_fprop_halo_stats(bsl_ctx* ctx, const HaloPlan& pl, bool res, i
 // sum of squares of the bf16 outputs, reduced deterministically from per-CTA partials.
 // group_imgs > 0: instance statistics, sums is [n / group_imgs][2][cout] (one group = group_imgs consecutive images).
 static int conv2d_fprop_halo(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
-                             double* sums, cudaStream_t stream, const bsl_pipe* wait = nullptr, int group_imgs = 0) {
+                             double* sums, cudaStream_t stream, int group_imgs = 0) {
   const int halo = d->kh == 3 ? 1 : 0;
   HaloPlan pl = plan_halo(ctx, d->w, d->h, d->n, d->cout);
   int res_stages = 0, res_smem = 0;
   bool res = false;
   const void* w_k = nullptr;   // K-major copy of the filter (resident CTA pairs)
-  // (also under image-slice flags, `wait`: the fused statistics are summed per CTA, so both schedules must run the same
-  //  kernel to stay bit-identical -- tests/test_gpu_unet.py::test_image_slice_pipelining_is_bit_identical)
   if (d->cout == pl.bn && d->cin % 64 == 0 && d->x_ld >= d->cin &&
       plan_resident_pair(ctx, pl.bn, d->kh * d->kw, d->cin / 64, pl.n_sub_total, &pl.nsub, &res_stages, &res_smem)) {
     void* wk = nullptr;
@@ -927,7 +764,7 @@ static int conv2d_fprop_halo(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void*
   } else {
     res = plan_resident(pl.bn, d->kh * d->kw, d->cin / 64, &pl.nsub, &res_stages, &res_smem);
     if (res) replan_units(ctx, pl);
-    else if (!wait) pair_replan(ctx, pl, d->cout, 256, d->kh * d->kw);
+    else pair_replan(ctx, pl, d->cout, 256, d->kh * d->kw);
   }
   const int box[4] = {8 + 2 * halo, 16 + 2 * halo, 1, 1};
   CUtensorMap ta, tb;
@@ -952,7 +789,6 @@ static int conv2d_fprop_halo(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void*
   a.a_stages = res_stages;
   a.b_rows_per_tap = d->cout;   // (K-major copy of a resident CTA pair; unused otherwise)
   a.status = ctx->d_status;
-  if ((rc = attach_wait(ctx, a, wait, d->n))) return rc;
   return launch_fprop_halo_stats(ctx, pl, res, res_smem, ta, tb, a, sums, group_imgs, d->n, d->h, d->w, d->cout, y,
                                  d->y_ld, stream);
 }
@@ -974,25 +810,10 @@ int bsl_conv2d_fprop_group_stats(bsl_ctx* ctx, const bsl_conv2d_desc* d, const v
   if (!x || !w || !y || !sums) return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop_group_stats: null buffer");
   if (imgs_per_group < 1 || d->n % imgs_per_group)
     return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop_group_stats: imgs_per_group=%d must divide n=%d", imgs_per_group, d->n);
-  if (halo_eligible(d->w, d->h)) return conv2d_fprop_halo(ctx, d, x, w, y, sums, as_stream(stream), nullptr, imgs_per_group);
+  if (halo_eligible(d->w, d->h)) return conv2d_fprop_halo(ctx, d, x, w, y, sums, as_stream(stream), imgs_per_group);
   if ((rc = bsl_conv2d_fprop(ctx, d, x, w, y, stream))) return rc;
   return bsl_stats_bf16(ctx, y, (long long)imgs_per_group * d->h * d->w, d->n / imgs_per_group, d->cout, d->y_ld, sums,
                         as_stream(stream));
-}
-
-int bsl_conv2d_fprop_pipe(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
-                          double* sums, const bsl_pipe* wait, void* stream) {
-  int rc = check_conv(ctx, d, true);
-  if (rc) return rc;
-  if (!x || !w || !y) return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop_pipe: null buffer");
-  if (!halo_eligible(d->w, d->h))
-    return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv2d_fprop_pipe: %dx%d is not on the halo-tile kernel", d->h, d->w);
-  return conv2d_fprop_halo(ctx, d, x, w, y, sums, as_stream(stream), wait);
-}
-
-int bsl_conv2d_pipe_ok(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
-  (void)ctx;
-  return d && halo_eligible(d->w, d->h) ? 1 : 0;
 }
 
 int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
@@ -1023,50 +844,24 @@ int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, cons
   return launch_igemm<MODE_PIX_M, true>(ctx, bn, ta, tb, a, grid, as_stream(stream));
 }
 
-static int conv2d_dgrad_impl(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,
-                             const bsl_pipe* wait, const void* relu_act, int mask_col0, void* stream);
-
 int bsl_conv2d_dgrad(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,
                      void* stream) {
-  return conv2d_dgrad_impl(ctx, d, dy, w, dx, nullptr, nullptr, 0, stream);
-}
-
-int bsl_conv2d_dgrad_pipe(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,
-                          const bsl_pipe* wait, void* stream) {
-  return conv2d_dgrad_impl(ctx, d, dy, w, dx, wait, nullptr, 0, stream);
-}
-
-int bsl_conv2d_dgrad_relu(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,
-                          const void* act, int col0, const bsl_pipe* wait, void* stream) {
-  if (!act || col0 < 0 || col0 % 32 || (d && col0 > d->cin))
-    return bsl_fail(ctx, BSL_EINVAL, "conv2d_dgrad_relu: act required, col0 a multiple of 32 within cin");
-  if (d && !halo_eligible(d->w, d->h))
-    return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv2d_dgrad_relu: %dx%d is not on the halo-tile kernel", d->h, d->w);
-  if (d && (d->x_ld % 16 || (reinterpret_cast<uintptr_t>(act) & 31) || (reinterpret_cast<uintptr_t>(dx) & 31)))
-    return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv2d_dgrad_relu: dx / act need 32-byte aligned pixels (x_ld %% 16 == 0)");
-  return conv2d_dgrad_impl(ctx, d, dy, w, dx, wait, act, col0, stream);
-}
-
-static int conv2d_dgrad_impl(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,
-                             const bsl_pipe* wait, const void* relu_act, int mask_col0, void* stream) {
   int rc = check_conv(ctx, d);
   if (rc) return rc;
   if (!dy || !w || !dx) return bsl_fail(ctx, BSL_EINVAL, "conv2d_dgrad: null buffer");
-  if (wait && !halo_eligible(d->w, d->h))
-    return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv2d_dgrad_pipe: %dx%d is not on the halo-tile kernel", d->h, d->w);
   if (halo_eligible(d->w, d->h)) {
     const int halo = d->kh == 3 ? 1 : 0;
     HaloPlan pl = plan_halo(ctx, d->w, d->h, d->n, d->cin);
     int res_stages = 0, res_smem = 0;
     bool res = false, res_pair = false;
-    if (!wait && !relu_act && d->cin == pl.bn &&
+    if (d->cin == pl.bn &&
         plan_resident_pair(ctx, pl.bn, d->kh * d->kw, d->cout / 64, pl.n_sub_total, &pl.nsub, &res_stages, &res_smem)) {
       res = res_pair = true;
       replan_pair_units(ctx, pl);
     } else {
       res = plan_resident(pl.bn, d->kh * d->kw, d->cout / 64, &pl.nsub, &res_stages, &res_smem);
       if (res) replan_units(ctx, pl);
-      else if (!wait && !relu_act) pair_replan(ctx, pl, d->cin, 128, d->kh * d->kw);
+      else pair_replan(ctx, pl, d->cin, 128, d->kh * d->kw);
     }
     const int hbox[4] = {8 + 2 * halo, 16 + 2 * halo, 1, 1};
     CUtensorMap ta, tb;
@@ -1087,9 +882,6 @@ static int conv2d_dgrad_impl(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void*
     a.n_total = d->cin;
     a.a_stages = res_stages;
     a.status = ctx->d_status;
-    if ((rc = attach_wait(ctx, a, wait, d->n))) return rc;
-    a.relu_mask = relu_act;
-    a.mask_col0 = mask_col0;
     if (res_pair) return launch_halo_res_pair<false>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, res_smem, as_stream(stream));
     if (res) return launch_halo_res<false, false, false>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, res_smem, as_stream(stream));
     CUtensorMap tbh;
@@ -1124,9 +916,7 @@ static int conv2d_dgrad_impl(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void*
 
 size_t bsl_conv2d_wgrad_workspace(bsl_ctx* ctx, const bsl_conv2d_desc* d) {
   if (!ctx || !d || check_conv(ctx, d, true)) return 0;
-  if (wgrad2_eligible(d))
-    return wgrad3_on() ? wgrad3_ws_bytes(cached_wgrad3(ctx, d), 1, (size_t)d->cin * d->cout)
-                       : cached_wgrad2(ctx, d).ws_floats * sizeof(float);
+  if (wgrad_wide_eligible(d)) return wgrad3_ws_bytes(cached_wgrad3(ctx, d), 1, (size_t)d->cin * d->cout);
   if (wgrad_halo_eligible(d)) {
     const WgradPlan p = plan_wgrad_halo(ctx, d);
     return p.splits > 1 ? (size_t)p.splits * 9 * d->cin * d->cout * sizeof(float) : 0;
@@ -1146,9 +936,7 @@ int bsl_conv2d_wgrad(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, cons
   int rc = check_conv(ctx, d, true);
   if (rc) return rc;
   if (!x || !dy || !dw) return bsl_fail(ctx, BSL_EINVAL, "conv2d_wgrad: null buffer");
-  if (wgrad2_eligible(d))
-    return wgrad3_on() ? conv2d_wgrad3(ctx, d, x, dy, dw, workspace, workspace_bytes, as_stream(stream))
-                       : conv2d_wgrad2(ctx, d, x, dy, dw, workspace, workspace_bytes, as_stream(stream));
+  if (wgrad_wide_eligible(d)) return conv2d_wgrad3(ctx, d, x, dy, dw, workspace, workspace_bytes, as_stream(stream));
   if (wgrad_halo_eligible(d)) {
     const WgradPlan p = plan_wgrad_halo(ctx, d);
     const size_t need = p.splits > 1 ? (size_t)p.splits * 9 * d->cin * d->cout * sizeof(float) : 0;
@@ -1233,11 +1021,6 @@ static int check_convT(bsl_ctx* ctx, const bsl_convT2d_desc* d) {
   return BSL_OK;
 }
 
-int bsl_convT2d_fwd(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x, const void* w,
-                    const float* bias, void* y, void* stream) {
-  return bsl_convT2d_fwd_pipe(ctx, d, x, w, bias, y, nullptr, stream);
-}
-
 // cout = 32 into a pixel-pair packed tensor: output voxel (2y + a, 2x + b) lane co lives at
 // y[((n * 2h + 2y + a) * w + x) * y_ld + b * 32 + co], y_ld = lanes per voxel PAIR. The GEMM columns (a, b, co) are
 // the filter's own row order, so this is a transposed conv with 2 "taps" (a) of 64 columns each.
@@ -1278,13 +1061,11 @@ int bsl_convT2d_fwd_pairs(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x
              : launch_halo<false, false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, as_stream(stream));
 }
 
-int bsl_convT2d_fwd_pipe(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x, const void* w,
-                         const float* bias, void* y, const bsl_pipe* wait, void* stream) {
+int bsl_convT2d_fwd(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x, const void* w,
+                    const float* bias, void* y, void* stream) {
   int rc = check_convT(ctx, d);
   if (rc) return rc;
   if (!x || !w || !y) return bsl_fail(ctx, BSL_EINVAL, "convT2d_fwd: null buffer");
-  if (wait && !halo_eligible(d->w, d->h))
-    return bsl_fail(ctx, BSL_EUNSUPPORTED, "convT2d_fwd_pipe: %dx%d is not on the halo-tile kernel", d->h, d->w);
   if (halo_eligible(d->w, d->h)) {
     HaloPlan pl = plan_halo(ctx, d->w, d->h, d->n, 4 * d->cout);
     if (pl.bn == 256 && d->cin <= 256) {
@@ -1320,7 +1101,6 @@ int bsl_convT2d_fwd_pipe(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x,
     a.n_total = 4 * d->cout;
     a.a_stages = res_stages;
     a.status = ctx->d_status;
-    if ((rc = attach_wait(ctx, a, wait, d->n))) return rc;
     return res ? launch_halo_res<false, false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, res_smem, as_stream(stream))
                : launch_halo<false, false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, as_stream(stream));
   }
@@ -1357,8 +1137,7 @@ int bsl_convT2d_bwd_data(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* dy
   int rc = check_convT(ctx, d);
   if (rc) return rc;
   if (!dyr || !w || !dx) return bsl_fail(ctx, BSL_EINVAL, "convT2d_bwd_data: null buffer");
-  static const int up_off = getenv("BSL_CONVT_DGRAD_V1") ? atoi(getenv("BSL_CONVT_DGRAD_V1")) : 0;
-  if (!up_off && halo_eligible(d->w, d->n * d->h)) {
+  if (halo_eligible(d->w, d->n * d->h)) {
     // Persistent halo-tile kernel as a 1-tap GEMM: dx[p, ci] = sum over (a, b, co) of dy[2y+a, 2x+b, co] w[a,b,co,ci].
     // For a fixed row parity a the pair (b, co) is the channel axis of a row-strided view of dy, so the reduction is
     // 2 "depth" steps (a) x 2 (b) x co/64 dense TMA boxes, no element-strided gather; the rows of all images form one
@@ -1611,7 +1390,7 @@ PhaseTaps phase_taps(int in, int k, int s, int phase) {
 }  // namespace
 
 bool bsl_conv3d_halo_dgrad_strided_ok(const bsl_conv3d_desc* d) {
-  if (force_v1() || d->sd != 1 || !(d->kd == 1 || d->kd == 3) || (d->sh == 1 && d->sw == 1)) return false;
+  if (d->sd != 1 || !(d->kd == 1 || d->kd == 3) || (d->sh == 1 && d->sw == 1)) return false;
   if (d->kh < 2 || d->kh > 3 || d->kw < 2 || d->kw > 3 || d->h % d->sh || d->w % d->sw) return false;
   if (!halo_eligible(d->w / d->sw, d->h / d->sh)) return false;
   for (int ph = 0; ph < d->sh; ++ph)
@@ -1675,13 +1454,13 @@ int bsl_conv3d_halo_dgrad_strided(bsl_ctx* ctx, const bsl_conv3d_desc* d, const 
 }
 
 bool bsl_conv3d_halo_wgrad_ok(const bsl_conv3d_desc* d) {
-  return !force_v1() && d3_stride1(d) && tiles_ok(d->w, d->h, WG_TW, WG_TH);
+  return d3_stride1(d) && tiles_ok(d->w, d->h, WG_TW, WG_TH);
 }
 
 namespace {
 struct Wgrad3Plan {
   bool wide;
-  Wgrad2Plan w2;
+  WideWgradPlan w2;
   int k_tiles, per, splits;
   size_t ws_bytes;
 };
@@ -1703,16 +1482,10 @@ Wgrad3Plan plan_wgrad3_halo_uncached(bsl_ctx* ctx, const bsl_conv3d_desc* d) {
   Wgrad3Plan p = {};
   p.k_tiles = cdiv(d->w, WG_TW) * cdiv(d->h, WG_TH) * d->n * d->d;
   const size_t per_tap = (size_t)d->cin * d->cout;
-  static const int v2off = getenv("BSL_WGRAD_V2") ? atoi(getenv("BSL_WGRAD_V2")) == 0 : 0;
-  p.wide = !v2off && d->cout % 128 == 0;
-  if (p.wide && wgrad3_on()) {
-    p.w2 = plan_wgrad3_core(ctx, p.k_tiles, d->cin / 64, (d->cout / 128) * d->kd, per_tap);
+  p.wide = d->cout % 128 == 0;
+  if (p.wide) {
+    p.w2 = plan_wgrad3_core(ctx, p.k_tiles, d->cin / 64, (d->cout / 128) * d->kd);
     p.ws_bytes = wgrad3_ws_bytes(p.w2, d->kd, per_tap);
-  } else if (p.wide) {
-    p.w2 = plan_wgrad2_core(ctx, p.k_tiles, (d->cin / 64) * (d->cout / 128) * d->kd, per_tap);
-    const bool direct_a = p.w2.splits_a == 1 && d->kd == 1, direct_b = p.w2.splits_b == 1 && d->kd == 1;
-    p.ws_bytes = ((direct_a ? 0 : (size_t)p.w2.splits_a * 6) + (direct_b ? 0 : (size_t)p.w2.splits_b * 3)) * d->kd * per_tap *
-                 sizeof(float);
   } else {
     const int mn = (d->cin / 64) * (d->cout / 64) * d->kd;
     int splits = std::max(1, ctx->sm_count / mn);
@@ -1738,54 +1511,12 @@ int bsl_conv3d_halo_wgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x,
   if ((rc = ndhwc_halo_map(ctx, dy, d->cout, d->w, d->h, d->d, d->n, d->y_ld, WG_TW, WG_TH, &ty))) return rc;
   const long long per_tap = (long long)d->cin * d->cout;
   float* ws = reinterpret_cast<float*>(workspace);
-  if (p.wide && wgrad3_on()) {
+  if (p.wide) {
     CUtensorMap txa, txb;
     if ((rc = ndhwc_halo_map(ctx, x, d->cin, d->w, d->h, d->d, d->n, d->x_ld, WG_TW + 2, WG_TH + 1, &txa))) return rc;
     if ((rc = ndhwc_halo_map(ctx, x, d->cin, d->w, d->h, d->d, d->n, d->x_ld, WG_TW + 2, WG_TH, &txb))) return rc;
     return launch_wgrad3(ctx, p.w2, txa, txb, ty, d->w, d->h, d->n * d->d, d->cin, d->cout, d->kd, d->d, dw, workspace,
                          workspace_bytes, stream);
-  }
-  if (p.wide) {
-    const Wgrad2Plan& q = p.w2;
-    WgradHalo2Args a = {};
-    a.ntile_w = cdiv(d->w, WG_TW);
-    a.ntile_h = cdiv(d->h, WG_TH);
-    a.n = d->n * d->d;
-    a.k_tiles_total = q.k_tiles;
-    a.splits_a = q.splits_a;
-    a.per_a = q.per_a;
-    a.splits_b = q.splits_b;
-    a.per_b = q.per_b;
-    a.cin = d->cin;
-    a.cout = d->cout;
-    a.kd = d->kd;
-    a.depth = d->d;
-    // partial layouts [split][kd][taps]; with a single split the kernel writes dW rows directly, which needs the
-    // per-depth stride of dW (9 taps) instead of 6 / 3: only taken when kd == 1, otherwise always through partials
-    const bool direct_a = q.splits_a == 1 && d->kd == 1, direct_b = q.splits_b == 1 && d->kd == 1;
-    const size_t need = ((direct_a ? 0 : (size_t)q.splits_a * 6) + (direct_b ? 0 : (size_t)q.splits_b * 3)) * d->kd * per_tap *
-                        sizeof(float);
-    if (need > workspace_bytes) return bsl_fail(ctx, BSL_EWORKSPACE, "conv3d_wgrad: workspace %zu < %zu", workspace_bytes, need);
-    a.out_a = direct_a ? dw : ws;
-    a.out_b = direct_b ? dw + 6 * per_tap : ws + (direct_a ? 0 : (long long)q.splits_a * d->kd * 6 * per_tap);
-    a.status = ctx->d_status;
-    static bool configured = false;
-    if (!configured) {
-      BSL_CUDA(ctx, cudaFuncSetAttribute(wgrad_halo2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG2_SMEM_BYTES));
-      configured = true;
-    }
-    bsl_launch(wgrad_halo2_kernel, dim3(dim3(d->cin / 64, d->cout / 128, d->kd * (q.splits_a + q.splits_b))), dim3(WG_THREADS), WG2_SMEM_BYTES, stream, tx, ty, a);
-    BSL_LAUNCH_CHECK(ctx, "wgrad_halo2_kernel launch (3-D)");
-    for (int k = 0; k < d->kd; ++k) {   // partial[split][kd][taps] -> dW[kd][9]: split stride = kd * taps * per_tap
-      if (!direct_a && (rc = reduce_splits_strided(ctx, a.out_a + (long long)k * 6 * per_tap, dw + (long long)k * 9 * per_tap,
-                                                   6 * per_tap, q.splits_a, (long long)d->kd * 6 * per_tap, stream)))
-        return rc;
-      if (!direct_b && (rc = reduce_splits_strided(ctx, a.out_b + (long long)k * 3 * per_tap,
-                                                   dw + ((long long)k * 9 + 6) * per_tap, 3 * per_tap, q.splits_b,
-                                                   (long long)d->kd * 3 * per_tap, stream)))
-        return rc;
-    }
-    return BSL_OK;
   }
   WgradHaloArgs a = {};
   a.ntile_w = cdiv(d->w, WG_TW);

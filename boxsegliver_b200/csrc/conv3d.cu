@@ -140,7 +140,7 @@ SplitPlan plan_split(bsl_ctx* ctx, int mn_tiles, int k_tiles) {
 }
 
 __global__ void reduce_splits3_kernel(const float* __restrict__ part, float* __restrict__ out, long long n, int splits) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * 4;
   if (i >= n) return;
   float4 acc = *reinterpret_cast<const float4*>(part + i);
@@ -265,8 +265,7 @@ int bsl_conv3d_dgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy, con
   if (rc) return rc;
   if (!dy || !w || !dx) return bsl_fail(ctx, BSL_EINVAL, "conv3d_dgrad: null buffer");
   if (bsl_conv3d_halo_ok(d)) return bsl_conv3d_halo_dgrad(ctx, d, dy, w, dx, as_stream(stream));
-  static const bool no_halo_strided = getenv("BSL_DGRAD_STRIDED_V1") && atoi(getenv("BSL_DGRAD_STRIDED_V1"));
-  if (!no_halo_strided && bsl_conv3d_halo_dgrad_strided_ok(d))
+  if (bsl_conv3d_halo_dgrad_strided_ok(d))
     return bsl_conv3d_halo_dgrad_strided(ctx, d, dy, w, dx, as_stream(stream));
   for (int i = 0; i < 3; ++i)
     if (g.in[i] % g.s[i]) return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv3d_dgrad: extents must be multiples of the stride");

@@ -25,7 +25,7 @@ __device__ __forceinline__ float dropout_scale(const bsl_dropout_desc& dd, unsig
 __global__ void fc_fwd_kernel(int n, int cin, int cout, const float* __restrict__ x, const float* __restrict__ w,
                               const float* __restrict__ b, int relu, bsl_dropout_desc dd, int use_dropout,
                               float* __restrict__ y) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n * cout) return;
   const int s = i / cout, co = i - s * cout;
@@ -40,7 +40,7 @@ __global__ void fc_fwd_kernel(int n, int cin, int cout, const float* __restrict_
 // dpre = dy * d(out)/d(pre): out = relu(pre) * mask / keep, so out > 0 <=> (pre > 0 and kept).
 __global__ void fc_dpre_kernel(int total, const float* __restrict__ y, const float* __restrict__ dy, int relu,
                                float inv_keep, float* __restrict__ dpre) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   float g = dy[i];
@@ -50,7 +50,7 @@ __global__ void fc_dpre_kernel(int total, const float* __restrict__ y, const flo
 
 __global__ void fc_dw_kernel(int n, int cin, int cout, const float* __restrict__ x, const float* __restrict__ dpre,
                              float* __restrict__ dw, float* __restrict__ db) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (cin + 1) * cout) return;
   const int ci = i / cout, co = i - ci * cout;
@@ -67,7 +67,7 @@ __global__ void fc_dw_kernel(int n, int cin, int cout, const float* __restrict__
 // one warp per (sample, input feature): lanes stride over cout (coalesced rows of w), shuffle tree at the end
 __global__ void fc_dx_kernel(int n, int cin, int cout, const float* __restrict__ dpre, const float* __restrict__ w,
                              float* __restrict__ dx) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= n * cin) return;
   const int s = warp / cin, ci = warp - s * cin;
@@ -79,7 +79,7 @@ __global__ void fc_dx_kernel(int n, int cin, int cout, const float* __restrict__
 }
 
 __global__ void avgpool2x2_f32_kernel(int n, int h, int w, int c, const float* __restrict__ x, float* __restrict__ y) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int ho = h / 2, wo = w / 2;
   const long long total = (long long)n * ho * wo * c;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -98,7 +98,7 @@ __global__ void avgpool2x2_f32_kernel(int n, int h, int w, int c, const float* _
 // norm + ReLU + pool pass). bf16 rounding is monotonic, so round(max) == max(round).
 __global__ void maxpool2x2_f32_bf16_kernel(int n, int h, int w, int c, const float* __restrict__ x,
                                            __nv_bfloat16* __restrict__ y, int y_ld) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int ho = h / 2, wo = w / 2;
   const long long total = (long long)n * ho * wo * c;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -118,7 +118,7 @@ __global__ void maxpool2x2_f32_bf16_kernel(int n, int h, int w, int c, const flo
 // y_ld (the remaining lanes of the zero-initialised buffer pad the first conv's input to a 64-channel block).
 __global__ void image_gradients_pack_kernel(int n, int h, int w, int c, const float* __restrict__ x,
                                             __nv_bfloat16* __restrict__ y, int y_ld) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const long long total = (long long)n * h * w * c;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     long long t = i;
@@ -140,7 +140,7 @@ __global__ void image_gradients_pack_kernel(int n, int h, int w, int c, const fl
 // Philox counters (flat element index over the dense [pixels, c] tensor, as bsl_dropout_mask enumerates it).
 __global__ void dropout_bf16_kernel(long long pixels, int c, bsl_dropout_desc dd, const __nv_bfloat16* __restrict__ x,
                                     int x_ld, __nv_bfloat16* __restrict__ out, int o_ld) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int cg = c / 8;
   const long long total = pixels * cg;
   const float inv = 1.0f / dd.keep_prob;
@@ -174,7 +174,7 @@ __global__ void dropout_bf16_kernel(long long pixels, int c, bsl_dropout_desc dd
 }
 
 __global__ void dropout_mask_kernel(int total, bsl_dropout_desc dd, float* __restrict__ out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < total) out[i] = dropout_scale(dd, (unsigned long long)i);
 }

@@ -86,7 +86,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   const uint32_t tfull = smem_u32(&bars[2 * STAGES]);
   DeviceStatus* st = p.status;
 
-  pdl_trigger();
   if (threadIdx.x == 0) dead = *reinterpret_cast<volatile int*>(&st->error);
   __syncthreads();
   if (dead) return;

@@ -61,7 +61,6 @@ wgrad_halo_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
   const uint32_t tfull = smem_u32(&bars[2 * WG_STAGES]);
   DeviceStatus* st = p.status;
 
-  pdl_trigger();
   if (threadIdx.x == 0) dead = *reinterpret_cast<volatile int*>(&st->error);
   __syncthreads();
   if (dead) return;
@@ -148,7 +147,6 @@ wgrad_halo_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
         if (++stage == WG_STAGES) { stage = 0; phase ^= 1; }
       }
       if (ok) umma_commit(tfull);
-      pdl_trigger_late();
     }
   } else {
     const int q4 = warp & 3;
@@ -188,183 +186,12 @@ wgrad_halo_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
 }
 
 // ------------------------------------------------------------------------------------------------ wgrad, wide
-// Second filter-gradient kernel for layers with cout % 128 == 0. wgrad_halo_kernel issues 128 x 64 x 16 UMMAs, whose
-// operand fetch (6 KB per 32 tensor-pipe cycles) saturates the shared-memory read path at ~55 % tensor utilisation
-// (profiles/r01_ncu_full_conv_kernels.txt: l1tex tc wavefronts 82 %). Here the roles are swapped: A = dy tile
-// (M = 128 output channels), B = THREE taps of one filter row read from the halo tile as a 192-wide MN-major operand
-// (the 64-element blocks of the descriptor are 128 B = one pixel apart), so one UMMA is 128 x 192 x 16: 10 KB of
-// operands per 96 cycles. A CTA owns 64 input x 128 output channels and either filter rows r = 0, 1 (two 192-column
-// accumulators) or row r = 2 (one accumulator, given twice the pixel range), split-K over pixel tiles.
-struct WgradHalo2Args {
-  int ntile_w, ntile_h, n;       // pixel tiles of 16 (w) x 4 (h)
-  int k_tiles_total;
-  int splits_a, per_a;           // blockIdx.z <  splits_a: rows 0, 1 over tiles [z * per_a, ...)
-  int splits_b, per_b;           // blockIdx.z >= splits_a: row 2 over tiles [(z - splits_a) * per_b, ...)
-  int cin, cout;
-  float* out_a;                  // [splits_a][kd][6][cin][cout]
-  float* out_b;                  // [splits_b][kd][3][cin][cout]
-  int kd, depth;                 // filter depth: blockIdx.z = class offset + kdi * splits + split
-  long long* dbg;                // tuning (bsl_debug_set key 3): per CTA (linear id < 1024) {issuer cycles, cycles waiting for
-                                 // a full stage, class (0 = rows 0,1; 1 = row 2) << 32 | pixel tiles, start ns}
-  DeviceStatus* status;
-};
-
-constexpr int WG2_DY_BYTES = 2 * WG_DY_BYTES;           // 128 output channels = two 64-channel blocks
-constexpr int WG2_STAGE_BYTES = WG_X_BYTES + WG2_DY_BYTES;
-constexpr int WG2_STAGES = 7;
-constexpr int WG2_SMEM_BYTES = WG2_STAGES * WG2_STAGE_BYTES + 1024;
-
-// grid = (cin / 64, cout / 128, splits_a + splits_b)
-__global__ void __launch_bounds__(WG_THREADS)
-wgrad_halo2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmDY,
-                   const WgradHalo2Args p) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bars[2 * WG2_STAGES + 1];
-  __shared__ uint32_t tmem_slot;
-  __shared__ int dead;
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t full0 = smem_u32(&bars[0]);
-  const uint32_t empty0 = smem_u32(&bars[WG2_STAGES]);
-  const uint32_t tfull = smem_u32(&bars[2 * WG2_STAGES]);
-  DeviceStatus* st = p.status;
-
-  pdl_trigger();
-  if (threadIdx.x == 0) dead = *reinterpret_cast<volatile int*>(&st->error);
-  __syncthreads();
-  if (dead) return;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tensormap(&tmX);
-    prefetch_tensormap(&tmDY);
-    for (int s = 0; s < WG2_STAGES; ++s) {
-      mbar_init(full0 + 8 * s, 1);
-      mbar_init(empty0 + 8 * s, 1);
-    }
-    mbar_init(tfull, 1);
-    fence_barrier_init();
-  } else if (warp == 1) {
-    tmem_alloc<512>(smem_u32(&tmem_slot));
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  pdl_wait();   // the prologue above touches no data of the previous kernel in the stream
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(&tmem_slot);
-
-  const int cb = blockIdx.x, nb = blockIdx.y;
-  const bool type_a = (int)blockIdx.z < p.kd * p.splits_a;
-  const int zz = type_a ? blockIdx.z : blockIdx.z - p.kd * p.splits_a;
-  const int nsplit = type_a ? p.splits_a : p.splits_b;
-  const int kdi = zz / nsplit, zi = zz - kdi * nsplit;
-  const int per = type_a ? p.per_a : p.per_b;
-  const int k_begin = zi * per;
-  const int k_end = min(p.k_tiles_total, k_begin + per);
-  const int num_k = max(k_end - k_begin, 0);
-  const int nacc = type_a ? 2 : 1;
-  const int r0 = type_a ? 0 : 2;
-
-  if (warp == 0) {
-    if (elect_one_sync()) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int kk = 0; kk < num_k; ++kk) {
-        if (!mbar_wait(empty0 + 8 * stage, phase ^ 1, st, 14)) break;
-        int t = k_begin + kk;
-        const int tx = t % p.ntile_w;
-        t /= p.ntile_w;
-        const int ty = t % p.ntile_h;
-        const int img = t / p.ntile_h;
-        const uint32_t fb = full0 + 8 * stage;
-        const uint32_t sx = smem_base + stage * WG2_STAGE_BYTES;
-        mbar_arrive_expect_tx(fb, WG_X_ROWS * 128 + WG2_DY_BYTES);
-        const int z = img % p.depth, vol = img / p.depth;
-        tma_load_5d(sx, &tmX, fb, cb * 64, tx * WG_TW - 1, ty * WG_TH - 1, z + kdi - (p.kd >> 1), vol);
-        tma_load_5d(sx + WG_X_BYTES, &tmDY, fb, nb * 128, tx * WG_TW, ty * WG_TH, z, vol);
-        tma_load_5d(sx + WG_X_BYTES + WG_DY_BYTES, &tmDY, fb, nb * 128 + 64, tx * WG_TW, ty * WG_TH, z, vol);
-        if (++stage == WG2_STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
-  } else if (warp == 1) {
-    if (elect_one_sync()) {
-      constexpr uint32_t idesc = make_idesc_bf16(128, 192, true, true);
-      int stage = 0;
-      uint32_t phase = 0;
-      bool ok = true;
-      const bool timed = p.dbg != nullptr;
-      long long t_all = 0, w_full = 0, t0 = 0;
-      unsigned long long ns0 = 0;
-      if (timed) { t_all = clock64(); ns0 = globaltimer_ns(); }
-      for (int kk = 0; kk < num_k; ++kk) {
-        if (timed) t0 = clock64();
-        if (!mbar_wait(full0 + 8 * stage, phase, st, 15)) { ok = false; break; }
-        if (timed) w_full += clock64() - t0;
-        tc_fence_after();
-        const uint32_t sx = smem_base + stage * WG2_STAGE_BYTES;
-        const uint64_t da0 = make_smem_desc_sw128(sx + WG_X_BYTES, WG_DY_BYTES, 1024);
-        const uint32_t first = kk != 0;
-#pragma unroll
-        for (int y = 0; y < WG_TH; ++y) {
-          for (int a = 0; a < nacc; ++a) {
-            // taps (r0 + a, 0..2): three 64-channel blocks one pixel (128 B) apart, 16 pixels of row y as K
-            const uint64_t db = make_smem_desc_sw128(sx + ((r0 + a + y) * WG_PITCH) * 128, 128, 1024);
-            umma_bf16(tmem_base + a * 192, da0 + (uint64_t)((y * WG_TW * 128) >> 4), db, idesc,
-                      first | (uint32_t)(y != 0));
-          }
-        }
-        umma_commit(empty0 + 8 * stage);
-        if (++stage == WG2_STAGES) { stage = 0; phase ^= 1; }
-      }
-      if (ok) umma_commit(tfull);
-      pdl_trigger_late();
-      if (timed) {
-        const int id = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
-        if (id < 1024) {
-          p.dbg[id * 4 + 0] = clock64() - t_all;
-          p.dbg[id * 4 + 1] = w_full;
-          p.dbg[id * 4 + 2] = ((long long)(type_a ? 0 : 1) << 32) | num_k;
-          p.dbg[id * 4 + 3] = (long long)ns0;
-        }
-      }
-    }
-  } else {
-    const int q4 = warp & 3;
-    const int row = q4 * 32 + lane;  // accumulator row = output channel within the 128-block
-    const bool alive = mbar_wait(tfull, 0, st, 16);
-    tc_fence_after();
-    if (alive) {
-      const uint32_t trow = tmem_base + (static_cast<uint32_t>(q4 * 32) << 16);
-      const int ntap = type_a ? 6 : 3;
-      float* obase = (type_a ? p.out_a : p.out_b) + ((long long)zi * p.kd + kdi) * ntap * p.cin * p.cout + nb * 128 + row;
-#pragma unroll 1
-      for (int a = 0; a < nacc; ++a) {
-#pragma unroll 1
-        for (int c = 0; c < 192; c += 32) {
-          uint32_t v[32];
-          tmem_ld_32x32(trow + a * 192 + c, v);
-          tmem_ld_wait();
-          const int tap = a * 3 + c / 64;             // local tap index within this CTA's rows
-          float* o = obase + ((long long)tap * p.cin + cb * 64 + (c & 63)) * p.cout;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) o[(long long)j * p.cout] = num_k ? __uint_as_float(v[j]) : 0.f;
-        }
-      }
-    }
-    tc_fence_before();
-  }
-
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<512>(tmem_base);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------ wgrad, wide, v3
-// Third filter-gradient kernel (cout % 128 == 0). Per-CTA cycle counters in wgrad_halo2_kernel (tools/gpu_conv_bench.py
+// Filter gradient of layers with cout % 128 == 0. wgrad_halo_kernel issues 128 x 64 x 16 UMMAs, whose operand fetch
+// (6 KB per 32 tensor-pipe cycles) saturates the shared-memory read path at ~55 % tensor utilisation
+// (profiles/r01_ncu_full_conv_kernels.txt). Here the roles are swapped: A = dy tile (M = 128 output channels), B = THREE
+// taps of one filter row read from the halo tile as a 192-wide MN-major operand (the 64-element blocks of the descriptor
+// are 128 B = one pixel apart), so one UMMA is 128 x 192 x 16. An earlier version of this kernel (since removed) gave
+// each CTA either filter rows 0, 1 or row 2; per-CTA cycle counters (tools/gpu_conv_bench.py
 // --ops wgrad --waits, profiles/r02_wgrad_class_timing.log) showed its two CTA classes apart: the rows-0,1 class issues a
 // pixel tile's 8 UMMAs (768 tensor cycles) every ~790 cycles, but the row-2 class needs ~630 cycles for 4 UMMAs (384 tensor
 // cycles): a CTA cannot take in more than ~48 B per cycle from L2 (30 KB of operands per tile either way), and the split
@@ -391,14 +218,15 @@ struct WgradHalo3Args {
   DeviceStatus* status;
 };
 
+constexpr int WG3_DY_BYTES = 2 * WG_DY_BYTES;                         // 128 output channels = two 64-channel blocks
 constexpr int WG3_XA_BYTES = 12288;                                  // 18 x 5 pixels x 128 B = 11520, padded to 1024
 constexpr int WG3_XB_BYTES = WG_PITCH * WG_TH * 128;                 // 18 x 4 pixels x 128 B = 9216
-constexpr int WG3_STAGE_A = WG3_XA_BYTES + WG2_DY_BYTES;             // 28672
-constexpr int WG3_STAGE_B = 2 * WG3_XB_BYTES + WG2_DY_BYTES;         // 34816
+constexpr int WG3_STAGE_A = WG3_XA_BYTES + WG3_DY_BYTES;             // 28672
+constexpr int WG3_STAGE_B = 2 * WG3_XB_BYTES + WG3_DY_BYTES;         // 34816
 // Pipeline depth: 8 / 6 stages fit (225 KB), but a CTA that fills the SM's shared memory keeps the HBM-bound passes of
 // the main stream from running beside it (the filter gradient runs on a side stream). Timed alone the kernel is equally
 // fast with 5 .. 8 stages (4 / 3 stages: 5 % slower); 6 / 5 stages = 171 KB leave room for the neighbours
-// (BSL_WG3_STAGES_A / _B; profiles/r02_ab_experiments.md).
+// (profiles/r02_ab_experiments.md).
 constexpr int WG3_MAX_STAGES = 8;
 constexpr int WG3_STAGES_A = 6, WG3_STAGES_B = 5;
 constexpr int wg3_smem_bytes(int sa, int sb) {
@@ -421,7 +249,6 @@ wgrad_halo3_kernel(const __grid_constant__ CUtensorMap tmXa, const __grid_consta
   const uint32_t tfull = smem_u32(&bars[2 * WG3_MAX_STAGES]);
   DeviceStatus* st = p.status;
 
-  pdl_trigger();
   if (threadIdx.x == 0) dead = *reinterpret_cast<volatile int*>(&st->error);
   __syncthreads();
   if (dead) return;
@@ -470,7 +297,7 @@ wgrad_halo3_kernel(const __grid_constant__ CUtensorMap tmXa, const __grid_consta
     if (elect_one_sync()) {
       int stage = 0;
       uint32_t phase = 0;
-      const uint32_t tx_bytes = (type_a ? WG_PITCH * (WG_TH + 1) * 128 : nacc * WG3_XB_BYTES) + WG2_DY_BYTES;
+      const uint32_t tx_bytes = (type_a ? WG_PITCH * (WG_TH + 1) * 128 : nacc * WG3_XB_BYTES) + WG3_DY_BYTES;
       for (int kk = 0; kk < num_k; ++kk) {
         if (!mbar_wait(empty0 + 8 * stage, phase ^ 1, st, 17)) break;
         int t = k_begin + kk;
@@ -527,7 +354,6 @@ wgrad_halo3_kernel(const __grid_constant__ CUtensorMap tmXa, const __grid_consta
         if (++stage == nstage) { stage = 0; phase ^= 1; }
       }
       if (ok) umma_commit(tfull);
-      pdl_trigger_late();
       if (timed && blockIdx.x < 1024) {
         p.dbg[blockIdx.x * 4 + 0] = clock64() - t_all;
         p.dbg[blockIdx.x * 4 + 1] = w_full;
@@ -599,21 +425,11 @@ struct ConvHaloArgs {
   int a_stages;                  // B_RES kernels: activation stages that fit beside the resident filter
   int kd;                        // filter depth (1, or 3 for the (3,3,3) layers of UNet3D): the reduction runs over
   int depth;                     //   (kd, 64-channel block, tap); an "image" is slice z = img % depth of volume img / depth
-  // ---- optional image-slice flags (2-D only): the A producer loads a tile of image i only after
-  //      wait_flags[i / wait_imgs] >= wait_epoch (the pass that writes the A tensor runs beside this kernel)
-  const int* wait_flags;
-  int wait_epoch, wait_imgs;
-  int narrow_store;              // tuning: 128-bit epilogue stores instead of 256-bit (BSL_NARROW_STORE=1)
-  int slow_issue;                // tuning: the generic UMMA issue loop also for 3x3 windows (BSL_SLOW_ISSUE=1)
   // ---- transposed-conv backward-data: the A tensor map is upsampled_map (c, b, w, a, n*h); the reduction runs over
   //      (a = kd index, b, 64-channel block): K block cbx -> a = cbx / cblocks, b = cb / up_cpb, channel (cb % up_cpb) * 64
   int up_cpb;                    // 0 = ordinary (c, x, y, z, vol) coordinates
   long long* dbg;                // tuning (bsl_debug_set key 3): per CTA {total, wait acc_empty, wait a_full, wait b_full}
                                  // cycles of the UMMA issuer thread
-  // ---- optional fused ReluGrad (dgrad into a concat buffer): output columns >= mask_col0 are zeroed where the
-  //      activation stored at the same (pixel, column) of `relu_mask` (same strides as `out`) is not positive
-  const void* relu_mask;
-  int mask_col0;
   // ---- optional per-tap tables (tap_table != 0): one output phase of a STRIDED layer's dgrad is a stride-1 correlation
   //      over dy with a subset of the filter taps -- tap t reads the halo tile at byte offset tap_off[t] and the filter
   //      tap tap_b[kdi * ntaps + t] (conv3d.cu / bsl_conv3d_halo_dgrad_strided)
@@ -652,19 +468,7 @@ constexpr int CH_THREADS = (3 + CH_EPI_WARPS) * 32;
 // 32 fp32 accumulator columns of one pixel row -> 32 bf16 (64 B) in global memory.
 template <bool SCATTER>
 __device__ __forceinline__ void ch_store_chunk(const uint32_t (&v)[32], __nv_bfloat16* o, const float* bias,
-                                               int relu, uint32_t (&packed)[16], int narrow = 0,
-                                               const __nv_bfloat16* mask = nullptr) {
-  uint32_t keep[16];
-  if (mask != nullptr) {   // ReluGrad: keep a gradient only where the stored activation is > 0
-    uint32_t w[16];
-    ld_global_nc_v8(mask, w);          // 2 x 256-bit: whole sectors per lane, as for the stores
-    ld_global_nc_v8(mask + 16, w + 8);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-      const uint32_t lo = w[i] & 0xffffu, hi = w[i] >> 16;
-      keep[i] = ((lo != 0 && lo < 0x8000u) ? 0xffffu : 0u) | ((hi != 0 && hi < 0x8000u) ? 0xffff0000u : 0u);
-    }
-  }
+                                               int relu, uint32_t (&packed)[16]) {
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
     float a = __uint_as_float(v[2 * i]);
@@ -679,9 +483,8 @@ __device__ __forceinline__ void ch_store_chunk(const uint32_t (&v)[32], __nv_bfl
     }
     __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
     packed[i] = *reinterpret_cast<uint32_t*>(&h);
-    if (mask != nullptr) packed[i] &= keep[i];
   }
-  if (!narrow && (reinterpret_cast<uintptr_t>(o) & 31) == 0) {
+  if ((reinterpret_cast<uintptr_t>(o) & 31) == 0) {
     // two 256-bit stores: every lane fills whole 32-byte sectors (lanes of a warp are different pixels, so a
     // 128-bit store would touch 32 sectors and fill half of each)
     st_global_v8(o, packed[0], packed[1], packed[2], packed[3], packed[4], packed[5], packed[6], packed[7]);
@@ -735,7 +538,9 @@ constexpr int CH_MAX_A_STAGES = 4;
 // EVEN CTA's full barriers (cp.async.bulk.tensor.cta_group::2); the issuer's commits arrive on the empty / accumulator
 // barriers of both CTAs (multicast); the peer's epilogue warps arrive on the even CTA's acc_empty barrier through DSMEM.
 template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool B_RES = false, bool TMA_ST = false, bool PAIR = false>
-__global__ void __launch_bounds__(CH_THREADS)
+// One CTA per SM: the shared-memory ring takes the SM anyway; with that bound ptxas keeps the epilogue's accumulator
+// values in registers instead of spilling them.
+__global__ void __launch_bounds__(CH_THREADS, 1)
 conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmO, const ConvHaloArgs p) {
   static_assert(!TMA_ST || (!STATS && !SCATTER && !B_RES), "TMA-store epilogue: plain streamed-filter variant only");
@@ -778,7 +583,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int u_count = PAIR ? p.n_units >> 1 : p.n_units;
   auto pixel_unit = [&](int u) { return PAIR ? 2 * (u / p.n_ntiles) + (int)rank : u / p.n_ntiles; };
 
-  pdl_trigger();
   if (threadIdx.x == 0) dead = *reinterpret_cast<volatile int*>(&st->error);
   if (STATS) {
     for (int i = threadIdx.x; i < CH_EPI_WARPS * 2 * BN; i += CH_THREADS) s_stats[i] = 0.f;
@@ -831,7 +635,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       int stage = 0;
       uint32_t phase = 0;
       bool ok = true;
-      unsigned long long ready = 0;   // image slices already seen complete (wait_flags)
       for (int u = u_first; u < u_count && ok; u += u_step) {
         const int pu = pixel_unit(u);
         int nsub = p.n_sub_total - pu * NSUB;
@@ -844,21 +647,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           s /= p.ntile_w;
           ty[j] = s % p.ntile_h;
           img[j] = s / p.ntile_h;
-        }
-        if (p.wait_flags != nullptr) {
-          bool fresh = false;
-#pragma unroll
-          for (int j = 0; j < NSUB; ++j) {
-            if (j < nsub && ok) {
-              const int f = img[j] / p.wait_imgs;
-              if (!((ready >> f) & 1ull)) {
-                ok = pipe_wait(p.wait_flags + f, p.wait_epoch, st, 28);
-                ready |= 1ull << f;
-                fresh = true;
-              }
-            }
-          }
-          if (fresh) fence_proxy_async_global();
         }
         for (int cbx = 0; cbx < kblocks && ok; ++cbx) {
           if (!mbar_wait(a_empty + 8 * stage, phase ^ 1, st, 21)) { ok = false; break; }
@@ -987,7 +775,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       bool ok = true;
       long long t_all = clock64(), w_acc = 0, w_a = 0, w_b = 0, t0;
       const bool timed = p.dbg != nullptr;
-      const bool fast9 = p.ntaps == 9 && p.halo != 0 && p.tap_table == 0 && p.slow_issue == 0;
+      const bool fast9 = p.ntaps == 9 && p.halo != 0 && p.tap_table == 0;
       const uint64_t db_base = B_MN ? make_smem_desc_sw128(sB0, 8192, 1024) : make_smem_desc_sw128(sB0, 16, 1024);
       if (B_RES && u_first < u_count) ok = mbar_wait(b_full, 0, st, 27);
       for (int u = u_first; u < u_count && ok; u += u_step) {
@@ -1010,7 +798,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             // the halo tile, sub-tile, K slice): ~2.5 instructions per UMMA. The generic loop below spends ~10 (offset
             // arithmetic, parameter loads, vector-to-uniform moves) in this single thread, which bounded the 128-wide tiles
             // (8 UMMAs of 64 cycles per tap): -14 % on those layers, -4 % on the 64-wide, -2 % on the 256-wide ones
-            // (tools/gpu_conv_bench.py, BSL_SLOW_ISSUE=1 for the old loop; profiles/r02_ab_experiments.md).
+            // (tools/gpu_conv_bench.py against the generic loop; profiles/r02_ab_experiments.md).
             const uint64_t da = make_smem_desc_sw128(a_stage, 16, 10 * 128);
             const uint64_t db_res = db_base + (uint64_t)((cb * 9 * B_BYTES) >> 4);
 #pragma unroll
@@ -1073,7 +861,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         if (ok) commit(acc_full + 8 * buf);
         if (++buf == ACC_BUFS) { buf = 0; pacc ^= 1; }
       }
-      pdl_trigger_late();
       if (p.dbg != nullptr) {
         p.dbg[blockIdx.x * 4 + 0] = clock64() - t_all;
         p.dbg[blockIdx.x * 4 + 1] = w_acc;
@@ -1227,10 +1014,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               } else {
                 o = obase + col;
               }
-              const __nv_bfloat16* mk = nullptr;
-              if (!SCATTER && p.relu_mask != nullptr && col >= p.mask_col0)
-                mk = reinterpret_cast<const __nv_bfloat16*>(p.relu_mask) + (o - reinterpret_cast<__nv_bfloat16*>(p.out));
-              if (inside) ch_store_chunk<SCATTER>(hc ? v1 : v0, o, bias, p.relu, packed, p.narrow_store, mk);
+              if (inside) ch_store_chunk<SCATTER>(hc ? v1 : v0, o, bias, p.relu, packed);
             }
           }
         }
@@ -1272,7 +1056,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 tmem_ld_32x32(tq + jj * BN + c, v);
                 tmem_ld_wait();
                 if (inside[jj]) {
-                  ch_store_chunk<false>(v, ob[jj] + c, nullptr, 0, packed, p.narrow_store);
+                  ch_store_chunk<false>(v, ob[jj] + c, nullptr, 0, packed);
                 } else {                         // a row of a ragged edge tile outside the image: no store, no count
 #pragma unroll
                   for (int i = 0; i < 16; ++i) packed[i] = 0u;

@@ -29,7 +29,7 @@ __device__ __forceinline__ long long flipped_index(const Dims& s, long long i, i
 
 // dst[i] = (accumulate ? dst[i] : 0) + src[flip(i)]
 __global__ void flip_f32_kernel(Dims s, int axes, int accumulate, const float* __restrict__ src, float* __restrict__ dst) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const long long total = s.n * s.d * s.h * s.w * s.c;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const float v = src[flipped_index(s, i, axes)];
@@ -40,7 +40,7 @@ __global__ void flip_f32_kernel(Dims s, int axes, int accumulate, const float* _
 template <int C>
 __global__ void tta_finalize_kernel(long long pixels, float count, const float* __restrict__ acc, float* __restrict__ avg,
                                     uint8_t* __restrict__ pred) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < pixels; p += (long long)gridDim.x * blockDim.x) {
     float best = 0.f;
     int arg = 0;
@@ -57,7 +57,7 @@ __global__ void tta_finalize_kernel(long long pixels, float count, const float* 
 // out[0..3] += tp, fp, tn, fn of test = (t == test_value, or t != 0 when test_value < 0) vs ref = (label == ref_value)
 __global__ void confusion_kernel(long long n, const uint8_t* __restrict__ t, int test_value, const int* __restrict__ labels,
                                  int ref_value, unsigned long long* __restrict__ out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   unsigned long long tp = 0, fp = 0, tn = 0, fn = 0;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const bool a = test_value < 0 ? t[i] != 0 : t[i] == test_value;

@@ -59,9 +59,8 @@ int bsl_check_cuda(bsl_ctx* ctx, cudaError_t e, const char* what);
 
 // Kernel launch with the programmatic-stream-serialization attribute (on by default, BSL_PDL=0 turns it off): the grid may be
 // scheduled while the previous kernel of the stream drains. Every kernel launched through here calls
-// bsl::pdl_wait() (or pdl_enter()) before its first access to global data (ptx.cuh).
+// bsl::pdl_wait() before its first access to global data (ptx.cuh).
 bool bsl_pdl_enabled();
-void bsl_pdl_set(int on);
 template <typename... KArgs, typename... Args>
 inline cudaError_t bsl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                               Args&&... args) {
@@ -129,8 +128,5 @@ bool bsl_conv3d_halo_wgrad_ok(const bsl_conv3d_desc* d);
 size_t bsl_conv3d_halo_wgrad_ws(bsl_ctx* ctx, const bsl_conv3d_desc* d);
 int bsl_conv3d_halo_wgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x, const void* dy, float* dw, void* workspace,
                           size_t workspace_bytes, cudaStream_t s);
-
-// Forces the lazily loaded slice-publishing kernels of norm.cu into the context (see the definition).
-void bsl_preload_pipe_kernels();
 
 static inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }

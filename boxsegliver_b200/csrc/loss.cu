@@ -28,7 +28,7 @@ __device__ __forceinline__ double block_sum(double v, double* sm) {
 
 // counts[n][c] = #pixels of image n with label c (labels outside [0, classes) are ignored)
 __global__ void label_counts_kernel(const int* __restrict__ labels, int hw, int classes, int* __restrict__ counts) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ int sc[MAXC];
   if (threadIdx.x < MAXC) sc[threadIdx.x] = 0;
   __syncthreads();
@@ -54,7 +54,7 @@ __global__ void label_counts_kernel(const int* __restrict__ labels, int hw, int 
 // One warp: lane i takes images i, i + 32, ...; the count of weighted pixels is a sum of integers, exact in any order.
 __global__ void weight_table_kernel(bsl_loss_desc d, const int* __restrict__ counts, float* __restrict__ wtab,
                                     double* __restrict__ nz_out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   if (blockIdx.x || threadIdx.x >= 32) return;
   double nz = 0.0;
   for (int img = threadIdx.x; img < d.n; img += 32) {
@@ -128,7 +128,7 @@ template <int C, bool VEC>
 __global__ void wxent_kernel(const float* __restrict__ logits, const int* __restrict__ labels, int hw,
                              long long pixels, const float* __restrict__ wtab, const double* __restrict__ nz_p,
                              float loss_scale, float* __restrict__ dlogits, double* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double sm[32];
   const double nz = *nz_p;
   const float inv_nz = nz > 0.0 ? (float)(1.0 / nz) : 0.f;
@@ -176,7 +176,7 @@ __global__ void wxent_kernel(const float* __restrict__ logits, const int* __rest
 // One warp: lane i adds partials i, i + 32, ... in order, then a fixed xor tree over the lanes.
 __global__ void wxent_final_kernel(const double* __restrict__ part, int blocks, const double* __restrict__ nz_p,
                                    float* __restrict__ loss) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   if (blockIdx.x || threadIdx.x >= 32) return;
   double s = 0.0;
   for (int b = threadIdx.x; b < blocks; b += 32) s += part[b];
@@ -190,7 +190,7 @@ template <int C>
 __global__ void softmax_threshold_kernel(const float* __restrict__ logits, const int* __restrict__ labels, int hw,
                                          long long pixels, float* __restrict__ prob, uint8_t* __restrict__ masks,
                                          uint8_t* __restrict__ argmax, unsigned int* __restrict__ ilr) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long p0 = blockIdx.x * (long long)blockDim.x; p0 < pixels; p0 += stride) {
     const long long p = p0 + threadIdx.x;
@@ -246,7 +246,7 @@ __global__ void softmax_threshold_kernel(const float* __restrict__ logits, const
 template <int C>
 __global__ void dice_reduce_kernel(const float* __restrict__ logits, const int* __restrict__ labels, int hw,
                                    double* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double sm[32];
   const int img = blockIdx.y;
   double ai = 0.0, au = 0.0;
@@ -277,7 +277,7 @@ __global__ void dice_reduce_kernel(const float* __restrict__ logits, const int* 
 // took 0.24 ms at batch 32 -- profiles/r02_ncu_launches_cfg3.txt.)
 __global__ void dice_final_kernel(const double* __restrict__ part, int blocks, int n, float eps,
                                   double* __restrict__ iu, float* __restrict__ loss) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
   for (int img = warp; img < n; img += nwarps) {
     double si = 0.0, su = 0.0;
@@ -307,7 +307,7 @@ template <int C>
 __global__ void dice_bwd_kernel(const float* __restrict__ logits, const int* __restrict__ labels, int hw,
                                 long long pixels, int n, float eps, const double* __restrict__ iu, float loss_scale,
                                 int accumulate, float* __restrict__ dlogits) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < pixels;
        p += (long long)gridDim.x * blockDim.x) {
     float lg[C], pr[C], lse, mx;

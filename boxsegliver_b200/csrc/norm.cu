@@ -18,7 +18,7 @@ namespace bsl {
 // L2 round trips, 41 launches per training step.
 __global__ void __launch_bounds__(1024) pixel_reduce_final_kernel(const float* __restrict__ part, int blocks, int kc,
                                                                   double* __restrict__ out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double sm[32][33];
   const int il = threadIdx.x & 31, q = threadIdx.x >> 5;
   const int i = blockIdx.x * 32 + il;
@@ -187,7 +187,7 @@ __global__ void norm_finalize_kernel(int groups, int c, double m, float eps, flo
                                      float* __restrict__ moving_mean, float* __restrict__ moving_var,
                                      float* __restrict__ mean_o, float* __restrict__ rstd_o,
                                      float* __restrict__ scale_o, float* __restrict__ shift_o) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= groups * c) return;
   const int g = i / c, ch = i - g * c;
@@ -225,8 +225,8 @@ __global__ void norm_apply_kernel(const __nv_bfloat16* __restrict__ y, int y_ld,
                                   int a_ld, long long pixels_per_group, int c, int relu,
                                   const float* __restrict__ scale, const float* __restrict__ shift,
                                   const float* __restrict__ guide, const float* __restrict__ wsp, int wsp_ld,
-                                  int gstride, PipeSignal sig) {
-  bsl::pdl_enter();
+                                  int gstride) {
+  bsl::pdl_wait();
   // blockIdx.y = group (instance norm: gstride = c) or image slice of the batch (batch norm, gstride = 0)
   const int cg = c / 8;
   const int rows = blockDim.x / cg;
@@ -279,7 +279,6 @@ __global__ void norm_apply_kernel(const __nv_bfloat16* __restrict__ y, int y_ld,
     }
     st16(a + (base + p) * a_ld + ch0, pack8(v));
   }
-  if (sig.flags != nullptr) pipe_signal_block(sig, blockIdx.y / sig.imgs_per_slice);
 }
 
 // norm_apply_kernel (no guide) that also evaluates the 1x1 logits convolution on the activation it has just produced
@@ -302,7 +301,7 @@ norm_apply_head_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, __nv_bfloa
                        const float* __restrict__ scale, const float* __restrict__ shift, int gstride,
                        const float* __restrict__ wh, const float* __restrict__ bh,
                        float* __restrict__ logits) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   using HS = HeadSmem<COUT>;
   __shared__ __align__(16) float s_par[32 * HS::LANE];
   const int cg = c / 8;                    // power of two <= 32: the lanes of a pixel sit in one warp
@@ -386,8 +385,8 @@ __global__ void norm_apply_pool_kernel(const __nv_bfloat16* __restrict__ y, int 
                                        int a_ld, __nv_bfloat16* __restrict__ pooled, int p_ld, int h, int w, int c,
                                        int per_sample, int relu, const float* __restrict__ scale,
                                        const float* __restrict__ shift, const float* __restrict__ guide,
-                                       const float* __restrict__ wsp, int wsp_ld, PipeSignal sig) {
-  bsl::pdl_enter();
+                                       const float* __restrict__ wsp, int wsp_ld) {
+  bsl::pdl_wait();
   const int cg = c / 8, ho = h / 2, wo = w / 2;
   const int rows = blockDim.x / cg;
   const int g = threadIdx.x % cg, r = threadIdx.x / cg;
@@ -438,7 +437,6 @@ __global__ void norm_apply_pool_kernel(const __nv_bfloat16* __restrict__ y, int 
     }
     st16(pooled + (out0 + q) * p_ld + ch0, pack8(mx));
   }
-  if (sig.flags != nullptr) pipe_signal_block(sig, img / sig.imgs_per_slice);
 }
 
 // Block = 32 channels x 32 group lanes (instance norm: one group per sample): c1 / c2 per (group, channel) are
@@ -449,7 +447,7 @@ norm_bwd_finalize_kernel(int groups, int c, double m, const double* __restrict__
                          const float* __restrict__ rstd_unused, float* __restrict__ c1,
                          float* __restrict__ c2, float* __restrict__ dgamma,
                          float* __restrict__ dbeta) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double red[2][32][33];
   const int chl = threadIdx.x & 31, gl = threadIdx.x >> 5;
   const int ch = blockIdx.x * 32 + chl;
@@ -488,8 +486,8 @@ __global__ void norm_bwd_apply_kernel(const __nv_bfloat16* __restrict__ y, int y
                                       const float* __restrict__ scale, const float* __restrict__ shift,
                                       const float* __restrict__ c1, const float* __restrict__ c2,
                                       const float* __restrict__ guide, const float* __restrict__ wsp, int wsp_ld,
-                                      int gstride, PipeSignal sig, int premul) {
-  bsl::pdl_enter();
+                                      int gstride, int premul) {
+  bsl::pdl_wait();
   const int cg = c / 8;
   const int rows = blockDim.x / cg;
   const int g = threadIdx.x % cg, r = threadIdx.x / cg;
@@ -553,7 +551,6 @@ __global__ void norm_bwd_apply_kernel(const __nv_bfloat16* __restrict__ y, int y
     }
     st16(dy + (base + p) * dy_ld + ch0, pack8(v));
   }
-  if (sig.flags != nullptr) pipe_signal_block(sig, blockIdx.y / sig.imgs_per_slice);
 }
 
 // GUNet density modulation folded into the per-(sample, channel) affine of an instance-norm layer
@@ -561,7 +558,7 @@ __global__ void norm_bwd_apply_kernel(const __nv_bfloat16* __restrict__ y, int y
 __global__ void norm_modulate_kernel(int n, int c, const float* __restrict__ gamma_mod, int gm_ld,
                                      const float* __restrict__ sp_bias, float* __restrict__ scale,
                                      float* __restrict__ shift) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n * c) return;
   const int s = i / c, ch = i - s * c;
@@ -582,7 +579,7 @@ norm_bwd_finalize_mod_kernel(int n, int c, int K, double m, const double* __rest
                              float* __restrict__ c1, float* __restrict__ c2, float* __restrict__ dgamma,
                              float* __restrict__ dbeta, float* __restrict__ dgamma_mod,
                              float* __restrict__ dw_guide, int dw_ld, float* __restrict__ dbias_guide) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double red[5][FM_S][33];
   const int chl = threadIdx.x & 31, sl = threadIdx.x >> 5;
   const int ch = blockIdx.x * 32 + chl;
@@ -622,7 +619,7 @@ __global__ void norm_affine_fold_kernel(int n, int c, int G, const float* __rest
                                         float* __restrict__ scale, float* __restrict__ shift,
                                         float* __restrict__ scale_pre, float* __restrict__ shift_pre,
                                         const float* __restrict__ w, int w_ld, float* __restrict__ w_eff) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n * c) {
     const int ch = i % c;
@@ -651,7 +648,7 @@ __global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, c
                                                 float* __restrict__ dgamma_mod, float* __restrict__ dw_guide, int dw_ld,
                                                 float* __restrict__ dbias_guide, float* __restrict__ dga,
                                                 float* __restrict__ dba) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int ch = blockIdx.x * blockDim.x + threadIdx.x;
   if (ch >= c) return;
   const double gam = gamma ? (double)gamma[ch] : 1.0, be = beta ? (double)beta[ch] : 0.0, a = (double)ga[ch];
@@ -688,7 +685,7 @@ __global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, c
 __global__ void norm_modulate_bn_kernel(int n, int c, const float* __restrict__ gamma_mod, int gm_ld,
                                         const float* __restrict__ sp_bias, float* __restrict__ mean,
                                         float* __restrict__ rstd, float* __restrict__ scale, float* __restrict__ shift) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int ch = blockIdx.x * blockDim.x + threadIdx.x;
   if (ch >= c) return;
   const float mu = mean[ch], rs = rstd[ch], sc = scale[ch], sh = shift[ch], b = sp_bias ? sp_bias[ch] : 0.f;
@@ -712,7 +709,7 @@ __global__ void norm_bwd_finalize_bnmod_kernel(int n, int c, int K, double m_all
                                                float* __restrict__ c2r, float* __restrict__ dgamma,
                                                float* __restrict__ dbeta, float* __restrict__ dgamma_mod,
                                                float* __restrict__ dw_guide, int dw_ld, float* __restrict__ dbias_guide) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int ch = blockIdx.x * blockDim.x + threadIdx.x;
   if (ch >= c) return;
   const double ga = gamma ? (double)gamma[ch] : 1.0, be = beta ? (double)beta[ch] : 0.0;
@@ -744,7 +741,7 @@ __global__ void maxpool_bwd_add_kernel(const __nv_bfloat16* __restrict__ act, in
                                        const __nv_bfloat16* __restrict__ dpool, int p_ld,
                                        const __nv_bfloat16* __restrict__ dskip, int s_ld,
                                        __nv_bfloat16* __restrict__ out, int o_ld, int n, int h, int w, int c) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int cg = c / 8, ho = h / 2, wo = w / 2;
   const long long total = (long long)n * ho * wo * cg;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
@@ -789,7 +786,7 @@ __global__ void maxpool_bwd_add_kernel(const __nv_bfloat16* __restrict__ act, in
 
 __global__ void relu_bwd_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv_bfloat16* __restrict__ dy,
                                 int dy_ld, __nv_bfloat16* __restrict__ out, int o_ld, long long pixels, int c) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int cg = c / 8;
   const int rows = blockDim.x / cg;
   const int g = threadIdx.x % cg, r = threadIdx.x / cg;
@@ -826,7 +823,7 @@ __global__ void relu_bwd_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, c
 
 __global__ void add_bf16_kernel(const __nv_bfloat16* __restrict__ a, int a_ld, const __nv_bfloat16* __restrict__ b,
                                 int b_ld, __nv_bfloat16* __restrict__ out, int o_ld, long long pixels, int c) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int cg = c / 8;
   const int rows = blockDim.x / cg;
   const int g = threadIdx.x % cg, r = threadIdx.x / cg;
@@ -879,49 +876,7 @@ int check_norm(bsl_ctx* ctx, const bsl_norm_desc* d) {
   return BSL_OK;
 }
 
-// Launch geometry of an apply pass that publishes image slices: grid.y = `gy` entries, `per` of them per slice, and
-// enough blocks per entry that the blocks of one slice fill the GPU (slices then complete one after the other).
-int plan_signal(bsl_ctx* ctx, const bsl_pipe* sg, int n, int gy, unsigned blocks_x, PipeSignal* out) {
-  *out = PipeSignal{nullptr, nullptr, 0, 0, 1};
-  if (!sg) return BSL_OK;
-  if (!sg->flags || !sg->counters || sg->slices < 1 || sg->slices > 64 || n % sg->slices || gy % sg->slices)
-    return bsl_fail(ctx, BSL_EINVAL, "pipe: slices=%d must divide n=%d and be <= 64", sg->slices, n);
-  out->flags = sg->flags;
-  out->counters = sg->counters;
-  out->imgs_per_slice = gy / sg->slices;
-  out->expected = (int)blocks_x * out->imgs_per_slice;
-  out->epoch = sg->epoch;
-  return BSL_OK;
-}
-
-EwPlan ew_plan_sliced(bsl_ctx* ctx, long long pixels_per_entry, int entries_per_slice, int c, int unroll) {
-  EwPlan p = ew_plan(ctx, pixels_per_entry, 1, c, unroll);
-  long long want = (pixels_per_entry + (long long)p.rows * unroll - 1) / ((long long)p.rows * unroll);
-  long long cap = (8LL * ctx->sm_count + entries_per_slice - 1) / entries_per_slice;
-  if (want > cap) want = cap;
-  if (want < 1) want = 1;
-  p.blocks = (unsigned)want;
-  return p;
-}
-
 }  // namespace
-
-// CUDA loads kernels lazily, and the first launch of a function may wait for the device to drain. A pass that
-// publishes image slices (bsl_pipe) is launched while its consumer already spins on the flags, so its code must be
-// resident beforehand: bsl_init calls this once.
-void bsl_preload_pipe_kernels() {
-  cudaFuncAttributes a;
-  cudaFuncGetAttributes(&a, norm_apply_kernel<0>);
-  cudaFuncGetAttributes(&a, norm_apply_kernel<1>);
-  cudaFuncGetAttributes(&a, norm_apply_kernel<2>);
-  cudaFuncGetAttributes(&a, norm_apply_pool_kernel<0>);
-  cudaFuncGetAttributes(&a, norm_apply_pool_kernel<1>);
-  cudaFuncGetAttributes(&a, norm_apply_pool_kernel<2>);
-  cudaFuncGetAttributes(&a, norm_bwd_apply_kernel<0>);
-  cudaFuncGetAttributes(&a, norm_bwd_apply_kernel<1>);
-  cudaFuncGetAttributes(&a, norm_bwd_apply_kernel<2>);
-  (void)cudaGetLastError();
-}
 
 int bsl_stats_bf16(bsl_ctx* ctx, const void* x, long long pixels_per_group, int groups, int c, int ld, double* sums,
                    cudaStream_t stream) {
@@ -973,30 +928,14 @@ static int check_guide(bsl_ctx* ctx, const bsl_norm_desc* d, const bsl_guide* g,
 
 int bsl_norm_apply_mod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const float* scale, const float* shift,
                        const bsl_guide* guide, void* y, void* stream) {
-  return bsl_norm_apply_mod_pipe(ctx, d, x, scale, shift, guide, y, nullptr, stream);
-}
-
-int bsl_norm_apply_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const float* scale,
-                            const float* shift, const bsl_guide* guide, void* y, const bsl_pipe* signal,
-                            void* stream) {
   int rc = check_norm(ctx, d);
   if (rc) return rc;
   if (!x || !scale || !shift || !y) return bsl_fail(ctx, BSL_EINVAL, "norm_apply: null buffer");
   int G;
   if ((rc = check_guide(ctx, d, guide, &G))) return rc;
-  int groups = d->mode ? d->n : 1;
-  long long ppg = d->mode ? d->hw : (long long)d->n * d->hw;
-  EwPlan pl = ew_plan(ctx, ppg, groups, d->c, EW_UNROLL);
-  if (signal) {
-    if (signal->slices < 1 || d->n % signal->slices) return bsl_fail(ctx, BSL_EINVAL, "pipe: bad slice count");
-    if (!d->mode) {            // batch norm: one grid row per image slice, all rows use the batch statistics
-      groups = signal->slices;
-      ppg = (long long)(d->n / signal->slices) * d->hw;
-    }
-    pl = ew_plan_sliced(ctx, ppg, groups / signal->slices, d->c, EW_UNROLL);
-  }
-  PipeSignal sg;
-  if ((rc = plan_signal(ctx, signal, d->n, groups, pl.blocks, &sg))) return rc;
+  const int groups = d->mode ? d->n : 1;
+  const long long ppg = d->mode ? d->hw : (long long)d->n * d->hw;
+  const EwPlan pl = ew_plan(ctx, ppg, groups, d->c, EW_UNROLL);
   const int gstride = d->mode ? d->c : 0;
   const dim3 grid(pl.blocks, groups);
   auto xb = reinterpret_cast<const __nv_bfloat16*>(x);
@@ -1004,13 +943,13 @@ int bsl_norm_apply_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x,
   cudaStream_t s = as_stream(stream);
   if (G == 0)
     bsl_launch(norm_apply_kernel<0>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, ppg, d->c, d->relu, scale, shift,
-                                                     nullptr, nullptr, 0, gstride, sg);
+                                                     nullptr, nullptr, 0, gstride);
   else if (G == 1)
     bsl_launch(norm_apply_kernel<1>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, ppg, d->c, d->relu, scale, shift,
-                                                     guide->map, guide->w, guide->w_ld, gstride, sg);
+                                                     guide->map, guide->w, guide->w_ld, gstride);
   else
     bsl_launch(norm_apply_kernel<2>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, ppg, d->c, d->relu, scale, shift,
-                                                     guide->map, guide->w, guide->w_ld, gstride, sg);
+                                                     guide->map, guide->w, guide->w_ld, gstride);
   BSL_LAUNCH_CHECK(ctx, "norm_apply_kernel");
   return BSL_OK;
 }
@@ -1053,12 +992,6 @@ int bsl_norm_apply(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const fl
 int bsl_norm_apply_pool_mod(bsl_ctx* ctx, const bsl_norm_desc* d, int h, int w, const void* x, const float* scale,
                             const float* shift, const bsl_guide* guide, void* y, void* pooled, int pooled_ld,
                             void* stream) {
-  return bsl_norm_apply_pool_mod_pipe(ctx, d, h, w, x, scale, shift, guide, y, pooled, pooled_ld, nullptr, stream);
-}
-
-int bsl_norm_apply_pool_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, int h, int w, const void* x,
-                                 const float* scale, const float* shift, const bsl_guide* guide, void* y,
-                                 void* pooled, int pooled_ld, const bsl_pipe* signal, void* stream) {
   int rc = check_norm(ctx, d);
   if (rc) return rc;
   if (!x || !scale || !shift || !y || !pooled) return bsl_fail(ctx, BSL_EINVAL, "norm_apply_pool: null buffer");
@@ -1066,13 +999,7 @@ int bsl_norm_apply_pool_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, int h, in
     return bsl_fail(ctx, BSL_EINVAL, "norm_apply_pool: h=%d w=%d must be even and match hw=%d", h, w, d->hw);
   int G;
   if ((rc = check_guide(ctx, d, guide, &G))) return rc;
-  EwPlan pl = ew_plan(ctx, (long long)(h / 2) * (w / 2), d->n, d->c, 1);
-  if (signal) {
-    if (signal->slices < 1 || d->n % signal->slices) return bsl_fail(ctx, BSL_EINVAL, "pipe: bad slice count");
-    pl = ew_plan_sliced(ctx, (long long)(h / 2) * (w / 2), d->n / signal->slices, d->c, 1);
-  }
-  PipeSignal sg;
-  if ((rc = plan_signal(ctx, signal, d->n, d->n, pl.blocks, &sg))) return rc;
+  const EwPlan pl = ew_plan(ctx, (long long)(h / 2) * (w / 2), d->n, d->c, 1);
   const dim3 grid(pl.blocks, d->n);
   auto xb = reinterpret_cast<const __nv_bfloat16*>(x);
   auto yb = reinterpret_cast<__nv_bfloat16*>(y);
@@ -1080,13 +1007,13 @@ int bsl_norm_apply_pool_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, int h, in
   cudaStream_t s = as_stream(stream);
   if (G == 0)
     bsl_launch(norm_apply_pool_kernel<0>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, pb, pooled_ld, h, w, d->c, d->mode,
-                                                          d->relu, scale, shift, nullptr, nullptr, 0, sg);
+                                                          d->relu, scale, shift, nullptr, nullptr, 0);
   else if (G == 1)
     bsl_launch(norm_apply_pool_kernel<1>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, pb, pooled_ld, h, w, d->c, d->mode,
-                                                          d->relu, scale, shift, guide->map, guide->w, guide->w_ld, sg);
+                                                          d->relu, scale, shift, guide->map, guide->w, guide->w_ld);
   else
     bsl_launch(norm_apply_pool_kernel<2>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, yb, d->y_ld, pb, pooled_ld, h, w, d->c, d->mode,
-                                                          d->relu, scale, shift, guide->map, guide->w, guide->w_ld, sg);
+                                                          d->relu, scale, shift, guide->map, guide->w, guide->w_ld);
   BSL_LAUNCH_CHECK(ctx, "norm_apply_pool_kernel");
   return BSL_OK;
 }
@@ -1131,7 +1058,7 @@ norm_bwd_reduce4_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __n
                         const float* __restrict__ scale, const float* __restrict__ shift, int c, int relu,
                         long long pixels_per_group, long long ppb, float* __restrict__ part,
                         const float* __restrict__ dl, const float* __restrict__ wh) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sm[];   // [rows][2][c]
   constexpr int HK = HEAD ? HEAD : 1;
   const int cg = c / 4;
@@ -1247,7 +1174,7 @@ norm_bwd_apply4_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv
                        const float* __restrict__ scale, const float* __restrict__ shift,
                        const float* __restrict__ c1, const float* __restrict__ c2, int gstride,
                        const float* __restrict__ dl, const float* __restrict__ wh) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   constexpr int HK = HEAD ? HEAD : 1;
   const int cg = c / 4;
   const int rows = blockDim.x / cg;
@@ -1343,101 +1270,9 @@ norm_bwd_apply4_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv
   }
 }
 
-// Guided variants of the 4-channels-per-thread backward passes (GUNet's modulated layers, G = 1 or 2 guide channels):
-// z = y * scale + shift + sum_g guide[p][g] * wsp[g][c]; the reduce carries G extra rows sum(dz * guide_g). Same thread
-// layout and partial format as the un-guided kernels ([block][2 + G][c]); 8-byte accesses, <= 64 registers.
-template <int U, int G>
-__global__ void __launch_bounds__(256, 4)
-norm_bwd_reduce4g_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv_bfloat16* __restrict__ da, int da_ld,
-                         const float* __restrict__ mean, const float* __restrict__ rstd,
-                         const float* __restrict__ scale, const float* __restrict__ shift, int c, int relu,
-                         long long pixels_per_group, long long ppb, float* __restrict__ part,
-                         const float* __restrict__ guide, const float* __restrict__ wsp, int wsp_ld) {
-  bsl::pdl_enter();
-  extern __shared__ float sm[];   // [rows][2 + G][c]
-  constexpr int K = 2 + G;
-  const int cg = c / 4;
-  const int rows = blockDim.x / cg;
-  const int g = threadIdx.x % cg, r = threadIdx.x / cg;
-  const int group = blockIdx.y;
-  const int ch0 = g * 4;
-  float acc[K][4];
-#pragma unroll
-  for (int k = 0; k < K; ++k)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[k][j] = 0.f;
-  if (r < rows) {
-    float sc[4], sh[4], rs[4], mr[4], ws[G][4];
-    const int o = group * c + ch0;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      sc[j] = scale[o + j];
-      sh[j] = shift[o + j];
-      rs[j] = rstd[o + j];
-      mr[j] = mean[o + j] * rstd[o + j];
-#pragma unroll
-      for (int q = 0; q < G; ++q) ws[q][j] = wsp[q * wsp_ld + ch0 + j];
-    }
-    const long long p0 = blockIdx.x * ppb, p1 = min(pixels_per_group, p0 + ppb);
-    const long long base = (long long)group * pixels_per_group;
-    auto one = [&](const uint2& ry, const uint2& rd, const float (&gm)[G]) {
-      const __nv_bfloat162* hy = reinterpret_cast<const __nv_bfloat162*>(&ry);
-      const __nv_bfloat162* hd = reinterpret_cast<const __nv_bfloat162*>(&rd);
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const float2 v = __bfloat1622float2(hy[h]), d2 = __bfloat1622float2(hd[h]);
-        const float vv[2] = {v.x, v.y}, dd[2] = {d2.x, d2.y};
-#pragma unroll
-        for (int t = 0; t < 2; ++t) {
-          const int j = 2 * h + t;
-          float z = fmaf(vv[t], sc[j], sh[j]);
-#pragma unroll
-          for (int q = 0; q < G; ++q) z = fmaf(gm[q], ws[q][j], z);
-          const float dz = (!relu || z > 0.f) ? dd[t] : 0.f;
-          const float xh = fmaf(vv[t], rs[j], -mr[j]);
-          acc[0][j] += dz;
-          acc[1][j] = fmaf(dz, xh, acc[1][j]);
-#pragma unroll
-          for (int q = 0; q < G; ++q) acc[2 + q][j] = fmaf(dz, gm[q], acc[2 + q][j]);
-        }
-      }
-    };
-    long long p = p0 + r;
-    for (; p + (long long)(U - 1) * rows < p1; p += (long long)U * rows) {
-      uint2 ry[U], rd[U];
-      float gm[U][G];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const long long px = base + p + (long long)u * rows;
-        ry[u] = *reinterpret_cast<const uint2*>(y + px * y_ld + ch0);
-        rd[u] = *reinterpret_cast<const uint2*>(da + px * da_ld + ch0);
-#pragma unroll
-        for (int q = 0; q < G; ++q) gm[u][q] = __ldg(guide + px * G + q);
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) one(ry[u], rd[u], gm[u]);
-    }
-    for (; p < p1; p += rows) {
-      float gm[G];
-#pragma unroll
-      for (int q = 0; q < G; ++q) gm[q] = __ldg(guide + (base + p) * G + q);
-      one(*reinterpret_cast<const uint2*>(y + (base + p) * y_ld + ch0),
-          *reinterpret_cast<const uint2*>(da + (base + p) * da_ld + ch0), gm);
-    }
-#pragma unroll
-    for (int k = 0; k < K; ++k)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) sm[(r * K + k) * c + ch0 + j] = acc[k][j];
-  }
-  __syncthreads();
-  float* out = part + ((long long)group * gridDim.x + blockIdx.x) * K * c;
-  for (int i = threadIdx.x; i < K * c; i += blockDim.x) {
-    float s = 0.f;
-    for (int rr = 0; rr < rows; ++rr) s += sm[rr * K * c + i];
-    out[i] = s;
-  }
-}
-
+// Guided variant of the 4-channels-per-thread backward apply (GUNet's modulated layers, G = 1 or 2 guide channels):
+// z = y * scale + shift + sum_g guide[p][g] * wsp[g][c]. Same thread layout as the un-guided kernel; 8-byte accesses,
+// <= 64 registers.
 template <int U, int G>
 __global__ void __launch_bounds__(256, 4)
 norm_bwd_apply4g_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv_bfloat16* __restrict__ da, int da_ld,
@@ -1446,7 +1281,7 @@ norm_bwd_apply4g_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __n
                         const float* __restrict__ scale, const float* __restrict__ shift,
                         const float* __restrict__ c1, const float* __restrict__ c2, int gstride,
                         const float* __restrict__ guide, const float* __restrict__ wsp, int wsp_ld) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int cg = c / 4;
   const int rows = blockDim.x / cg;
   const int g = threadIdx.x % cg, r = threadIdx.x / cg;
@@ -1516,34 +1351,6 @@ norm_bwd_apply4g_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __n
   }
 }
 
-// Host side of norm_bwd_reduce4g_kernel: partials [group][block][2 + G][c] -> pixel_reduce_final_kernel -> fp64 sums.
-template <int G>
-int run_bwd_reduce4g(bsl_ctx* ctx, const bsl_norm_desc* d, const __nv_bfloat16* xb, const __nv_bfloat16* db, int dy_ld,
-                     const float* mean, const float* rstd, const float* scale, const float* shift, const bsl_guide* guide,
-                     long long ppg, int groups, double* sums, cudaStream_t stream) {
-  constexpr int K = 2 + G;
-  const int c = d->c, cg = c / 4;
-  int rows = 256 / cg;
-  while ((size_t)rows * K * c * sizeof(float) > 48 * 1024 && rows > 1) rows /= 2;
-  const int threads = rows * cg;
-  long long want = (ppg * c + 32767) / 32768;
-  long long cap = (8LL * ctx->sm_count + groups - 1) / groups;
-  if (want > cap) want = cap;
-  if (want < 1) want = 1;
-  const int blocks = (int)want;
-  const long long ppb = (ppg + blocks - 1) / blocks;
-  float* part = nullptr;
-  int rc = bsl_scratch(ctx, (size_t)groups * blocks * K * c * sizeof(float), &part, stream);
-  if (rc) return rc;
-  const size_t smem = (size_t)rows * K * c * sizeof(float);
-  bsl_launch(norm_bwd_reduce4g_kernel<(G == 1 ? 4 : 2), G>, dim3(blocks, groups), dim3(threads), smem, stream, xb, d->x_ld, db, dy_ld, mean,
-             rstd, scale, shift, c, d->relu, ppg, ppb, part, guide->map, guide->w, guide->w_ld);
-  BSL_LAUNCH_CHECK(ctx, "norm_bwd_reduce4g_kernel");
-  bsl_launch(pixel_reduce_final_kernel, dim3((K * c + 31) / 32, groups), dim3(1024), 0, stream, part, blocks, K * c, sums);
-  BSL_LAUNCH_CHECK(ctx, "pixel_reduce_final_kernel");
-  return BSL_OK;
-}
-
 int run_bwd_reduce4(bsl_ctx* ctx, const bsl_norm_desc* d, const __nv_bfloat16* xb, const __nv_bfloat16* db, int dy_ld,
                     const float* mean, const float* rstd, const float* scale, const float* shift, long long ppg,
                     int groups, double* sums, cudaStream_t stream, const float* dl = nullptr,
@@ -1594,20 +1401,13 @@ int bsl_norm_bwd_reduce_mod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x,
   auto xb = reinterpret_cast<const __nv_bfloat16*>(x);
   auto db = reinterpret_cast<const __nv_bfloat16*>(dy);
   if (G == 0) {
-    static const int slim = getenv("BSL_BWD_REDUCE4") ? atoi(getenv("BSL_BWD_REDUCE4")) : 1;
-    if (slim && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 && dy_ld % 4 == 0)
+    if (d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 && dy_ld % 4 == 0)
       return run_bwd_reduce4(ctx, d, xb, db, dy_ld, mean, rstd, scale, shift, ppg, groups, sums, as_stream(stream));
     BwdFG<0> f{nullptr, nullptr, 0, xb, db, mean, rstd, scale, shift, d->x_ld, dy_ld, d->c, d->relu};
     return run_pixel_reduce(ctx, f, ppg, groups, d->c, sums, as_stream(stream));
   }
-  // measured on cfg3 (8 guided layers per step): 1.50 ms against 1.28 ms for the 8-channel functor below, so the
-  // 4-channel guided reduce stays opt-in (the guided APPLY, norm_bwd_apply4g_kernel, is the one that pays: 3.80 -> 3.45 ms)
-  static const int guide4 = getenv("BSL_BWD_GUIDE4_REDUCE") ? atoi(getenv("BSL_BWD_GUIDE4_REDUCE")) : 0;
-  if (guide4 && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 && dy_ld % 4 == 0) {
-    if (G == 1)
-      return run_bwd_reduce4g<1>(ctx, d, xb, db, dy_ld, mean, rstd, scale, shift, guide, ppg, groups, sums, as_stream(stream));
-    return run_bwd_reduce4g<2>(ctx, d, xb, db, dy_ld, mean, rstd, scale, shift, guide, ppg, groups, sums, as_stream(stream));
-  }
+  // guided layers stay on the 8-channel functor: a 4-channel guided reduce measured 1.50 ms against 1.28 ms on cfg3
+  // (8 guided layers per step); the guided APPLY, norm_bwd_apply4g_kernel, is the one that pays (3.80 -> 3.45 ms)
   if (G == 1) {
     BwdFG<1> f{guide->map, guide->w, guide->w_ld, xb, db, mean, rstd, scale, shift, d->x_ld, dy_ld, d->c, d->relu};
     return run_pixel_reduce(ctx, f, ppg, groups, d->c, sums, as_stream(stream));
@@ -1790,24 +1590,16 @@ int bsl_norm_bwd_finalize_affine(bsl_ctx* ctx, const bsl_norm_desc* d, const dou
   return BSL_OK;
 }
 
+static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
+                               const float* mean, const float* rstd, const float* scale, const float* shift,
+                               const float* c1, const float* c2, const bsl_guide* guide, void* dx, int dx_ld,
+                               void* stream, int premul);
+
 int bsl_norm_bwd_apply_mod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
                            const float* mean, const float* rstd, const float* scale, const float* shift,
                            const float* c1, const float* c2, const bsl_guide* guide, void* dx, int dx_ld,
                            void* stream) {
-  return bsl_norm_bwd_apply_mod_pipe(ctx, d, x, dy, dy_ld, mean, rstd, scale, shift, c1, c2, guide, dx, dx_ld, nullptr,
-                                     stream);
-}
-
-static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
-                               const float* mean, const float* rstd, const float* scale, const float* shift,
-                               const float* c1, const float* c2, const bsl_guide* guide, void* dx, int dx_ld,
-                               const bsl_pipe* signal, void* stream, int premul);
-
-int bsl_norm_bwd_apply_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
-                                const float* mean, const float* rstd, const float* scale, const float* shift,
-                                const float* c1, const float* c2, const bsl_guide* guide, void* dx, int dx_ld,
-                                const bsl_pipe* signal, void* stream) {
-  return norm_bwd_apply_impl(ctx, d, x, dy, dy_ld, mean, rstd, scale, shift, c1, c2, guide, dx, dx_ld, signal, stream, 0);
+  return norm_bwd_apply_impl(ctx, d, x, dy, dy_ld, mean, rstd, scale, shift, c1, c2, guide, dx, dx_ld, stream, 0);
 }
 
 int bsl_norm_bwd_apply_bnmod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
@@ -1816,40 +1608,29 @@ int bsl_norm_bwd_apply_bnmod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x
                              void* stream) {
   if (d && d->mode != 1)
     return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_apply_bnmod: pass the per-sample (mode 1) view of the layer");
-  return norm_bwd_apply_impl(ctx, d, x, dy, dy_ld, mean, rstd, scale, shift, c1r, c2r, guide, dx, dx_ld, nullptr, stream, 1);
+  return norm_bwd_apply_impl(ctx, d, x, dy, dy_ld, mean, rstd, scale, shift, c1r, c2r, guide, dx, dx_ld, stream, 1);
 }
 
 static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,
                                const float* mean, const float* rstd, const float* scale, const float* shift,
                                const float* c1, const float* c2, const bsl_guide* guide, void* dx, int dx_ld,
-                               const bsl_pipe* signal, void* stream, int premul) {
+                               void* stream, int premul) {
   int rc = check_norm(ctx, d);
   if (rc) return rc;
   if (!x || !dy || !mean || !rstd || !scale || !shift || !c1 || !c2 || !dx)
     return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_apply: null buffer");
   int G;
   if ((rc = check_guide(ctx, d, guide, &G))) return rc;
-  int groups = d->mode ? d->n : 1;
-  long long ppg = d->mode ? d->hw : (long long)d->n * d->hw;
-  EwPlan pl = ew_plan(ctx, ppg, groups, d->c, 4);
-  if (signal) {
-    if (signal->slices < 1 || d->n % signal->slices) return bsl_fail(ctx, BSL_EINVAL, "pipe: bad slice count");
-    if (!d->mode) {
-      groups = signal->slices;
-      ppg = (long long)(d->n / signal->slices) * d->hw;
-    }
-    pl = ew_plan_sliced(ctx, ppg, groups / signal->slices, d->c, 4);
-  }
-  PipeSignal sg;
-  if ((rc = plan_signal(ctx, signal, d->n, groups, pl.blocks, &sg))) return rc;
+  const int groups = d->mode ? d->n : 1;
+  const long long ppg = d->mode ? d->hw : (long long)d->n * d->hw;
+  const EwPlan pl = ew_plan(ctx, ppg, groups, d->c, 4);
   const int gstride = d->mode ? d->c : 0;
   const dim3 grid(pl.blocks, groups);
   auto xb = reinterpret_cast<const __nv_bfloat16*>(x);
   auto db = reinterpret_cast<const __nv_bfloat16*>(dy);
   auto ob = reinterpret_cast<__nv_bfloat16*>(dx);
   cudaStream_t s = as_stream(stream);
-  static const int slim = getenv("BSL_BWD_APPLY4") ? atoi(getenv("BSL_BWD_APPLY4")) : 1;
-  if (slim && !premul && G == 0 && !signal && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 &&
+  if (!premul && G == 0 && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 &&
       dy_ld % 4 == 0 && dx_ld % 4 == 0) {
     const int cg4 = d->c / 4, rows4 = 256 / cg4;
     long long want = (ppg + (long long)rows4 * 4 - 1) / ((long long)rows4 * 4);
@@ -1862,8 +1643,7 @@ static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void*
     BSL_LAUNCH_CHECK(ctx, "norm_bwd_apply4_kernel");
     return BSL_OK;
   }
-  static const int guide4 = getenv("BSL_BWD_GUIDE4") ? atoi(getenv("BSL_BWD_GUIDE4")) : 1;
-  if (guide4 && !premul && G > 0 && !signal && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 &&
+  if (!premul && G > 0 && d->c % 4 == 0 && d->c <= 1024 && 256 % (d->c / 4) == 0 && d->x_ld % 4 == 0 &&
       dy_ld % 4 == 0 && dx_ld % 4 == 0) {
     const int cg4 = d->c / 4, rows4 = 256 / cg4;
     long long want = (ppg + (long long)rows4 * 4 - 1) / ((long long)rows4 * 4);
@@ -1881,15 +1661,15 @@ static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void*
   }
   if (G == 0)
     bsl_launch(norm_bwd_apply_kernel<0>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, db, dy_ld, ob, dx_ld, ppg, d->c, d->relu, mean,
-                                                         rstd, scale, shift, c1, c2, nullptr, nullptr, 0, gstride, sg, premul);
+                                                         rstd, scale, shift, c1, c2, nullptr, nullptr, 0, gstride, premul);
   else if (G == 1)
     bsl_launch(norm_bwd_apply_kernel<1>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, db, dy_ld, ob, dx_ld, ppg, d->c, d->relu, mean,
                                                          rstd, scale, shift, c1, c2, guide->map, guide->w, guide->w_ld,
-                                                         gstride, sg, premul);
+                                                         gstride, premul);
   else
     bsl_launch(norm_bwd_apply_kernel<2>, dim3(grid), dim3(pl.threads), 0, s, xb, d->x_ld, db, dy_ld, ob, dx_ld, ppg, d->c, d->relu, mean,
                                                          rstd, scale, shift, c1, c2, guide->map, guide->w, guide->w_ld,
-                                                         gstride, sg, premul);
+                                                         gstride, premul);
   BSL_LAUNCH_CHECK(ctx, "norm_bwd_apply_kernel");
   return BSL_OK;
 }

@@ -17,7 +17,7 @@ __global__ void adam_kernel(float* __restrict__ w, const float* __restrict__ g, 
                             float* __restrict__ v, __nv_bfloat16* __restrict__ shadow, size_t n, float lr_t,
                             float beta1, float beta2, float eps, float l2, float gscale, float decay,
                             double* __restrict__ sq_part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double sm[32];
   double sq = 0.0;
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
@@ -48,7 +48,7 @@ __global__ void adam_kernel(float* __restrict__ w, const float* __restrict__ g, 
 __global__ void momentum_kernel(float* __restrict__ w, const float* __restrict__ g, float* __restrict__ acc,
                                 __nv_bfloat16* __restrict__ shadow, size_t n, float lr, float mom, int nesterov,
                                 float l2, float gscale, double* __restrict__ sq_part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ double sm[32];
   double sq = 0.0;
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
@@ -74,7 +74,7 @@ __global__ void momentum_kernel(float* __restrict__ w, const float* __restrict__
 }
 
 __global__ void sumsq_final_kernel(const double* __restrict__ part, int blocks, double* __restrict__ out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   if (blockIdx.x || threadIdx.x >= 32) return;   // one warp: lane i adds partials i, i + 32, ..., then a fixed xor tree
   double s = 0.0;
   for (int b = threadIdx.x; b < blocks; b += 32) s += part[b];

@@ -17,7 +17,7 @@ inline unsigned grid_for(long long work, int per_block, int cap) {
 
 __global__ void cast_f32_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                      size_t n) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   size_t i = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) * 4;
   const size_t stride = (size_t)gridDim.x * blockDim.x * 4;
   for (; i + 3 < n; i += stride) {
@@ -32,7 +32,7 @@ __global__ void cast_f32_bf16_kernel(const float* __restrict__ src, __nv_bfloat1
 
 __global__ void cast_bf16_f32_kernel(const __nv_bfloat16* __restrict__ src, float* __restrict__ dst,
                                      size_t n) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   size_t i = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) * 4;
   const size_t stride = (size_t)gridDim.x * blockDim.x * 4;
   for (; i + 3 < n; i += stride) {
@@ -46,7 +46,7 @@ __global__ void cast_bf16_f32_kernel(const __nv_bfloat16* __restrict__ src, floa
 }
 
 __global__ void scale_f32_kernel(float* __restrict__ x, size_t n, float a) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
     x[i] *= a;
 }
@@ -54,7 +54,7 @@ __global__ void scale_f32_kernel(float* __restrict__ x, size_t n, float a) {
 // Filter re-layout by index table (UNet3D pixel-pair packing, unet3d_engine.py): dst[i] = bf16(src[idx[i]]) or 0.
 __global__ void gather_f32_bf16_kernel(const float* __restrict__ src, const int* __restrict__ idx, size_t n,
                                        __nv_bfloat16* __restrict__ dst) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     const int j = idx[i];
     dst[i] = __float2bfloat16_rn(j >= 0 ? src[j] : 0.f);
@@ -64,7 +64,7 @@ __global__ void gather_f32_bf16_kernel(const float* __restrict__ src, const int*
 // ... and its adjoint for the gradient: dst[j] = src[idx2[j][0]] + src[idx2[j][1]] (negative index: no term).
 __global__ void gather_add2_f32_kernel(const float* __restrict__ src, const int* __restrict__ idx2, size_t n,
                                        float* __restrict__ dst) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   for (size_t j = blockIdx.x * (size_t)blockDim.x + threadIdx.x; j < n; j += (size_t)gridDim.x * blockDim.x) {
     const int a = idx2[2 * j], b = idx2[2 * j + 1];
     dst[j] = (a >= 0 ? src[a] : 0.f) + (b >= 0 ? src[b] : 0.f);
@@ -74,7 +74,7 @@ __global__ void gather_add2_f32_kernel(const float* __restrict__ src, const int*
 // Statistics of a pixel-pair packed tensor: the conv epilogue sums over 2 * c "super" channels (voxel parity, lane);
 // the real channel's moments are the sum of its two halves. src [groups][2][2c] -> dst [groups][2][c].
 __global__ void fold_pair_sums_kernel(const double* __restrict__ src, int total, int c, double* __restrict__ dst) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int row = i / c, ch = i - row * c;
@@ -126,7 +126,7 @@ struct ReluBiasF {
 };
 
 __global__ void f64_to_f32_kernel(const double* __restrict__ src, float* __restrict__ dst, int n) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) dst[i] = (float)src[i];
 }
@@ -157,7 +157,7 @@ __global__ void __launch_bounds__(256, 4)
 relu_bwd_bias4_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv_bfloat16* __restrict__ dy, int dy_ld,
                       __nv_bfloat16* __restrict__ out, int o_ld, int c, long long pixels, long long ppb,
                       float* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sm[];   // [rows][c]
   const int cg = c / 4;
   const int rows = blockDim.x / cg;
@@ -219,8 +219,7 @@ extern "C" int bsl_relu_bwd_bias(bsl_ctx* ctx, long long pixels, int c, const vo
   if (!y || !dy || !out || !dbias) return bsl_fail(ctx, BSL_EINVAL, "relu_bwd_bias: null buffer");
   if (c % 8 || y_ld % 8 || dy_ld % 8 || out_ld % 8) return bsl_fail(ctx, BSL_EUNSUPPORTED, "relu_bwd_bias: c%%8");
   cudaStream_t s = as_stream(stream);
-  static const int slim = getenv("BSL_RELU_BIAS4") ? atoi(getenv("BSL_RELU_BIAS4")) : 1;
-  if (slim && c <= 1024 && 256 % (c / 4) == 0) {
+  if (c <= 1024 && 256 % (c / 4) == 0) {
     const int cg = c / 4, rows = 256 / cg;
     long long want = (pixels * c + 32767) / 32768;
     const long long cap = 8LL * ctx->sm_count;

@@ -45,33 +45,11 @@ __device__ __forceinline__ bool elect_one_sync() {
 
 // ------------------------------------------------------------------- programmatic dependent launch
 // A kernel enqueued with cudaLaunchAttributeProgrammaticStreamSerialization (bsl_launch, internal.h) may become
-// resident while its predecessor in the stream still runs. pdl_trigger() lets the successor's blocks be scheduled
-// as soon as every block of this grid has called it; pdl_wait() returns once the predecessor grid has completed
+// resident while its predecessor in the stream still runs. pdl_wait() returns once the predecessor grid has completed
 // and its writes are visible. Nothing may read or write global data the predecessor touches before pdl_wait().
-// Both are no-ops in a launch without the attribute.
-#ifndef BSL_PDL_TRIGGER
-#define BSL_PDL_TRIGGER 0
-#endif
-__device__ __forceinline__ void pdl_trigger() {
-#if BSL_PDL_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-// Late trigger (one thread per CTA is enough): issued by the UMMA issuer of the tensor-core kernels once its last
-// accumulator is committed, so the successor's blocks are scheduled, and run their prologue, under the last epilogue.
-#ifndef BSL_PDL_LATE
-#define BSL_PDL_LATE 0
-#endif
-__device__ __forceinline__ void pdl_trigger_late() {
-#if BSL_PDL_LATE
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+// It is a no-op in a launch without the attribute. No kernel issues the early trigger (griddepcontrol.launch_dependents):
+// it made the training step 0.8-1.0 ms slower on B200 (profiles/r01_ab_experiments.md).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_enter() {
-  pdl_trigger();
-  pdl_wait();
-}
 
 // ----------------------------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -128,77 +106,12 @@ __device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, DeviceS
   }
 }
 
-// ----------------------------------------------------------------------------------------- image-slice flags
-// Producer / consumer flags between two kernels that run side by side on different streams (DESIGN.md 3.4): an
-// HBM-bound pass publishes "images [s * k, (s + 1) * k) are written" by storing the step's epoch into flags[s];
-// the TMA producer thread of a tensor-core kernel waits for the slice of the tile it is about to load.
-struct PipeSignal {
-  int* flags;       // [slices] last epoch completed
-  int* counters;    // [slices] arrivals of the current epoch; the last arriver resets it to 0
-  int expected;     // arrivals (thread blocks) per slice
-  int epoch;
-  int imgs_per_slice;
-};
-
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_release_gpu(int* p, int v) {
-  asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-// generic-proxy writes of other SMs (made visible by the acquire above) -> this thread's TMA (async proxy) reads
-__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-
-// Called by every thread of a block after its last global store of the slice.
-__device__ __forceinline__ void pipe_signal_block(const PipeSignal& sg, int slice) {
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const int prev = atomicAdd(&sg.counters[slice], 1);
-    if (prev == sg.expected - 1) {
-      sg.counters[slice] = 0;
-      __threadfence();
-      st_release_gpu(&sg.flags[slice], sg.epoch);
-    }
-  }
-}
-
-// Bounded wait for flags[slice] >= epoch (epochs only grow). Returns false if the pipeline is dead.
-__device__ __forceinline__ bool pipe_wait(const int* flag, int epoch, DeviceStatus* st, int site) {
-  if (ld_acquire_gpu(flag) - epoch >= 0) return true;
-  uint64_t t0 = globaltimer_ns();
-  uint32_t spins = 0;
-  while (true) {
-    if (ld_acquire_gpu(flag) - epoch >= 0) return true;
-    __nanosleep(spins < 8 ? 500 : 2000);   // one poller per CTA; keep the flag's L2 line quiet for the writer
-    if ((++spins & 0x3f) == 0) {
-      if (*reinterpret_cast<volatile int*>(&st->error) != 0) return false;
-      if (globaltimer_ns() - t0 > BSL_WAIT_TIMEOUT_NS) {
-        if (atomicCAS(&st->error, 0, 1) == 0) {
-          st->block = blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z);
-          st->site = site;
-        }
-        return false;
-      }
-    }
-  }
-}
-
 // 256-bit global store (sm_100: STG.E.256), 32-byte aligned address.
 __device__ __forceinline__ void st_global_v8(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint32_t e,
                                              uint32_t f, uint32_t g, uint32_t h) {
   asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d), "r"(e),
                "r"(f), "r"(g), "r"(h)
                : "memory");
-}
-
-// 256-bit read-only global load, 32-byte aligned address.
-__device__ __forceinline__ void ld_global_nc_v8(const void* p, uint32_t* v) {
-  asm volatile("ld.global.nc.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "l"(p));
 }
 
 // ----------------------------------------------------------------------------------------- TMA

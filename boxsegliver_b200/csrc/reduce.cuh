@@ -42,7 +42,7 @@ __device__ __forceinline__ void st16(__nv_bfloat16* p, const uint4& v) { *reinte
 template <class F, int UNROLL>
 __global__ void pixel_reduce_kernel(F f, long long pixels_per_group, long long ppb, int c,
                                     float* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sm[];  // [rows][K][c]
   constexpr int K = F::K;
   constexpr int NIN = F::NIN;

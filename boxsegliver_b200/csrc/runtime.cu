@@ -1,28 +1,21 @@
 // Context, device memory, streams/events/graphs and TMA tensor-map encoding for libbsl_b200.so.
 // This is the part of the boundary the TF wrapper would NOT use (TF owns memory and streams,
 // SURVEY.md section 8b); the ctypes host in boxsegliver_b200/ uses it instead of PyTorch.
-#include <atomic>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstdio>
 #include <cstring>
 #include "internal.h"
 
-// -1 = not read yet; BSL_PDL in the environment sets the initial value, bsl_debug_set(ctx, 4, v) changes it at run time
-// (the engine turns it off for the phases where a second stream shares the SMs, see engine.py).
-// A process-wide tuning knob (bsl_launch has no context argument): atomic, so engines on different threads may flip it
-// without a data race; the launch attribute only changes scheduling, never results.
-static std::atomic<int> g_bsl_pdl{-1};
+// BSL_PDL=0 in the environment turns the launch attribute off for the whole process (read once), the way to isolate a
+// fault from launch overlap; the attribute only changes scheduling, never results.
 bool bsl_pdl_enabled() {
-  int v = g_bsl_pdl.load(std::memory_order_relaxed);
-  if (v < 0) {
+  static const bool on = [] {
     const char* e = getenv("BSL_PDL");
-    v = e ? (atoi(e) != 0) : 1;
-    g_bsl_pdl.store(v, std::memory_order_relaxed);
-  }
-  return v != 0;
+    return e ? atoi(e) != 0 : true;
+  }();
+  return on;
 }
-void bsl_pdl_set(int on) { g_bsl_pdl.store(on ? 1 : 0, std::memory_order_relaxed); }
 
 int bsl_fail(bsl_ctx* ctx, int code, const char* fmt, ...) {
   char buf[512];
@@ -111,7 +104,6 @@ int bsl_init(int device, bsl_ctx** out) {
     delete ctx;
     return BSL_ECUDA;
   }
-  bsl_preload_pipe_kernels();
   *out = ctx;
   return BSL_OK;
 }

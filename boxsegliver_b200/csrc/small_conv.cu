@@ -15,7 +15,7 @@ template <int CIN>
 __global__ void stem_fprop_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                   __nv_bfloat16* __restrict__ y, int y_ld, int n, int h, int wd, int cout, int kh,
                                   int kw) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sw[];  // [taps*CIN][cout]
   const int taps = kh * kw;
   for (int i = threadIdx.x; i < taps * CIN * cout; i += blockDim.x) sw[i] = w[i];
@@ -69,7 +69,7 @@ __global__ void stem_fprop_kernel(const float* __restrict__ x, const float* __re
 constexpr int IM2COL_STRIP = 256;
 __global__ void stem_im2col_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col, int n, int h, int wd,
                                    int cin, int kh, int kw, int cols) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float patch[];  // [kh][strip + kw - 1][cin]
   const int strips = (wd + IM2COL_STRIP - 1) / IM2COL_STRIP;
   const int ph = (kh - 1) / 2, pw = (kw - 1) / 2;
@@ -111,7 +111,7 @@ __global__ void stem_im2col_kernel(const float* __restrict__ x, __nv_bfloat16* _
 template <int CIN>
 __global__ void stem_im2col3_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col, int n, int h, int wd,
                                     int cols) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   constexpr int KW = 3, KH = 3, KCOLS = KH * KW * CIN;
   constexpr int PITCH = (IM2COL_STRIP + KW - 1) * CIN;
   __shared__ float patch[KH * PITCH];
@@ -156,7 +156,7 @@ __global__ void stem_im2col3_kernel(const float* __restrict__ x, __nv_bfloat16* 
 template <int CIN, int KW>
 __global__ void stem_wgrad_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy, int dy_ld, int n,
                                   int h, int wd, int cout, int kh, long long ppb, float* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int lane = threadIdx.x & 31;
   const int cg = threadIdx.x >> 5;  // 8-channel group handled by this warp
   const int groups = cout / 8;
@@ -212,7 +212,7 @@ __global__ void stem_wgrad_kernel(const float* __restrict__ x, const __nv_bfloat
 
 // One warp per output: lane l adds chunks l, l + 32, ... in order (fp64), then a fixed xor tree over the lanes.
 __global__ void sum_chunks_kernel(const float* __restrict__ part, int chunks, int n, float* __restrict__ out) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (i >= n) return;   // warp-uniform
   double s = 0.0;
@@ -227,7 +227,7 @@ __global__ void sum_chunks_kernel(const float* __restrict__ part, int chunks, in
 template <int COUT>
 __global__ void head_fprop_kernel(const __nv_bfloat16* __restrict__ x, int x_ld, const float* __restrict__ w,
                                   const float* __restrict__ bias, float* __restrict__ y, long long pixels, int cin) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sw[];  // [cin][COUT]
   for (int i = threadIdx.x; i < cin * COUT; i += blockDim.x) sw[i] = w[i];
   __syncthreads();
@@ -273,7 +273,7 @@ __global__ void head_fprop_kernel(const __nv_bfloat16* __restrict__ x, int x_ld,
 template <int COUT>
 __global__ void head_dgrad_kernel(const float* __restrict__ dl, const float* __restrict__ w,
                                   __nv_bfloat16* __restrict__ dx, int dx_ld, long long pixels, int cin) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   extern __shared__ float sw[];
   for (int i = threadIdx.x; i < cin * COUT; i += blockDim.x) sw[i] = w[i];
   __syncthreads();
@@ -341,7 +341,7 @@ struct HeadWgradF {
 
 // sums[k*cin + c] (fp64) -> dw[c*COUT + k] (fp32, [1,1,cin,cout] = HWIO)
 __global__ void head_wgrad_finish_kernel(const double* __restrict__ sums, float* __restrict__ dw, int cin, int cout) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= cin * cout) return;
   const int c = i / cout, k = i - c * cout;
@@ -351,7 +351,7 @@ __global__ void head_wgrad_finish_kernel(const double* __restrict__ sums, float*
 // column sums of a dense fp32 [rows][cols] matrix, cols <= 8 (bias gradient of the logits layer)
 __global__ void colsum_partial_kernel(const float* __restrict__ a, long long rows, int cols, long long rpb,
                                       float* __restrict__ part) {
-  bsl::pdl_enter();
+  bsl::pdl_wait();
   __shared__ float sm[8][8];  // [warp][col]
   const long long r0 = blockIdx.x * rpb, r1 = min(rows, r0 + rpb);
   float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};

@@ -16,7 +16,6 @@ Memory plan (all NHWC, bf16 unless noted):
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -207,42 +206,19 @@ class UNetEngine:
         self.comm_stream = None
         self._graph = None
         self._grad_stream = self.stream
-        self._overlap_wgrad = cfg.training and os.environ.get("BSL_WGRAD_OVERLAP", "1") != "0"
-        self._fork_pre = os.environ.get("BSL_WGRAD_FORK", "pre") == "pre"
-        # Programmatic dependent launch (csrc/internal.h bsl_launch): 0 off, 1 every launch (default), 2 only in the
-        # phases where the compute stream has the SMs to itself (forward, loss head, optimizer). Measured on B200
-        # (tools/ab.sh, profiles/r01_ab_experiments.md): the launch attribute alone, every kernel waiting with griddepcontrol.wait before its first
-        # global access, is worth 0.15-0.25 ms per step; an explicit early trigger (BSL_PDL_TRIGGER in ptx.cuh) makes
-        # the step 0.6-0.9 ms SLOWER with or without the filter-gradient stream, so it is compiled out.
-        self._pdl_mode = int(os.environ.get("BSL_PDL", "1"))
+        self._overlap_wgrad = cfg.training
         self._ev_ring, self._ev_ring_i = [ctx.new_event() for _ in range(160)], 0
         if cfg.training:
             self.wg_stream = ctx.new_stream()
             self._dy_events = [ctx.new_event(), ctx.new_event()]
             self._dy_busy = [None, None]
-        # Image-slice pipelining (bsl_pipe, include/bsl_b200.h): the HBM-bound normalisation apply of layer L runs on
-        # `aux_stream` beside the tensor-core kernel that consumes its output (fprop of layer L + 1 / dgrad of layer L),
-        # which loads the tiles of an image only after the apply pass has published that image's slice.
-        # Measured on B200 (profiles/r01_pipe_experiment.md): beside a tcgen05 kernel the apply passes run 2-4x slower
-        # (the UMMA operand fetch saturates the SM's L1 / shared-memory data path that their loads share), so the
-        # step gets SLOWER (23.8 -> 25.1 ms at cfg2); the schedule stays available for experiments, off by default.
-        self._pipe_on = os.environ.get("BSL_PIPE", "0") != "0"
-        # measured: the mask loads in the epilogue cost dgrad +0.45 ms, more than the 0.49 ms relu_bwd pass they replace
-        self._fuse_relu_bwd = os.environ.get("BSL_FUSE_RELU_BWD", "0") != "0"
-        self._fuse_head = os.environ.get("BSL_FUSE_HEAD", "1") != "0"
-        # instance-norm statistics out of the conv epilogue instead of a pass over the conv output (bit-identical outputs)
-        self._fuse_inst_stats = os.environ.get("BSL_FUSE_INST_STATS", "1") != "0"
+        # logits out of the last normalised layer's apply pass (bsl_norm_apply_head) instead of a 1x1 conv over the stored
+        # activation; bit-identical (tests/test_gpu_unet.py compares both ways)
+        self._fuse_head = True
         # backward of the last normalised layer with the logits-layer dgrad recomputed per pixel from dlogits
         # (bsl_norm_bwd_reduce_head / _apply_head) instead of a 128-byte-per-pixel gradient tensor; bit-identical
-        self._fuse_head_bwd = os.environ.get("BSL_FUSE_HEAD_BWD", "1") != "0"
+        self._fuse_head_bwd = True
         self._head_grad = None
-        self.aux_stream = ctx.new_stream()
-        self._pipe_rows = 2 * len(self.layers)
-        self.pipe_buf = self._alloc(2 * self._pipe_rows * 64 * 4).zero()
-        self._pipe_epoch = 0
-        cap = int(os.environ.get("BSL_PIPE_SLICES", "8")) if cfg.normalizer == "batch_norm" else 64
-        self._pipe_slices = max(d for d in range(1, min(cfg.batch, cap) + 1) if cfg.batch % d == 0)
-        self._pending = None
 
     # ------------------------------------------------------------------ per-kernel timing (bench roofline)
     def enable_conv_timing(self, on: bool = True):
@@ -319,12 +295,11 @@ class UNetEngine:
         # the final bucket closes at the stem's filter gradient, the last kernel of backward, and overlaps nothing: a
         # boundary at the first conv of the second level keeps it down to the first level's ~40 K values
         early = next((L.scope for L in self.layers if L.kind == "conv" and L.level == 1), None)
-        split_early = os.environ.get("BSL_BUCKET_EARLY_SPLIT", "1") != "0"
         for L in reversed(self.layers):
             p = self.params[f"{L.scope}/weights"]
             acc = end - p.offset
             last = L
-            full = acc >= self.BUCKET_ELEMS or (split_early and L.scope == early and acc > 0)
+            full = acc >= self.BUCKET_ELEMS or (L.scope == early and acc > 0)
             if full and len(self._bucket_at) < len(self._ev_ready) - 1:
                 self._bucket_at[L.scope] = (p.offset, acc)
                 end, acc = p.offset, 0
@@ -539,7 +514,7 @@ class UNetEngine:
         self.images = self._alloc(n * cfg.height * cfg.width * cfg.channel * F32)
         # im2col rows of the stem: 9 * channels live columns in a pitch of 32 (3 input channels) or 64 columns; the conv
         # kernels read a 32-column matrix as cin = 64 with the upper half zero-filled by TMA (bsl_stem_im2col_ld)
-        sc = int(os.environ.get("BSL_STEM_COLS", "0")) or (32 if 9 * cfg.channel <= 32 else 64)
+        sc = 32 if 9 * cfg.channel <= 32 else 64
         self.stem_cols = sc
         self.stem_col = View(self._alloc(n * cfg.height * cfg.width * sc * BF16), n, cfg.height, cfg.width, sc)
         self.labels = self._alloc(n * cfg.height * cfg.width * 4)
@@ -735,38 +710,9 @@ class UNetEngine:
             self.labels.upload(np.ascontiguousarray(labels, np.int32), stream)
 
     # ------------------------------------------------------------------ forward
-    # ------------------------------------------------------------------ image-slice pipelining
-    def _pipe(self, row: int) -> _lib.Pipe:
-        return _lib.Pipe(self.pipe_buf.ptr + row * 256, self.pipe_buf.ptr + (self._pipe_rows + row) * 256,
-                         self._pipe_slices, self._pipe_epoch)
-
-    def _pipe_active(self) -> bool:
-        return self._pipe_on and self.ctx._prof is None and not getattr(self, "_timing", False)
-
-    @staticmethod
-    def _pipe_shape_ok(L: ConvL) -> bool:
-        """The layer's tensor-core kernel is the halo-tile one (the only kernel that can wait on slices)."""
-        return L.kind in ("conv", "convT") and L.h % 16 == 0 and L.w % 8 == 0
-
-    def _take_pending(self, s):
-        """(pipe to wait on or None, completion callback): the previous layer's apply pass still running on the
-        auxiliary stream. The callback orders the main stream after that pass once the consumer is enqueued."""
-        pend, self._pending = self._pending, None
-        if pend is None:
-            return None, lambda: None
-        pipe, ev = pend
-        return pipe, lambda: self.ctx.call("bsl_stream_wait_event", s, ev)
-
-    def _pdl(self, on: bool):
-        if self._pdl_mode == 2:
-            self.ctx.call("bsl_debug_set", C.c_int(4), C.c_int(1 if on else 0))
-
     def forward(self, is_training: bool):
         ctx, s = self.ctx, self.stream
         call = ctx.call
-        self._pdl(True)
-        self._pipe_epoch += 1
-        piping = self._pipe_active()
         self._head_done = False
         for idx, L in enumerate(self.layers):
             ctx.tag = L.scope
@@ -777,12 +723,12 @@ class UNetEngine:
                 ns = self.norm_scope
                 bn = self.cfg.normalizer == "batch_norm"
                 # batch-norm training: the per-channel sums come out of the conv epilogue (no pass over y); instance norm
-                # (training and inference): per-(sample, channel) sums from the same epilogue (bsl_conv2d_fprop_group_stats)
-                fused = bn and is_training
-                inst = (not bn) and self._fuse_inst_stats
-                fn = "bsl_conv2d_fprop_stats" if fused else "bsl_conv2d_fprop"
-                extra = (q["sums"],) if fused else ()
-                if inst:
+                # (training and inference): per-(sample, channel) sums from the same epilogue (bsl_conv2d_fprop_group_stats);
+                # batch-norm inference normalises with the moving statistics and needs no sums
+                fn, extra = "bsl_conv2d_fprop", ()
+                if bn and is_training:
+                    fn, extra = "bsl_conv2d_fprop_stats", (q["sums"],)
+                elif not bn:
                     fn, extra = "bsl_conv2d_fprop_group_stats", (C.c_int(1), q["sums"])
                 wbf = self._pp(self.Wbf, f"{L.scope}/weights", BF16)
                 if L.kind == "stem":
@@ -791,16 +737,7 @@ class UNetEngine:
                     d1 = _lib.Conv2dDesc(self.cfg.batch, L.h, L.w, 64, L.cout, 1, 1, self.stem_cols, L.y.ld)
                     self._tc("fprop", self._flops(L), fn, C.byref(d1), self.stem_col.p, wbf, L.y.p, *extra, s)
                 else:
-                    pw, done = self._take_pending(s)
-                    if pw is not None:
-                        inst = False
-                        self._tc("fprop", self._flops(L), "bsl_conv2d_fprop_pipe", C.byref(d), L.x.p, wbf, L.y.p,
-                                 q["sums"] if fused else None, C.byref(pw), s)
-                        done()
-                    else:
-                        self._tc("fprop", self._flops(L), fn, C.byref(d), L.x.p, wbf, L.y.p, *extra, s)
-                if not fused and not inst and (not bn or is_training):
-                    call("bsl_norm_stats", C.byref(nd), L.y.p, q["sums"], s)
+                    self._tc("fprop", self._flops(L), fn, C.byref(d), L.x.p, wbf, L.y.p, *extra, s)
                 mm = C.c_void_p(self.S.ptr + self.params[f"{L.scope}/{ns}/moving_mean"].offset * F32) if bn else None
                 mv = C.c_void_p(self.S.ptr + self.params[f"{L.scope}/{ns}/moving_variance"].offset * F32) if bn else None
                 call("bsl_norm_finalize", C.byref(nd), C.c_int(1 if is_training else 0), q["sums"],
@@ -811,15 +748,6 @@ class UNetEngine:
                 nd = self._apply_desc(L, nd)
                 gp = C.byref(guide) if guide is not None else None
                 nxt = self.layers[idx + 1] if idx + 1 < len(self.layers) else None
-                sig, st = None, s
-                if piping and nxt is not None and self._pipe_shape_ok(nxt):
-                    # the apply pass goes to the auxiliary stream and publishes image slices; the next layer's
-                    # tensor-core kernel starts right away on the main stream and follows it slice by slice
-                    sig, st = self._pipe(idx), self.aux_stream
-                    ev = self._next_event()
-                    ctx.record(ev, s)
-                    call("bsl_stream_wait_event", st, ev)
-                sp = C.byref(sig) if sig is not None else None
                 cg = L.cout // 8
                 if (self._fuse_head and nxt is not None and nxt.kind == "logits" and gp is None and L.pooled is None
                         and cg <= 32 and cg & (cg - 1) == 0 and 2 <= self.cfg.num_classes <= 4):
@@ -829,22 +757,15 @@ class UNetEngine:
                          C.c_int(self.cfg.num_classes), self.logits.p, s)
                     self._head_done = True
                 elif L.pooled is not None:
-                    call("bsl_norm_apply_pool_mod_pipe", C.byref(nd), C.c_int(L.h), C.c_int(L.w), src, q["scale"],
-                         q["shift"], gp, L.a.p, L.pooled.p, C.c_int(L.pooled.ld), sp, st)
-                    self._after_pool(L, st)
+                    call("bsl_norm_apply_pool_mod", C.byref(nd), C.c_int(L.h), C.c_int(L.w), src, q["scale"],
+                         q["shift"], gp, L.a.p, L.pooled.p, C.c_int(L.pooled.ld), s)
+                    self._after_pool(L, s)
                 else:
-                    call("bsl_norm_apply_mod_pipe", C.byref(nd), src, q["scale"], q["shift"], gp, L.a.p, sp, st)
-                if sig is not None:
-                    ev = self._next_event()
-                    ctx.record(ev, st)
-                    self._pending = (sig, ev)
+                    call("bsl_norm_apply_mod", C.byref(nd), src, q["scale"], q["shift"], gp, L.a.p, s)
             elif L.kind == "convT":
                 d = self._convT_desc(L)
-                pw, done = self._take_pending(s)
-                self._tc("convT_fwd", self._flops(L), "bsl_convT2d_fwd_pipe", C.byref(d), L.x.p,
-                         self._pp(self.Wbf, f"{L.scope}/weights", BF16), self._pp(self.W, f"{L.scope}/biases"), L.a.p,
-                         C.byref(pw) if pw is not None else None, s)
-                done()
+                self._tc("convT_fwd", self._flops(L), "bsl_convT2d_fwd", C.byref(d), L.x.p,
+                         self._pp(self.Wbf, f"{L.scope}/weights", BF16), self._pp(self.W, f"{L.scope}/biases"), L.a.p, s)
             elif not self._head_done:
                 d = self._conv_desc(L)
                 call("bsl_conv2d_head_fprop", C.byref(d), L.x.p, self._pp(self.W, f"{L.scope}/weights"),
@@ -876,18 +797,16 @@ class UNetEngine:
         call("bsl_norm_bwd_finalize", C.byref(nd), q["sums"], q["c1"], q["c2"],
              self._pp(self.G, f"{L.scope}/{ns}/gamma"), self._pp(self.G, f"{L.scope}/{ns}/beta"), s)
 
-    def _norm_backward_apply(self, L: ConvL, nd, q, cur, oth, stream, sig=None):
-        """Second half: `cur` -> `oth` (gradient w.r.t. the conv output), optionally publishing image slices."""
+    def _norm_backward_apply(self, L: ConvL, nd, q, cur, oth, stream):
+        """Second half: `cur` -> `oth` (gradient w.r.t. the conv output)."""
         if self._head_grad is not None:
             dl, wh, classes = self._head_grad
             self._head_grad = None
-            assert sig is None
             self.ctx.call("bsl_norm_bwd_apply_head", C.byref(nd), L.y.p, dl, wh, C.c_int(classes), q["mean"], q["rstd"],
                           q["scale"], q["shift"], q["c1"], q["c2"], oth.p, C.c_int(L.cout), stream)
             return
-        self.ctx.call("bsl_norm_bwd_apply_mod_pipe", C.byref(nd), L.y.p, cur.p, C.c_int(L.cout), q["mean"], q["rstd"],
-                      q["scale"], q["shift"], q["c1"], q["c2"], None, oth.p, C.c_int(L.cout),
-                      C.byref(sig) if sig is not None else None, stream)
+        self.ctx.call("bsl_norm_bwd_apply_mod", C.byref(nd), L.y.p, cur.p, C.c_int(L.cout), q["mean"], q["rstd"],
+                      q["scale"], q["shift"], q["c1"], q["c2"], None, oth.p, C.c_int(L.cout), stream)
 
     def _norm_backward(self, L: ConvL, nd, q, cur, oth):
         self._norm_backward_reduce(L, nd, q, cur)
@@ -920,11 +839,6 @@ class UNetEngine:
         # overlap); a dY buffer is reused two conv layers later, behind an event.
         cur, alt = self.g1, self.g2
         overlap = self._overlap_wgrad and ctx._prof is None
-        if overlap:
-            self._pdl(False)
-        piping = self._pipe_active()
-        self._pipe_epoch += 1
-        relu_fused = set()      # levels whose transposed-conv ReluGrad was applied by the decoder dgrad's epilogue
         ws = self.wg_stream if overlap else s
         self._grad_stream = ws
         k = 0
@@ -946,7 +860,7 @@ class UNetEngine:
                 call("bsl_conv2d_head_wgrad", C.byref(d), L.x.p, self.dlogits.p, self._pp(self.G, f"{L.scope}/weights"),
                      self._pp(self.G, f"{L.scope}/biases"), ws)
                 prev = self.layers[idx - 1]
-                if (self._fuse_head_bwd and not piping and prev.kind == "conv" and prev.pooled is None
+                if (self._fuse_head_bwd and prev.kind == "conv" and prev.pooled is None
                         and not self._is_modulated(prev) and prev.a is L.x
                         and ctx.lib.bsl_norm_bwd_head_ok(ctx.h, C.byref(self._norm_desc(prev)), C.c_int(L.cout))):
                     # no Conv2DBackpropInput launch: the two normalisation-backward passes of `prev` recompute it
@@ -966,64 +880,28 @@ class UNetEngine:
                 dyb = self.dyb[k]
                 nd = self._norm_desc(L)
                 q = self._norm_ptrs(L)
-                # pipelined: the apply half runs on the auxiliary stream beside dgrad(L), which follows it image slice
-                # by image slice and writes into `alt` (its output must not overwrite the gradient apply still reads)
-                pipe_b = overlap and piping and L.kind == "conv" and self._pipe_shape_ok(L)
                 self._norm_backward_reduce(L, nd, q, cur)
-                sig, ev_apply = None, None
-                if pipe_b:
-                    sig, aux = self._pipe(len(self.layers) + idx), self.aux_stream
-                    ev = self._next_event()
-                    ctx.record(ev, s)
-                    call("bsl_stream_wait_event", aux, ev)
-                    if self._dy_busy[k] is not None:
-                        # on the MAIN stream too: dgrad(L) must not occupy the SMs (spinning on slices) while the
-                        # filter-gradient kernel that still reads this dY buffer waits for shared memory
-                        call("bsl_stream_wait_event", aux, self._dy_busy[k])
-                        call("bsl_stream_wait_event", s, self._dy_busy[k])
-                    self._norm_backward_apply(L, nd, q, cur, dyb, aux, sig)
-                    ev_apply = self._next_event()
-                    ctx.record(ev_apply, aux)
-                else:
-                    if overlap and self._dy_busy[k] is not None:   # the wgrad that read this buffer two layers ago
-                        call("bsl_stream_wait_event", s, self._dy_busy[k])
-                    self._norm_backward_apply(L, nd, q, cur, dyb, s)
+                if overlap and self._dy_busy[k] is not None:   # the wgrad that read this buffer two layers ago
+                    call("bsl_stream_wait_event", s, self._dy_busy[k])
+                self._norm_backward_apply(L, nd, q, cur, dyb, s)
                 # dyb = dY (gradient w.r.t. the conv output), dense with ld = cout
                 d = self._conv_desc(L)
                 d.y_ld = L.cout
                 gw = self._pp(self.G, f"{L.scope}/weights")
-                # dgrad first, on the main stream; the side stream forks AFTER it, so that the filter gradient of this
-                # layer runs beside the HBM-bound normalisation backward of the next one instead of beside dgrad
-                if self._fork_pre:
-                    fork()
+                # the side stream forks before dgrad, so that the filter gradient of this layer runs beside dgrad and the
+                # HBM-bound normalisation backward of the next one
+                fork()
                 if L.kind != "stem" and idx > 0:     # no gradient w.r.t. the network input
                     wbf = self._pp(self.Wbf, f"{L.scope}/weights", BF16)
                     dd = self._conv_desc(L)
                     dd.y_ld = L.cout
-                    wp = C.byref(sig) if sig is not None else None
                     if L.role == "dec1":
                         dc = self.dcat[L.level]
                         dd.x_ld = dc.ld
-                        if self._fuse_relu_bwd and self._pipe_shape_ok(L):
-                            # ReluGrad of the transposed conv (upper channel half of the concat) in the epilogue
-                            up = self.layers[idx - 1]
-                            assert up.kind == "convT" and up.level == L.level
-                            self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad_relu", C.byref(dd), dyb.p, wbf, dc.p,
-                                     self.cat[L.level].p, C.c_int(L.cin - up.cout), wp, s)
-                            relu_fused.add(L.level)
-                        else:
-                            self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad_pipe", C.byref(dd), dyb.p, wbf, dc.p, wp, s)
+                        self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad", C.byref(dd), dyb.p, wbf, dc.p, s)
                     else:
                         dd.x_ld = L.cin_dev or L.cin
-                        dst = alt if pipe_b else cur
-                        self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad_pipe", C.byref(dd), dyb.p, wbf, dst.p, wp, s)
-                        if pipe_b:
-                            cur, alt = alt, cur
-                if ev_apply is not None:
-                    call("bsl_stream_wait_event", s, ev_apply)
-                    call("bsl_stream_wait_event", ws, ev_apply)
-                if not self._fork_pre:
-                    fork()
+                        self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad", C.byref(dd), dyb.p, wbf, cur.p, s)
                 if L.kind == "stem":
                     d1 = _lib.Conv2dDesc(n, L.h, L.w, 64, L.cout, 1, 1, self.stem_cols, L.cout)
                     self._tc("wgrad", self._flops(L), "bsl_conv2d_wgrad", C.byref(d1), self.stem_col.p, dyb.p, gw,
@@ -1039,13 +917,10 @@ class UNetEngine:
             elif L.kind == "convT":
                 dc = self.dcat[L.level]
                 dup = dc.slice(L.cout, L.cout)
-                # ReluGrad in place on the upper half of dcat (unless dgrad's epilogue already applied it)
-                gb = self._pp(self.G, f"{L.scope}/biases")
-                if L.level not in relu_fused:
-                    # ... and the bias gradient (sum over pixels of the masked gradient) from the same pass
-                    call("bsl_relu_bwd_bias", C.c_longlong(L.a.pixels), C.c_int(L.cout), L.a.p, C.c_int(L.a.ld), dup.p,
-                         C.c_int(dup.ld), dup.p, C.c_int(dup.ld), gb, s)
-                    gb = None
+                # ReluGrad in place on the upper half of dcat, and the bias gradient (sum over pixels of the masked
+                # gradient) from the same pass
+                call("bsl_relu_bwd_bias", C.c_longlong(L.a.pixels), C.c_int(L.cout), L.a.p, C.c_int(L.a.ld), dup.p,
+                     C.c_int(dup.ld), dup.p, C.c_int(dup.ld), self._pp(self.G, f"{L.scope}/biases"), s)
                 d = self._convT_desc(L)
                 d.y_ld = dup.ld
                 d.x_ld = L.cin
@@ -1054,7 +929,7 @@ class UNetEngine:
                 fork()
                 d.x_ld = L.x.ld
                 self._tc("convT_wgrad", self._flops(L), "bsl_convT2d_bwd_filter", C.byref(d), L.x.p, dup.p,
-                         self._pp(self.G, f"{L.scope}/weights"), gb,
+                         self._pp(self.G, f"{L.scope}/weights"), None,
                          self.wgrad_ws.p, wsb, ws, stream=ws)
                 self._after_grad(L)
         if overlap:     # join: everything downstream (optimizer, host reads of G) is ordered after the filter gradients
@@ -1065,7 +940,6 @@ class UNetEngine:
 
     # ------------------------------------------------------------------ optimizer
     def optimizer_step(self, lr: float):
-        self._pdl(True)
         self.step_count += 1
         enqueue_optimizer(self, lr)
 

@@ -422,17 +422,16 @@ class GUNetEngine(UNetEngine):
              self._pp(self.G, f"{L.scope}/{ns}/gamma"), self._pp(self.G, f"{L.scope}/{ns}/beta"), dgm, dwg,
              C.c_int(2 * L.cout), dbg, s)
 
-    def _norm_backward_apply(self, L: ConvL, nd, q, cur, oth, stream, sig=None):
+    def _norm_backward_apply(self, L: ConvL, nd, q, cur, oth, stream):
         if self._head_grad is not None:
-            return super()._norm_backward_apply(L, nd, q, cur, oth, stream, sig)
+            return super()._norm_backward_apply(L, nd, q, cur, oth, stream)
         guide = self._guide_struct(L)
         if self._was_dropped(L):
-            assert sig is None
             call, ns = self.ctx.call, self.norm_scope
             T, dT, qn = self.drop[L.scope]["T"], self.drop_grad, self._drop_ptrs(L)
             c = C.c_int(L.cout)
-            call("bsl_norm_bwd_apply_mod_pipe", C.byref(nd), T.p, cur.p, c, q["mean"], q["rstd"], q["scale"], q["shift"],
-                 q["c1"], q["c2"], C.byref(guide) if guide is not None else None, dT.p, c, None, stream)
+            call("bsl_norm_bwd_apply_mod", C.byref(nd), T.p, cur.p, c, q["mean"], q["rstd"], q["scale"], q["shift"],
+                 q["c1"], q["c2"], C.byref(guide) if guide is not None else None, dT.p, c, stream)
             dd = self._drop_desc(L)
             call("bsl_dropout_bf16", C.byref(dd), C.c_longlong(self.cfg.batch * L.h * L.w), c, dT.p, c, dT.p, c, stream)
             ndn = _lib.NormDesc(nd.mode, nd.n, nd.hw, nd.c, nd.x_ld, nd.y_ld, nd.eps, nd.decay, 0, nd.center, nd.scale)
@@ -444,14 +443,13 @@ class GUNetEngine(UNetEngine):
                  qn["c1"], qn["c2"], oth.p, c, stream)
             return
         if self._bn_mod(L):
-            assert sig is None
             self.ctx.call("bsl_norm_bwd_apply_bnmod", C.byref(self._apply_desc(L, nd)), L.y.p, cur.p, C.c_int(L.cout),
                           q["mean"], q["rstd"], q["scale"], q["shift"], q["c1"], q["c2"],
                           C.byref(guide) if guide is not None else None, oth.p, C.c_int(L.cout), stream)
             return
-        self.ctx.call("bsl_norm_bwd_apply_mod_pipe", C.byref(nd), L.y.p, cur.p, C.c_int(L.cout), q["mean"], q["rstd"],
+        self.ctx.call("bsl_norm_bwd_apply_mod", C.byref(nd), L.y.p, cur.p, C.c_int(L.cout), q["mean"], q["rstd"],
                       q["scale"], q["shift"], q["c1"], q["c2"], C.byref(guide) if guide is not None else None, oth.p,
-                      C.c_int(L.cout), C.byref(sig) if sig is not None else None, stream)
+                      C.c_int(L.cout), stream)
 
     def loss_backward(self):
         super().loss_backward()

@@ -200,8 +200,7 @@ class UNet3DEngine:
         self._pair = (cfg.init_channels <= 32 and cfg.width % 16 == 0 and cfg.height % 32 == 0
                       and 9 * cfg.in_channels <= 32 and os.environ.get("BSL_UNET3D_PAIR", "1") != "0")
         # filter gradients on a side stream, as in engine.UNetEngine.loss_backward
-        self._overlap_wgrad = cfg.training and os.environ.get("BSL_WGRAD_OVERLAP", "1") != "0"
-        self._fuse_inst_stats = os.environ.get("BSL_FUSE_INST_STATS", "1") != "0"
+        self._overlap_wgrad = cfg.training
         if cfg.training:
             self.wg_stream = ctx.new_stream()
             self._dy_events = [ctx.new_event(), ctx.new_event()]
@@ -684,26 +683,20 @@ class UNet3DEngine:
                 # per-(volume, channel) statistics come from the conv epilogue: for layers that run as 2-D convolutions over
                 # n*d images a statistics group is the `depth` consecutive images of one volume; pixel-pair packed layers
                 # sum over super channels (voxel parity, lane), folded to the real channels afterwards.
-                fuse = self._fuse_inst_stats
-                sums = self.sums_sup.p if (fuse and L.pair in ("conv", "stem")) else q["sums"]
-                fn = "bsl_conv2d_fprop_group_stats" if fuse else "bsl_conv2d_fprop"
-                extra = (C.c_int(L.dhw[0]), sums) if fuse else ()
+                sums = self.sums_sup.p if L.pair in ("conv", "stem") else q["sums"]
+                depth = C.c_int(L.dhw[0])
                 if L.kind == "stem":
                     d0 = _lib.Conv2dDesc(n * L.dhw[0], L.dhw[1], L.dhw[2], L.cin, 64, 3, 3, L.cin, 64)
                     call("bsl_stem_im2col_ld", C.byref(d0), self.images.p, self.stem_col.p, C.c_int(L.cinp), s)
-                    call(fn, C.byref(self._desc_stem(L)), self.stem_col.p, wbf, L.y.p, *extra, s)
+                    call("bsl_conv2d_fprop_group_stats", C.byref(self._desc_stem(L)), self.stem_col.p, wbf, L.y.p, depth,
+                         sums, s)
                 elif self._is2d(L) and L.pair != "strided":
-                    call(fn, C.byref(self._desc2(L)), L.x.p, wbf, L.y.p, *extra, s)
+                    call("bsl_conv2d_fprop_group_stats", C.byref(self._desc2(L)), L.x.p, wbf, L.y.p, depth, sums, s)
                 else:
                     d3 = self._desc3s(L) if L.pair == "strided" else self._desc3(L)
-                    if fuse:
-                        call("bsl_conv3d_fprop_group_stats", C.byref(d3), L.x.p, wbf, L.y.p, sums, s)
-                    else:
-                        call("bsl_conv3d_fprop", C.byref(d3), L.x.p, wbf, L.y.p, s)
-                if fuse and L.pair in ("conv", "stem"):
+                    call("bsl_conv3d_fprop_group_stats", C.byref(d3), L.x.p, wbf, L.y.p, sums, s)
+                if L.pair in ("conv", "stem"):
                     call("bsl_fold_pair_sums", sums, C.c_int(n), C.c_int(L.coutp), q["sums"], s)
-                if not fuse:
-                    call("bsl_norm_stats", C.byref(nd), L.y.p, q["sums"], s)
                 call("bsl_norm_finalize", C.byref(nd), C.c_int(1 if is_training else 0), q["sums"],
                      self._pp(self.W, f"{L.scope}/InstanceNorm/gamma"), self._pp(self.W, f"{L.scope}/InstanceNorm/beta"),
                      None, None, q["mean"], q["rstd"], q["scale"], q["shift"], s)

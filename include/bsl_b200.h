@@ -111,36 +111,8 @@ typedef struct {
   int y_ld;        /* channel stride of the output buffer (elements), >= cout */
 } bsl_conv2d_desc;
 
-/* Image-slice flags between two kernels that run side by side on different streams. TF's executor starts an op when
- * its whole input tensor is ready (core/estimator.py:756-757 runs one graph); here the HBM-bound normalisation pass
- * that WRITES a tensor and the tensor-core convolution that READS it overlap: the batch is cut into `slices` groups of
- * n / slices consecutive images, the writer stores `epoch` into flags[s] when slice s is complete, and the reader's
- * TMA producer loads a tile of image i only once flags[i / (n / slices)] >= epoch. Results are bit-identical to the
- * un-pipelined calls. `counters` is scratch of the writer ([slices] ints, zero before first use, self-resetting);
- * epochs must grow from one use of the same flags to the next. slices <= 64 and n % slices == 0. */
-typedef struct {
-  int* flags;
-  int* counters;
-  int slices;
-  int epoch;
-} bsl_pipe;
-
 int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x_bf16,
                      const void* w_hwio_bf16, void* y_bf16, void* stream);
-/* 1 when the shape runs on the halo-tile kernel (h % 16 == 0, w % 8 == 0), the only one that can wait on a pipe. */
-int bsl_conv2d_pipe_ok(bsl_ctx* ctx, const bsl_conv2d_desc* d);
-/* bsl_conv2d_fprop[_stats] (sums nullable) whose input x is being written by a *_pipe normalisation pass. */
-int bsl_conv2d_fprop_pipe(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x_bf16, const void* w_hwio_bf16,
-                          void* y_bf16, double* sums, const bsl_pipe* wait, void* stream);
-int bsl_conv2d_dgrad_pipe(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy_bf16, const void* w_hwio_bf16,
-                          void* dx_bf16, const bsl_pipe* wait, void* stream);
-/* dgrad fused with the ReluGrad of the producer of part of its input (decoder conv1 reads concat(skip, up) --
- * NetworksV2/UNet.py:92-94 -- and `up` is the ReLU output of slim.conv2d_transpose): columns >= col0 of dx are
- * zeroed where act (same shape and channel stride as dx, the concat buffer itself) is not > 0, which is
- * bsl_relu_bwd applied in place afterwards, without the extra pass. Halo-tile shapes only (bsl_conv2d_pipe_ok);
- * col0 % 32 == 0; `wait` nullable. */
-int bsl_conv2d_dgrad_relu(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy_bf16, const void* w_hwio_bf16,
-                          void* dx_bf16, const void* act_bf16, int col0, const bsl_pipe* wait, void* stream);
 /* Conv2D fused with the reduction half of FusedBatchNorm (NetworksV2/base.py:154-162): also returns
  * sums[0][c] = sum over (n,h,w) of y, sums[1][c] = sum of y^2 (of the bf16-rounded outputs, fp64), which is
  * exactly what bsl_norm_stats(mode = batch) computes from y in a separate pass. */
@@ -181,8 +153,6 @@ int bsl_convT2d_fwd(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x_bf16,
  * (slim.conv3d_transpose(..., biases_initializer=None), NetworksV2/UNet3D.py:160-163). */
 int bsl_convT2d_fwd_pairs(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x_bf16, const void* w_kkoi_bf16,
                           void* y_bf16, void* stream);
-int bsl_convT2d_fwd_pipe(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* x_bf16, const void* w_kkoi_bf16,
-                         const float* bias_f32, void* y_bf16, const bsl_pipe* wait, void* stream);
 /* dyr must already carry the ReLU mask (dy * (y > 0)); see bsl_relu_bwd. */
 int bsl_convT2d_bwd_data(bsl_ctx* ctx, const bsl_convT2d_desc* d, const void* dyr_bf16,
                          const void* w_kkoi_bf16, void* dx_bf16, void* stream);
@@ -339,18 +309,6 @@ int bsl_norm_apply_pool_mod(bsl_ctx* ctx, const bsl_norm_desc* d, int h, int w, 
 int bsl_norm_apply_head(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x_bf16, const float* scale,
                         const float* shift, void* y_bf16, const float* w_head_f32, const float* b_head_f32,
                         int classes, float* logits_f32, void* stream);
-/* The same passes publishing image slices of their output through `signal` (bsl_pipe above), for a tensor-core
- * kernel that reads the output while the pass is still running. */
-int bsl_norm_apply_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x_bf16, const float* scale,
-                            const float* shift, const bsl_guide* guide, void* y_bf16, const bsl_pipe* signal,
-                            void* stream);
-int bsl_norm_apply_pool_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, int h, int w, const void* x_bf16,
-                                 const float* scale, const float* shift, const bsl_guide* guide, void* y_bf16,
-                                 void* pooled_bf16, int pooled_ld, const bsl_pipe* signal, void* stream);
-int bsl_norm_bwd_apply_mod_pipe(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x_bf16, const void* dy_bf16,
-                                int dy_ld, const float* mean, const float* rstd, const float* scale,
-                                const float* shift, const float* c1, const float* c2, const bsl_guide* guide,
-                                void* dx_bf16, int dx_ld, const bsl_pipe* signal, void* stream);
 /* sums: fp64 [n][2 + guide channels][c] = sum dz, sum dz * xhat, sum dz * guide_g. */
 int bsl_norm_bwd_reduce_mod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x_bf16, const void* dy_bf16, int dy_ld,
                             const float* mean, const float* rstd, const float* scale, const float* shift,

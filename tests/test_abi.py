@@ -23,7 +23,6 @@ def test_struct_layouts_match_header():
     assert C.sizeof(_lib.NormDesc) == 11 * 4
     assert C.sizeof(_lib.LossDesc) == 4 * 4 + 8 * 4 + 2 * 4
     assert C.sizeof(_lib.AdamDesc) == 8 * 4
-    assert C.sizeof(_lib.Pipe) == 2 * 8 + 2 * 4                       # bsl_pipe
     assert C.sizeof(_lib.InputDesc) == 7 * 4 + 2 * 4 + 4 + 2 * 8      # bsl_input_desc (4 bytes of padding before seed)
     assert C.sizeof(_lib.InputParams) == 8 * 8                        # bsl_input_params
 

@@ -366,88 +366,6 @@ def test_casts_roundtrip(ctx):
         b.free()
 
 
-def test_pipelined_apply_and_conv_match_serial(ctx):
-    """bsl_pipe: a normalisation apply pass publishing image slices on one stream, and the tensor-core conv that reads
-    its output following it slice by slice on another stream, give bit-identical results to the serial calls
-    (forward: apply -> fprop[_stats]; backward: bwd_apply -> dgrad)."""
-    import ctypes as C
-    from boxsegliver_b200 import _lib
-    from boxsegliver_b200.device import f32_to_bf16_bits
-    rng = np.random.default_rng(11)
-    n, h, w, c, co = 8, 32, 32, 64, 128
-    y = f32_to_bf16_bits(rng.standard_normal((n, h, w, c)).astype(np.float32))
-    wt = f32_to_bf16_bits((0.05 * rng.standard_normal((3, 3, c, co))).astype(np.float32))
-    scale = (1 + 0.1 * rng.standard_normal(c)).astype(np.float32)
-    shift = (0.1 * rng.standard_normal(c)).astype(np.float32)
-    by, bw, bsc, bsh = (ctx.from_numpy(a) for a in (y, wt, scale, shift))
-    ba = [ctx.alloc(y.nbytes) for _ in range(2)]
-    bo = [ctx.alloc(n * h * w * co * 2) for _ in range(2)]
-    bs = [ctx.alloc(2 * co * 8) for _ in range(2)]
-    flags = ctx.alloc(2 * 64 * 4).zero()
-    aux = ctx.new_stream()
-    nd = _lib.NormDesc(0, n, h * w, c, c, c, 1e-3, 0.999, 1, 1, 1)
-    cd = _lib.Conv2dDesc(n, h, w, c, co, 3, 3, c, co)
-    # serial
-    ctx.call("bsl_norm_apply_mod", C.byref(nd), by.p, bsc.p, bsh.p, None, ba[0].p, ctx.stream)
-    ctx.call("bsl_conv2d_fprop_stats", C.byref(cd), ba[0].p, bw.p, bo[0].p, bs[0].p, ctx.stream)
-    ctx.sync()
-    for epoch, slices in ((1, 4), (2, 8), (3, 1)):
-        ba[1].zero()
-        bo[1].zero()
-        ctx.sync()
-        pipe = _lib.Pipe(flags.ptr, flags.ptr + 256, slices, epoch)
-        # consumer first: it must wait for the producer that is enqueued after it on the other stream
-        ctx.call("bsl_conv2d_fprop_pipe", C.byref(cd), ba[1].p, bw.p, bo[1].p, bs[1].p, C.byref(pipe), ctx.stream)
-        ctx.call("bsl_norm_apply_mod_pipe", C.byref(nd), by.p, bsc.p, bsh.p, None, ba[1].p, C.byref(pipe), aux)
-        ctx.sync(aux)
-        ctx.check_device()
-        assert np.array_equal(ba[0].download(np.uint16, (n, h, w, c)), ba[1].download(np.uint16, (n, h, w, c)))
-        assert np.array_equal(bo[0].download(np.uint16, (n, h, w, co)), bo[1].download(np.uint16, (n, h, w, co)))
-        assert np.array_equal(bs[0].download(np.float64, (2, co)), bs[1].download(np.float64, (2, co)))
-    # instance-norm grouping + pooled output feeding a conv at half resolution
-    nd1 = _lib.NormDesc(1, n, h * w, c, c, c, 1e-6, 0.0, 1, 1, 1)
-    sc_n = ctx.from_numpy(np.tile(scale, (n, 1)) * (1 + 0.01 * np.arange(n, dtype=np.float32)[:, None]))
-    sh_n = ctx.from_numpy(np.tile(shift, (n, 1)))
-    bp = [ctx.alloc(y.nbytes // 4) for _ in range(2)]
-    bq = [ctx.alloc(n * (h // 2) * (w // 2) * co * 2) for _ in range(2)]
-    cd2 = _lib.Conv2dDesc(n, h // 2, w // 2, c, co, 3, 3, c, co)
-    ctx.call("bsl_norm_apply_pool_mod", C.byref(nd1), C.c_int(h), C.c_int(w), by.p, sc_n.p, sh_n.p, None, ba[0].p,
-             bp[0].p, C.c_int(c), ctx.stream)
-    ctx.call("bsl_conv2d_fprop", C.byref(cd2), bp[0].p, bw.p, bq[0].p, ctx.stream)
-    pipe = _lib.Pipe(flags.ptr, flags.ptr + 256, 8, 4)
-    ctx.call("bsl_conv2d_fprop_pipe", C.byref(cd2), bp[1].p, bw.p, bq[1].p, None, C.byref(pipe), ctx.stream)
-    ctx.call("bsl_norm_apply_pool_mod_pipe", C.byref(nd1), C.c_int(h), C.c_int(w), by.p, sc_n.p, sh_n.p, None, ba[1].p,
-             bp[1].p, C.c_int(c), C.byref(pipe), aux)
-    ctx.sync(aux)
-    ctx.check_device()
-    assert np.array_equal(ba[0].download(np.uint16, (n, h, w, c)), ba[1].download(np.uint16, (n, h, w, c)))
-    assert np.array_equal(bq[0].download(np.uint16, (n, h // 2, w // 2, co)),
-                          bq[1].download(np.uint16, (n, h // 2, w // 2, co)))
-    # backward: bwd_apply -> dgrad
-    da = ctx.from_numpy(f32_to_bf16_bits(rng.standard_normal((n, h, w, c)).astype(np.float32)))
-    mean, rstd, c1, c2 = (ctx.from_numpy((0.1 * rng.standard_normal(c)).astype(np.float32) + k) for k in (0, 1, 0, 0))
-    wd = ctx.from_numpy(f32_to_bf16_bits((0.05 * rng.standard_normal((3, 3, co, c))).astype(np.float32)))
-    cd3 = _lib.Conv2dDesc(n, h, w, co, c, 3, 3, co, c)
-    bdx = [ctx.alloc(n * h * w * co * 2) for _ in range(2)]
-    ctx.call("bsl_norm_bwd_apply", C.byref(nd), by.p, da.p, C.c_int(c), mean.p, rstd.p, bsc.p, bsh.p, c1.p, c2.p,
-             ba[0].p, C.c_int(c), ctx.stream)
-    ctx.call("bsl_conv2d_dgrad", C.byref(cd3), ba[0].p, wd.p, bdx[0].p, ctx.stream)
-    pipe = _lib.Pipe(flags.ptr, flags.ptr + 256, 4, 5)
-    ba[1].zero()
-    ctx.sync()
-    ctx.call("bsl_conv2d_dgrad_pipe", C.byref(cd3), ba[1].p, wd.p, bdx[1].p, C.byref(pipe), ctx.stream)
-    ctx.call("bsl_norm_bwd_apply_mod_pipe", C.byref(nd), by.p, da.p, C.c_int(c), mean.p, rstd.p, bsc.p, bsh.p, c1.p,
-             c2.p, None, ba[1].p, C.c_int(c), C.byref(pipe), aux)
-    ctx.sync(aux)
-    ctx.check_device()
-    assert np.array_equal(ba[0].download(np.uint16, (n, h, w, c)), ba[1].download(np.uint16, (n, h, w, c)))
-    assert np.array_equal(bdx[0].download(np.uint16, (n, h, w, co)), bdx[1].download(np.uint16, (n, h, w, co)))
-    with pytest.raises(Exception):
-        bad = _lib.Pipe(flags.ptr, flags.ptr + 256, 3, 6)      # 3 does not divide n = 8
-        ctx.call("bsl_conv2d_dgrad_pipe", C.byref(cd3), ba[1].p, wd.p, bdx[1].p, C.byref(bad), ctx.stream)
-    ctx.sync()
-
-
 def test_relu_bwd_bias_matches_two_passes(ctx):
     """bsl_relu_bwd_bias == bsl_relu_bwd followed by the bias-gradient reduction of bsl_convT2d_bwd_filter: the masked
     gradient bit for bit (also in place, with channel windows of a wider buffer), the bias gradient to fp32 rounding

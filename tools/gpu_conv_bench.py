@@ -4,8 +4,8 @@
 
 One line per (layer, op): ms and algorithmic TFLOP/s (2 * MACs, un-padded). Inputs are random bf16 bits
 replicated on the device; every tensor at the 256^2 levels is larger than L2, and successive reps of
-smaller layers are separated by a write of a 256 MB scratch buffer (L2 flush). Kernel variants are chosen
-with environment variables read by the library (BSL_IGEMM_V1, BSL_HALO_BN, BSL_HALO_NSUB).
+smaller layers are separated by a write of a 256 MB scratch buffer (L2 flush). The library picks the kernel of each
+layer from its shape, as in a training step.
 """
 import argparse
 import ctypes as C

@@ -18,9 +18,8 @@ from boxsegliver_b200.engine import EngineConfig, UNetEngine  # noqa: E402
 ctx = Context(0)
 n, hw = 8, 64
 images, labels = synthetic.make_batch(n, hw, hw, 3, seed=1401)
-names = ["default", "default again", "no overlap", "pipe+head", "relu fused", "no head fusion", "no head bwd"]
-flags = [dict(), dict(), dict(_overlap_wgrad=False), dict(_pipe_on=True), dict(_fuse_relu_bwd=True),
-         dict(_fuse_head=False), dict(_fuse_head_bwd=False)]
+names = ["default", "default again", "no overlap", "no head fusion", "no head bwd"]
+flags = [dict(), dict(), dict(_overlap_wgrad=False), dict(_fuse_head=False), dict(_fuse_head_bwd=False)]
 ref = None
 for name, fl in zip(names, flags):
     eng = UNetEngine(ctx, EngineConfig(batch=n, height=hw, width=hw, weight_decay_rate=1e-5,

@@ -48,5 +48,5 @@ ms = ctx.elapsed_ms(e0, e1) / a.steps
 ctx.check_device()
 fl = eng.step_flops()["fwd" if a.infer else "total"]
 print(json.dumps({"shape": f"{a.batch} x {a.h} x {a.w}", "mode": "inference" if a.infer else "training", "normalizer": a.normalizer,
-                  "ragged": os.environ.get("BSL_HALO_RAGGED", "1"), "ms_per_step": ms, "slices_per_s": a.batch / ms * 1e3,
+                  "ms_per_step": ms, "slices_per_s": a.batch / ms * 1e3,
                   "model_tflops_per_s": fl / ms / 1e9}))

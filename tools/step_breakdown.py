@@ -82,8 +82,7 @@ def alg_bytes(fn, L):
             "bsl_conv2d_head_fprop": n * L.h * L.w * (L.cin * 2 + 4 * L.cout),
             "bsl_conv2d_head_dgrad": n * L.h * L.w * (L.cin * 2 + 4 * L.cout),
             "bsl_norm_bwd_reduce_head": full + px_out * 12, "bsl_norm_bwd_apply_head": 2 * full + px_out * 12,
-            "bsl_norm_bwd_apply_mod_pipe": 3 * full, "bsl_norm_apply_mod_pipe": 2 * full,
-            "bsl_norm_apply_pool_mod_pipe": 2.25 * full, "bsl_relu_bwd_bias": 3 * full,
+            "bsl_norm_bwd_apply_mod": 3 * full, "bsl_relu_bwd_bias": 3 * full,
             "bsl_norm_apply_head": 2 * full + px_out * 12,
             "bsl_conv2d_head_wgrad": n * L.h * L.w * (L.cin * 2 + 4 * L.cout)}.get(fn)
 
