@@ -1301,7 +1301,7 @@ bool d3_stride1(const bsl_conv3d_desc* d) {
 bool bsl_conv3d_halo_ok(const bsl_conv3d_desc* d) { return d3_stride1(d) && halo_eligible(d->w, d->h); }
 
 int bsl_conv3d_halo_fprop(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x, const void* w, void* y,
-                          cudaStream_t stream, double* sums) {
+                          cudaStream_t stream, double* sums, bool per_volume) {
   HaloPlan pl = plan_halo(ctx, d->w, d->h, d->n * d->d, d->cout);
   int res_stages = 0, res_smem = 0;
   const bool res = plan_resident(pl.bn, 9 * d->kd, d->cin / 64, &pl.nsub, &res_stages, &res_smem);
@@ -1326,9 +1326,10 @@ int bsl_conv3d_halo_fprop(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x,
   a.n_total = d->cout;
   a.a_stages = res_stages;
   a.status = ctx->d_status;
-  // instance statistics per (volume, channel): a statistics group is the d slices of one volume
-  return launch_fprop_halo_stats(ctx, pl, res, res_smem, ta, tb, a, sums, d->d, d->n * d->d, d->h, d->w, d->cout, y,
-                                 d->y_ld, stream);
+  // per_volume: instance statistics per (volume, channel), a statistics group is the d slices of one volume;
+  // otherwise batch statistics per channel over all n * d slices
+  return launch_fprop_halo_stats(ctx, pl, res, res_smem, ta, tb, a, sums, per_volume ? d->d : 0, d->n * d->d, d->h, d->w,
+                                 d->cout, y, d->y_ld, stream);
 }
 
 int bsl_conv3d_halo_dgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy, const void* w, void* dx,

@@ -259,6 +259,20 @@ int bsl_conv3d_fprop_group_stats(bsl_ctx* ctx, const bsl_conv3d_desc* d, const v
                         as_stream(stream));
 }
 
+// fprop + per-channel sum and sum of squares of the bf16 outputs over the whole batch (batch norm): the same two paths,
+// with one statistics group.
+int bsl_conv3d_fprop_stats(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x, const void* w, void* y, double* sums,
+                           void* stream) {
+  Geo g;
+  int rc = geometry(ctx, d, &g);
+  if (rc) return rc;
+  if (!x || !w || !y || !sums) return bsl_fail(ctx, BSL_EINVAL, "conv3d_fprop_stats: null buffer");
+  if (bsl_conv3d_halo_ok(d)) return bsl_conv3d_halo_fprop(ctx, d, x, w, y, as_stream(stream), sums, false);
+  if ((rc = bsl_conv3d_fprop(ctx, d, x, w, y, stream))) return rc;
+  return bsl_stats_bf16(ctx, y, (long long)d->n * g.out[0] * g.out[1] * g.out[2], 1, d->cout, d->y_ld, sums,
+                        as_stream(stream));
+}
+
 int bsl_conv3d_dgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy, const void* w, void* dx, void* stream) {
   Geo g;
   int rc = geometry(ctx, d, &g);

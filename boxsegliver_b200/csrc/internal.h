@@ -121,8 +121,9 @@ bool bsl_conv3d_halo_ok(const bsl_conv3d_desc* d);
 bool bsl_conv3d_halo_dgrad_strided_ok(const bsl_conv3d_desc* d);
 int bsl_conv3d_halo_dgrad_strided(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy, const void* w, void* dx,
                                   cudaStream_t s);
+// sums (nullable): fp64 [n][2][cout] per (volume, channel) when per_volume, else [2][cout] over the whole batch.
 int bsl_conv3d_halo_fprop(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x, const void* w, void* y, cudaStream_t s,
-                          double* sums = nullptr);
+                          double* sums = nullptr, bool per_volume = true);
 int bsl_conv3d_halo_dgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy, const void* w, void* dx, cudaStream_t s);
 bool bsl_conv3d_halo_wgrad_ok(const bsl_conv3d_desc* d);
 size_t bsl_conv3d_halo_wgrad_ws(bsl_ctx* ctx, const bsl_conv3d_desc* d);

@@ -4,6 +4,9 @@ Mirrors /root/reference/NetworksV2/UNet3D.py:31-202: conv3d + instance-norm + Re
 (3,3,3), strided-conv down-sampling ((1,2,2), bridge (2,2,2)), bias-free conv3d_transpose + ReLU up-sampling, skip
 concat [encoder, up], 1x1x1 logits, weighted cross-entropy. What differs from the 2-D engine:
 
+  * --normalizer batch_norm (slim.batch_norm, eps 1e-3, decay 0.999) or instance_norm; batch statistics are per
+    channel over all n*d*h*w voxels of the replica's batch, the moving statistics live in their own arena (region S)
+    padded like gamma / beta, and eval-mode forwards normalise with them;
   * activations are NDHWC bf16; (1,3,3)/stride-1 layers run as 2-D convolutions over n*d images on the halo-tile
     kernels, everything else goes through bsl_conv3d_* / bsl_convT3d_* (csrc/conv3d.cu);
   * UNet3D's channel counts (30, 60, 120, 240, 320) are stored zero-padded to multiples of 64 (64, 64, 128, 256, 320)
@@ -72,6 +75,8 @@ class UNet3DConfig:
     adamw_weight_decay: float = None
     weight_init: str = "xavier"
     in_eps: float = 1e-6
+    bn_eps: float = 1e-3               # slim.batch_norm defaults (BaseNet._get_normalization)
+    bn_decay: float = 0.999
     training: bool = True
     world: int = 1
 
@@ -150,7 +155,7 @@ class Param3:
     layer: Layer3 = None
     offset: int = 0
     size: int = 0             # stored elements
-    region: str = "A"
+    region: str = "A"         # "A" regularised, "B" not, "S" moving statistics (not trained)
 
 
 def _cp(c):
@@ -177,8 +182,10 @@ def _model_config(pools: int):
 class UNet3DEngine:
     def __init__(self, ctx: Context, cfg: UNet3DConfig):
         self.ctx, self.cfg = ctx, cfg
-        if cfg.normalizer != "instance_norm":
-            raise NotImplementedError("UNet3D engine: --normalizer instance_norm (what the shipped 3-D scripts use)")
+        if cfg.normalizer not in ("batch_norm", "instance_norm"):
+            raise ValueError("Not supported normalization function: " + cfg.normalizer)
+        self.bn = cfg.normalizer == "batch_norm"
+        self.norm_scope = "BatchNorm" if self.bn else "InstanceNorm"
         if "xentropy" not in cfg.loss_type:
             raise ValueError("Not supported loss_type: {}".format(cfg.loss_type))   # UNet3D.py:198-199
         if cfg.loss_weight_type not in ("none", "numerical", "proportion"):
@@ -286,8 +293,12 @@ class UNet3DEngine:
             if L.kind in ("stem", "conv"):
                 ps = (L.cinp, L.coutp) if L.kind == "stem" else L.k + (L.cinp, L.coutp)
                 plist.append(Param3(f"{L.scope}/weights", L.k + (L.cin, L.cout), ps, L))
-                plist.append(Param3(f"{L.scope}/InstanceNorm/gamma", (L.cout,), (L.coutp,), L, region="B"))
-                plist.append(Param3(f"{L.scope}/InstanceNorm/beta", (L.cout,), (L.coutp,), L, region="B"))
+                ns = f"{L.scope}/{self.norm_scope}"
+                plist.append(Param3(f"{ns}/gamma", (L.cout,), (L.coutp,), L, region="B"))
+                plist.append(Param3(f"{ns}/beta", (L.cout,), (L.coutp,), L, region="B"))
+                if self.bn:
+                    plist.append(Param3(f"{ns}/moving_mean", (L.cout,), (L.coutp,), L, region="S"))
+                    plist.append(Param3(f"{ns}/moving_variance", (L.cout,), (L.coutp,), L, region="S"))
             elif L.kind == "convT":
                 plist.append(Param3(f"{L.scope}/weights", L.k + (L.cout, L.cin), L.k + (L.coutp, L.cinp), L))
             else:
@@ -303,9 +314,17 @@ class UNet3DEngine:
             if region == "A":
                 self.n_reg = off
         self.n_train = off
+        soff = 0
+        for p in plist:
+            if p.region == "S":
+                p.size = int(np.prod(p.pshape))
+                p.offset = soff
+                soff += _align(p.size)
+        self.n_stats = soff
         self.params = {p.name: p for p in plist}
         self.W = self._alloc(self.n_train * F32)
         self.Wbf = self._alloc(self.n_train * BF16)
+        self.S = self._alloc(max(self.n_stats, 1) * F32)
         if cfg.training:
             self.G = self._alloc(self.n_train * F32).zero()
             self.M = self._alloc(self.n_train * F32).zero()
@@ -520,9 +539,10 @@ class UNet3DEngine:
         return _lib.ConvT3dDesc(self.cfg.batch, L.dhw[0], L.dhw[1], L.dhw[2], L.cinp, L.coutp, L.s[0], L.x.ld, L.a.ld, 1)
 
     def _norm_desc(self, L: Layer3):
+        cfg = self.cfg
         a_ld = L.coutp if isinstance(L.a, PairView) else L.a.ld     # (the pair view is written by two half calls)
-        return _lib.NormDesc(1, self.cfg.batch, int(np.prod(L.odhw)), L.coutp, L.y.ld, a_ld, self.cfg.in_eps, 0.0,
-                             1, 1, 1)
+        return _lib.NormDesc(0 if self.bn else 1, cfg.batch, int(np.prod(L.odhw)), L.coutp, L.y.ld, a_ld,
+                             cfg.bn_eps if self.bn else cfg.in_eps, cfg.bn_decay if self.bn else 0.0, 1, 1, 1)
 
     def _norm_ptrs(self, L: Layer3):
         n = _align(self.cfg.batch * L.coutp, 16)
@@ -578,35 +598,41 @@ class UNet3DEngine:
         return a[:p.shape[0]].copy()
 
     def set_weights(self, weights: dict):
+        """Trainable variables and (batch norm) moving statistics, TF-shaped."""
         host = np.zeros(self.n_train, np.float32)
+        hostS = np.zeros(max(self.n_stats, 1), np.float32)
         for name, p in self.params.items():
             if name not in weights:
                 raise KeyError(f"missing variable {name}")
             a = np.asarray(weights[name], np.float32)
             if tuple(a.shape) != tuple(p.shape):
                 raise ValueError(f"{name}: shape {a.shape} != {p.shape}")
-            host[p.offset:p.offset + p.size] = self._pack(p, a).ravel()
+            (hostS if p.region == "S" else host)[p.offset:p.offset + p.size] = self._pack(p, a).ravel()
         self.W.upload(host)
         self.Wbf.upload(f32_to_bf16_bits(host))
+        self.S.upload(hostS)
 
     def get_weights(self) -> dict:
         host = self.W.download(np.float32, (self.n_train,))
-        return {name: self._unpack(p, host) for name, p in self.params.items()}
+        hostS = self.S.download(np.float32, (max(self.n_stats, 1),))
+        return {name: self._unpack(p, hostS if p.region == "S" else host) for name, p in self.params.items()}
 
     def get_grads(self) -> dict:
         host = self.G.download(np.float32, (self.n_train,))
-        return {name: self._unpack(p, host) for name, p in self.params.items()}
+        return {name: self._unpack(p, host) for name, p in self.params.items() if p.region != "S"}
 
     def get_slots(self) -> dict:
         """Optimizer slots in TF variable shapes (un-padded, [encoder | up] channel order): {name: (m, v)} / {name: (acc,)}."""
         arenas = [self.M.download(np.float32, (self.n_train,))]
         if self.V is not None:
             arenas.append(self.V.download(np.float32, (self.n_train,)))
-        return {name: tuple(self._unpack(p, a) for a in arenas) for name, p in self.params.items()}
+        return {name: tuple(self._unpack(p, a) for a in arenas) for name, p in self.params.items() if p.region != "S"}
 
     def set_slots(self, slots: dict):
         arenas = [np.zeros(self.n_train, np.float32) for _ in range(2 if self.V is not None else 1)]
         for name, p in self.params.items():
+            if p.region == "S":
+                continue
             if name not in slots:
                 raise KeyError(f"missing optimizer slots of {name}")
             for dst, a in zip(arenas, slots[name]):
@@ -630,7 +656,7 @@ class UNet3DEngine:
                 else:
                     lim = np.sqrt(6.0 / (rf * shp[3] + rf * shp[4]))
                     w[name] = rng.uniform(-lim, lim, size=shp).astype(np.float32)
-            elif name.endswith("gamma"):
+            elif name.endswith(("gamma", "moving_variance")):
                 w[name] = np.ones(shp, np.float32)
             else:
                 w[name] = np.zeros(shp, np.float32)
@@ -675,34 +701,46 @@ class UNet3DEngine:
         call = ctx.call
         n = cfg.batch
         self._pack_super_filters()
+        # statistics come from the conv epilogue: per (volume, channel) for instance norm -- for layers that run as 2-D
+        # convolutions over n*d images a statistics group is the `depth` consecutive images of one volume -- and per
+        # channel over the whole batch for batch norm in training; batch-norm inference normalises with the moving
+        # statistics and needs no sums. Pixel-pair packed layers sum over super channels (voxel parity, lane), folded to
+        # the real channels afterwards.
+        if self.bn and not is_training:
+            conv2, conv3 = "bsl_conv2d_fprop", "bsl_conv3d_fprop"
+        elif self.bn:
+            conv2, conv3 = "bsl_conv2d_fprop_stats", "bsl_conv3d_fprop_stats"
+        else:
+            conv2, conv3 = "bsl_conv2d_fprop_group_stats", "bsl_conv3d_fprop_group_stats"
+        with_sums = is_training or not self.bn
         for L in self.layers:
             ctx.tag = L.scope
             if L.kind in ("stem", "conv"):
                 wbf = self._wsup(L) if L.pair else self._pp(self.Wbf, f"{L.scope}/weights", BF16)
                 nd, q = self._norm_desc(L), self._norm_ptrs(L)
-                # per-(volume, channel) statistics come from the conv epilogue: for layers that run as 2-D convolutions over
-                # n*d images a statistics group is the `depth` consecutive images of one volume; pixel-pair packed layers
-                # sum over super channels (voxel parity, lane), folded to the real channels afterwards.
                 sums = self.sums_sup.p if L.pair in ("conv", "stem") else q["sums"]
-                depth = C.c_int(L.dhw[0])
+                extra3 = (sums,) if with_sums else ()
+                extra2 = ((sums,) if self.bn else (C.c_int(L.dhw[0]), sums)) if with_sums else ()
                 if L.kind == "stem":
                     d0 = _lib.Conv2dDesc(n * L.dhw[0], L.dhw[1], L.dhw[2], L.cin, 64, 3, 3, L.cin, 64)
                     call("bsl_stem_im2col_ld", C.byref(d0), self.images.p, self.stem_col.p, C.c_int(L.cinp), s)
-                    call("bsl_conv2d_fprop_group_stats", C.byref(self._desc_stem(L)), self.stem_col.p, wbf, L.y.p, depth,
-                         sums, s)
+                    call(conv2, C.byref(self._desc_stem(L)), self.stem_col.p, wbf, L.y.p, *extra2, s)
                 elif self._is2d(L) and L.pair != "strided":
-                    call("bsl_conv2d_fprop_group_stats", C.byref(self._desc2(L)), L.x.p, wbf, L.y.p, depth, sums, s)
+                    call(conv2, C.byref(self._desc2(L)), L.x.p, wbf, L.y.p, *extra2, s)
                 else:
                     d3 = self._desc3s(L) if L.pair == "strided" else self._desc3(L)
-                    call("bsl_conv3d_fprop_group_stats", C.byref(d3), L.x.p, wbf, L.y.p, sums, s)
-                if L.pair in ("conv", "stem"):
-                    call("bsl_fold_pair_sums", sums, C.c_int(n), C.c_int(L.coutp), q["sums"], s)
+                    call(conv3, C.byref(d3), L.x.p, wbf, L.y.p, *extra3, s)
+                if with_sums and L.pair in ("conv", "stem"):
+                    call("bsl_fold_pair_sums", sums, C.c_int(1 if self.bn else n), C.c_int(L.coutp), q["sums"], s)
+                ns = f"{L.scope}/{self.norm_scope}"
+                mm = self._pp(self.S, f"{ns}/moving_mean") if self.bn else None
+                mv = self._pp(self.S, f"{ns}/moving_variance") if self.bn else None
                 call("bsl_norm_finalize", C.byref(nd), C.c_int(1 if is_training else 0), q["sums"],
-                     self._pp(self.W, f"{L.scope}/InstanceNorm/gamma"), self._pp(self.W, f"{L.scope}/InstanceNorm/beta"),
-                     None, None, q["mean"], q["rstd"], q["scale"], q["shift"], s)
+                     self._pp(self.W, f"{ns}/gamma"), self._pp(self.W, f"{ns}/beta"), mm, mv, q["mean"], q["rstd"],
+                     q["scale"], q["shift"], s)
                 if isinstance(L.a, PairView):
                     # even / odd voxels of the dense 32-lane tensor -> the two 32-lane quarters of the encoder half
-                    ndh = _lib.NormDesc(1, n, nd.hw // 2, 32, 64, L.a.ld, cfg.in_eps, 0.0, 1, 1, 1)
+                    ndh = _lib.NormDesc(nd.mode, n, nd.hw // 2, 32, 64, L.a.ld, nd.eps, nd.decay, 1, 1, 1)
                     for b in (0, 1):
                         call("bsl_norm_apply", C.byref(ndh), C.c_void_p(L.y.p.value + b * 32 * BF16), q["scale"], q["shift"],
                              C.c_void_p(L.a.p.value + b * 32 * BF16), s)
@@ -782,7 +820,8 @@ class UNet3DEngine:
                 call("bsl_norm_bwd_reduce", C.byref(nd), L.y.p, cur.p, C.c_int(L.coutp), q["mean"], q["rstd"], q["scale"],
                      q["shift"], q["sums"], s)
                 call("bsl_norm_bwd_finalize", C.byref(nd), q["sums"], q["c1"], q["c2"],
-                     self._pp(self.G, f"{L.scope}/InstanceNorm/gamma"), self._pp(self.G, f"{L.scope}/InstanceNorm/beta"), s)
+                     self._pp(self.G, f"{L.scope}/{self.norm_scope}/gamma"),
+                     self._pp(self.G, f"{L.scope}/{self.norm_scope}/beta"), s)
                 call("bsl_norm_bwd_apply", C.byref(nd), L.y.p, cur.p, C.c_int(L.coutp), q["mean"], q["rstd"], q["scale"],
                      q["shift"], q["c1"], q["c2"], dyb.p, C.c_int(L.coutp), s)
                 # pixel-pair packed layers: the filter gradient of the SUPER filter goes to scratch and is folded back onto
@@ -858,8 +897,17 @@ class UNet3DEngine:
         self.step_count += 1
         enqueue_optimizer(self, lr)
 
+    def _allreduce_moving_stats(self):
+        # MirroredStrategy aggregates the moving-average updates with MEAN across replicas
+        # (/root/reference/core/estimator.py:570-613); batch statistics themselves stay per replica (no sync-BN)
+        if self.cfg.world > 1 and self.n_stats > 0:
+            self.ctx.call("bsl_allreduce_sum_f32", self.S.p, C.c_size_t(self.n_stats), self.stream)
+            self.ctx.call("bsl_scale_f32", self.S.p, C.c_size_t(self.n_stats), C.c_float(1.0 / self.cfg.world),
+                          self.stream)
+
     def train_step(self, lr: float, with_metrics: bool = False):
         self.forward(True)
+        self._allreduce_moving_stats()
         if with_metrics:
             self.predict_outputs(True)
         self.loss_backward()

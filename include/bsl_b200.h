@@ -182,6 +182,11 @@ int bsl_conv3d_fprop(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x_bf16,
  * channel), what slim.instance_norm's moments need (NetworksV2/UNet3D.py:151-158). */
 int bsl_conv3d_fprop_group_stats(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x_bf16, const void* w_dhwio_bf16,
                                  void* y_bf16, double* sums, void* stream);
+/* fprop + batch statistics: sums is fp64 [2][cout] (sum, sum of squares of the bf16 outputs over all n*d*h*w output
+ * voxels), the moments of slim.batch_norm after slim.conv3d (NetworksV2/UNet3D.py:151-158 with --normalizer batch_norm).
+ * The 3-D counterpart of bsl_conv2d_fprop_stats; the bf16 outputs are bit-identical to bsl_conv3d_fprop's. */
+int bsl_conv3d_fprop_stats(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* x_bf16, const void* w_dhwio_bf16,
+                           void* y_bf16, double* sums, void* stream);
 int bsl_conv3d_dgrad(bsl_ctx* ctx, const bsl_conv3d_desc* d, const void* dy_bf16, const void* w_dhwio_bf16,
                      void* dx_bf16, void* stream);
 size_t bsl_conv3d_wgrad_workspace(bsl_ctx* ctx, const bsl_conv3d_desc* d);

@@ -3,7 +3,7 @@ so that every model family has a number): cfg3 GUNet 512x512 batch 32, cfg4 UNet
 UNet 2-D inference. One JSON line per configuration; CUDA events over `--steps` steps after 3 warm-ups, inputs
 resident in HBM.
 
-  python tools/bench_models.py [--which gunet,unet3d,unet_infer] [--steps 5]
+  python tools/bench_models.py [--which gunet,unet3d,unet_infer] [--steps 5] [--normalizer instance_norm|batch_norm]
 """
 import argparse
 import json
@@ -20,6 +20,8 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--which", default="gunet,unet3d,unet_infer")
 ap.add_argument("--steps", type=int, default=5)
 ap.add_argument("--breakdown", action="store_true")
+ap.add_argument("--normalizer", default="instance_norm", choices=["instance_norm", "batch_norm"],
+                help="normaliser of the unet3d configuration (cfg4 is instance norm)")
 a = ap.parse_args()
 ctx = Context(0)
 peak = 1371.6
@@ -96,14 +98,14 @@ for which in a.which.split(","):
     elif which == "unet3d":
         from boxsegliver_b200.unet3d_engine import UNet3DConfig, UNet3DEngine
         n, d, h, w = 4, 64, 128, 128
-        cfg = UNet3DConfig(batch=n, depth=d, height=h, width=w, loss_numeric_w=(1.0, 1.0))
+        cfg = UNet3DConfig(batch=n, depth=d, height=h, width=w, loss_numeric_w=(1.0, 1.0), normalizer=a.normalizer)
         eng = UNet3DEngine(ctx, cfg)
         eng.init_weights(0)
         im, lb = synthetic.make_volume_batch(n, d, h, w)
         eng.set_inputs(im, lb)
         ms = timed(lambda: eng.train_step(3e-4), a.steps)
         fl = eng.step_flops()["total"]
-        line = {"config": "cfg4 UNet3D 64x128x128 patch, batch 4, instance_norm, weighted xent 1/1, Adam",
+        line = {"config": f"cfg4 UNet3D 64x128x128 patch, batch 4, {a.normalizer}, weighted xent 1/1, Adam",
                 "metric": "unet3d_train_voxels_per_s", "value": n * d * h * w / ms * 1e3, "unit": "voxels/s",
                 "patches_per_s": n / ms * 1e3, "ms_per_step": ms, "step_tflop_algorithmic": fl / 1e12,
                 "model_tflops_per_s": fl / ms / 1e9, "frac_of_sustained_bf16_peak": fl / ms / 1e9 / peak,

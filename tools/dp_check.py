@@ -1,8 +1,9 @@
 """Data-parallel correctness on real GPUs (run under torchrun, one rank per GPU):
 
-  python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/dp_check.py
+  python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/dp_check.py [unet3d]
 
-Checks, for the 2-D U-Net engine with the bucketed all-reduce overlapped with backward:
+Checks, for the 2-D U-Net engine with the bucketed all-reduce overlapped with backward (or, with `unet3d`, for the
+3-D U-Net engine with --normalizer batch_norm and its whole-arena gradient all-reduce):
   1. the all-reduced gradient arena equals the SUM over ranks of the local gradients (computed first without the
      communicator and exchanged through gloo), to fp32 rounding of a different summation order;
   2. batch-norm moving statistics are the cross-replica MEAN of the per-replica updates;
@@ -25,12 +26,24 @@ from boxsegliver_b200.engine import EngineConfig, UNetEngine  # noqa: E402
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 dist.init_process_group("gloo", rank=rank, world_size=world)
 ctx = Context(local)
-n, hw = 4, 128
-cfg = EngineConfig(batch=n, height=hw, width=hw, loss_weight_type="numerical", loss_numeric_w=(0.2, 0.4, 4.4),
-                   weight_decay_rate=1e-5, world=world)
-eng = UNetEngine(ctx, cfg)
+unet3d = sys.argv[1:] == ["unet3d"]
+if unet3d:
+    from boxsegliver_b200.unet3d_engine import UNet3DConfig, UNet3DEngine  # noqa: E402
+    n, d, hw = 2, 8, 64
+    eng = UNet3DEngine(ctx, UNet3DConfig(batch=n, depth=d, height=hw, width=hw, normalizer="batch_norm",
+                                         weight_decay_rate=3e-5, world=world))
+    im, lb = synthetic.make_volume_batch(n, d, hw, hw, seed=1357 + rank)
+
+    def allreduce_grads():
+        ctx.call("bsl_allreduce_sum_f32", eng.G.p, C.c_size_t(eng.n_train), eng.stream)
+else:
+    n, hw = 4, 128
+    cfg = EngineConfig(batch=n, height=hw, width=hw, loss_weight_type="numerical", loss_numeric_w=(0.2, 0.4, 4.4),
+                       weight_decay_rate=1e-5, world=world)
+    eng = UNetEngine(ctx, cfg)
+    im, lb = synthetic.make_batch(n, hw, hw, 3, seed=1357 + rank)
+    allreduce_grads = eng._allreduce_grads
 w0 = eng.init_weights(seed=0)
-im, lb = synthetic.make_batch(n, hw, hw, 3, seed=1357 + rank)
 eng.set_inputs(im, lb)
 
 # local gradients (no communicator attached yet: _after_grad is inert, no all-reduce is issued)
@@ -52,7 +65,7 @@ eng.set_weights(w0)
 eng.forward(True)
 eng._allreduce_moving_stats()
 eng.loss_backward()
-eng._allreduce_grads()
+allreduce_grads()
 ctx.check_device()
 g_dev = eng.G.download(np.float32, (eng.n_train,)).astype(np.float64)
 s_dev = eng.S.download(np.float32, (eng.n_stats,)).astype(np.float64)
@@ -71,7 +84,8 @@ dist.all_reduce(lo, op=dist.ReduceOp.MIN)
 dist.all_reduce(hi, op=dist.ReduceOp.MAX)
 assert bool((lo == hi).all()), "mirrored weights diverged across ranks"
 if rank == 0:
-    print(f"dp_check OK: world={world} buckets={len(eng._bucket_at)} grad rel err {e_g:.2e} moving-stat rel err {e_s:.2e} "
+    what = "unet3d batch_norm" if unet3d else f"unet buckets={len(eng._bucket_at)}"
+    print(f"dp_check OK: world={world} {what} grad rel err {e_g:.2e} moving-stat rel err {e_s:.2e} "
           f"weights bit-identical on all ranks after 3 steps")
 dist.barrier()
 dist.destroy_process_group()
