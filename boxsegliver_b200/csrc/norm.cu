@@ -636,8 +636,13 @@ __global__ void norm_affine_fold_kernel(int n, int c, int G, const float* __rest
 }
 
 // norm_bwd_finalize_mod_kernel with the folded channel-wise affine. S0 = sum dz, S1 = sum dz*xhat, T_g = sum dz*guide_g
-// are sums of the gradient AFTER the affine; u = xhat*(scale_pre/rstd) + (shift_pre + mean*scale_pre) + guide.w.
-__global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, const double* __restrict__ sums,
+// are sums of the gradient AFTER the affine, one row per group (a sample, or the whole batch in mode 0);
+// u = xhat*(scale_pre/rstd) + (shift_pre + mean*scale_pre) + guide.w. `jac` selects what c1 / c2 hold:
+//   BSL_NORM_JAC_GROUP   c1 = S0/m, c2 = S1/m per group (instance norm; batch norm on its single group)
+//   BSL_NORM_JAC_BATCH   the per-sample view of a batch-norm layer: c1r = rstd*gamma*ga*sum_n gm[n]*S0_n / m,
+//                        c2r likewise with S1 (m = n*hw), the same value for every sample (bsl_norm_bwd_apply_bnmod)
+//   BSL_NORM_JAC_NONE    identity normaliser: c1 = c2 = 0
+__global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, int jac, const double* __restrict__ sums,
                                                 const float* __restrict__ gamma_mod, int gm_ld,
                                                 const float* __restrict__ gamma, const float* __restrict__ beta,
                                                 const float* __restrict__ ga, const float* __restrict__ mean,
@@ -657,8 +662,10 @@ __global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, c
     const double* q = sums + (long long)s * K * c + ch;
     const double s0 = q[0], s1 = q[c];
     const int o = s * c + ch;
-    c1[o] = (float)(s0 / m);
-    c2[o] = (float)(s1 / m);
+    if (jac != BSL_NORM_JAC_BATCH) {
+      c1[o] = jac == BSL_NORM_JAC_GROUP ? (float)(s0 / m) : 0.f;
+      c2[o] = jac == BSL_NORM_JAC_GROUP ? (float)(s1 / m) : 0.f;
+    }
     const double sp = (double)scale_pre[o], hp = (double)shift_pre[o];
     double du = sp / (double)rstd[o] * s1 + (hp + (double)mean[o] * sp) * s0;
     for (int g = 0; g < K - 2; ++g) du += (double)w[g * w_ld + ch] * q[(long long)(2 + g) * c];
@@ -669,6 +676,14 @@ __global__ void norm_bwd_finalize_affine_kernel(int n, int c, int K, double m, c
     sb += gm * s0;
     s0all += s0;
     for (int g = 0; g < K - 2; ++g) t[g] += q[(long long)(2 + g) * c];
+  }
+  if (jac == BSL_NORM_JAC_BATCH) {
+    const double r = (double)rstd[ch] * gam * a / m;
+    const float k1 = (float)(r * sb), k2 = (float)(r * sg);
+    for (int s = 0; s < n; ++s) {
+      c1[s * c + ch] = k1;
+      c2[s * c + ch] = k2;
+    }
   }
   if (dgamma) dgamma[ch] = (float)(a * sg);
   if (dbeta) dbeta[ch] = (float)(a * sb);
@@ -1558,14 +1573,41 @@ int bsl_norm_affine_fold(bsl_ctx* ctx, const bsl_norm_desc* d, const float* gamm
                          int guide_channels, float* w_eff, void* stream) {
   int rc = check_norm(ctx, d);
   if (rc) return rc;
-  if (d->mode != 1) return bsl_fail(ctx, BSL_EUNSUPPORTED, "norm_affine_fold: instance_norm layers only");
   if (!gamma_a || !beta_a || !scale || !shift || !scale_pre || !shift_pre || guide_channels < 0 || guide_channels > 2 ||
       (guide_channels && (!w_guide || !w_eff || w_ld < d->c)))
     return bsl_fail(ctx, BSL_EINVAL, "norm_affine_fold: bad argument");
-  const int total = d->n > guide_channels ? d->n * d->c : guide_channels * d->c;
-  bsl_launch(norm_affine_fold_kernel, dim3((total + 127) / 128), dim3(128), 0, as_stream(stream), d->n, d->c,
+  const int groups = d->mode ? d->n : 1;
+  const int total = groups > guide_channels ? groups * d->c : guide_channels * d->c;
+  bsl_launch(norm_affine_fold_kernel, dim3((total + 127) / 128), dim3(128), 0, as_stream(stream), groups, d->c,
              guide_channels, gamma_a, beta_a, scale, shift, scale_pre, shift_pre, w_guide, w_ld, w_eff);
   BSL_LAUNCH_CHECK(ctx, "norm_affine_fold_kernel");
+  return BSL_OK;
+}
+
+int bsl_norm_bwd_finalize_affine_jac(bsl_ctx* ctx, const bsl_norm_desc* d, int jacobian, const double* sums,
+                                     int guide_channels, const float* gamma_mod, int gm_ld, const float* gamma,
+                                     const float* beta, const float* gamma_a, const float* mean, const float* rstd,
+                                     const float* scale_pre, const float* shift_pre, const float* w_guide, int w_ld,
+                                     float* c1, float* c2, float* dgamma, float* dbeta, float* dgamma_mod,
+                                     float* dw_guide, int dw_ld, float* dbias_guide, float* dgamma_a, float* dbeta_a,
+                                     void* stream) {
+  int rc = check_norm(ctx, d);
+  if (rc) return rc;
+  if (jacobian != BSL_NORM_JAC_GROUP && jacobian != BSL_NORM_JAC_BATCH && jacobian != BSL_NORM_JAC_NONE)
+    return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_finalize_affine: jacobian %d", jacobian);
+  if (jacobian == BSL_NORM_JAC_BATCH && d->mode != 1)
+    return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_finalize_affine: BSL_NORM_JAC_BATCH takes the per-sample (mode 1) view");
+  const int groups = d->mode ? d->n : 1;
+  if (!sums || !c1 || !c2 || !gamma_a || !mean || !rstd || !scale_pre || !shift_pre || !dgamma_a || !dbeta_a ||
+      guide_channels < 0 || guide_channels > 2 || (gamma_mod && (!dgamma_mod || groups != d->n)) ||
+      (guide_channels && (!dw_guide || dw_ld < d->c || !w_guide || w_ld < d->c)))
+    return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_finalize_affine: bad argument");
+  const double m = d->mode && jacobian != BSL_NORM_JAC_BATCH ? (double)d->hw : (double)d->n * d->hw;
+  bsl_launch(norm_bwd_finalize_affine_kernel, dim3((d->c + 127) / 128), dim3(128), 0, as_stream(stream), groups, d->c,
+             2 + guide_channels, m, jacobian, sums, gamma_mod, gm_ld, d->scale ? gamma : nullptr,
+             d->center ? beta : nullptr, gamma_a, mean, rstd, scale_pre, shift_pre, w_guide, w_ld, c1, c2, dgamma, dbeta,
+             dgamma_mod, dw_guide, dw_ld, dbias_guide, dgamma_a, dbeta_a);
+  BSL_LAUNCH_CHECK(ctx, "norm_bwd_finalize_affine_kernel");
   return BSL_OK;
 }
 
@@ -1575,19 +1617,9 @@ int bsl_norm_bwd_finalize_affine(bsl_ctx* ctx, const bsl_norm_desc* d, const dou
                                  const float* shift_pre, const float* w_guide, int w_ld, float* c1, float* c2,
                                  float* dgamma, float* dbeta, float* dgamma_mod, float* dw_guide, int dw_ld,
                                  float* dbias_guide, float* dgamma_a, float* dbeta_a, void* stream) {
-  int rc = check_norm(ctx, d);
-  if (rc) return rc;
-  if (d->mode != 1) return bsl_fail(ctx, BSL_EUNSUPPORTED, "norm_bwd_finalize_affine: instance_norm layers only");
-  if (!sums || !c1 || !c2 || !gamma_a || !mean || !rstd || !scale_pre || !shift_pre || !dgamma_a || !dbeta_a ||
-      guide_channels < 0 || guide_channels > 2 || (gamma_mod && !dgamma_mod) ||
-      (guide_channels && (!dw_guide || dw_ld < d->c || !w_guide || w_ld < d->c)))
-    return bsl_fail(ctx, BSL_EINVAL, "norm_bwd_finalize_affine: bad argument");
-  bsl_launch(norm_bwd_finalize_affine_kernel, dim3((d->c + 127) / 128), dim3(128), 0, as_stream(stream), d->n, d->c,
-             2 + guide_channels, (double)d->hw, sums, gamma_mod, gm_ld, d->scale ? gamma : nullptr,
-             d->center ? beta : nullptr, gamma_a, mean, rstd, scale_pre, shift_pre, w_guide, w_ld, c1, c2, dgamma, dbeta,
-             dgamma_mod, dw_guide, dw_ld, dbias_guide, dgamma_a, dbeta_a);
-  BSL_LAUNCH_CHECK(ctx, "norm_bwd_finalize_affine_kernel");
-  return BSL_OK;
+  return bsl_norm_bwd_finalize_affine_jac(ctx, d, BSL_NORM_JAC_GROUP, sums, guide_channels, gamma_mod, gm_ld, gamma,
+                                          beta, gamma_a, mean, rstd, scale_pre, shift_pre, w_guide, w_ld, c1, c2, dgamma,
+                                          dbeta, dgamma_mod, dw_guide, dw_ld, dbias_guide, dgamma_a, dbeta_a, stream);
 }
 
 static int norm_bwd_apply_impl(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x, const void* dy, int dy_ld,

@@ -11,10 +11,13 @@ hidden layers); the additive map is the level's 1x1 guide convolution (GUNet.py:
 the normalisation kernels, so modulation adds no pass over the activations. `after_affine` (5 of the 13 shipped
 ext_config/*.yml; slim_nets.channel_wise_affine before every encoder ReLU, GUNet.py:213-214) folds into the same
 per-(sample, channel) scale / shift and a gamma-scaled copy of the guide filter (bsl_norm_affine_fold): no extra pass.
+`--normalizer batch_norm` (GUNet.py:301,321-325): batch statistics; modulated and dropped blocks run on the per-sample view
+(bsl_norm_modulate_bn), un-modulated blocks keep per-channel scalars, and the affine folds into whichever the block has.
 Backbone `--dropout` (GUNet.py:189-190: slim.dropout behind the normaliser of the first conv of every encoder block, in
 front of the modulation; no shipped script enables it) runs un-fused: normalise without ReLU into a bf16 copy, multiply it
 by the Philox mask in place (bsl_dropout_bf16), then the ordinary modulated apply pass over that copy with an identity
-normaliser; backward mirrors the three stages.
+normaliser (folding the affine under after_affine); backward mirrors the three stages. Every combination of normaliser,
+after_affine and --dropout trains and evaluates.
 `--img_grad` (GUNet.py:333-337, scripts/103_grad.sh): the input becomes concat(images, dy, dx) of
 tf.image.image_gradients, packed as bf16 [n, h, w, 64] (9 live lanes) by bsl_image_gradients_pack; the first layer then
 runs as an ordinary 64-lane conv instead of the im2col stem.
@@ -30,6 +33,8 @@ import numpy as np
 
 from . import _lib
 from .engine import BF16, F32, ConvL, EngineConfig, Param, UNetEngine, View, _align
+
+JAC_GROUP, JAC_BATCH, JAC_NONE = 0, 1, 2      # BSL_NORM_JAC_* of include/bsl_b200.h
 
 
 @dataclass
@@ -64,16 +69,12 @@ class GUNetEngine(UNetEngine):
     prefix = "GUNet"      # variable-scope root (UNetInterEngine reuses the graph under "UNetInter")
 
     def __init__(self, ctx, cfg: GUNetConfig):
-        if cfg.normalizer == "batch_norm" and getattr(cfg, "after_affine", False):
-            raise NotImplementedError("GUNet engine: after_affine with --normalizer batch_norm is not supported")
         for flag in ("use_se", "fix", "without_norm"):
             if getattr(cfg, flag):
                 raise NotImplementedError(f"GUNet engine: --{flag} is not supported")
         if cfg.dropout:
             if not 0.0 < cfg.dropout < 1.0:
                 raise ValueError("--dropout must lie in (0, 1)")
-            if cfg.normalizer != "instance_norm" or getattr(cfg, "after_affine", False):
-                raise NotImplementedError("GUNet engine: --dropout is built for instance_norm without after_affine")
         if cfg.context_model != "fc":
             raise ValueError("Not supported context model")          # GUNet.py:79
         if cfg.use_spatial and cfg.guide_channel not in (1, 2):
@@ -180,8 +181,9 @@ class GUNetEngine(UNetEngine):
         return self.input_packed
 
     def _bn_mod(self, L: ConvL) -> bool:
-        """A modulated block under batch norm: batch statistics, per-sample scale / shift."""
-        return self.cfg.normalizer == "batch_norm" and (L.mod_off is not None or L.sp_off is not None)
+        """A modulated or --dropout block under batch norm: batch statistics, per-sample scale / shift (the mode-1 view).
+        An un-modulated block with only the affine keeps per-channel scalars and folds the affine into them."""
+        return self.cfg.normalizer == "batch_norm" and (L.mod_off is not None or L.sp_off is not None or self._drops(L))
 
     def _norm_groups(self, L: ConvL, default: int) -> int:
         return self.cfg.batch if self._bn_mod(L) else default
@@ -254,7 +256,10 @@ class GUNetEngine(UNetEngine):
             return L.y.p
         cfg, call, s = self.cfg, self.ctx.call, self.stream
         T, qn = self.drop[L.scope]["T"], self._drop_ptrs(L)
-        nbytes = C.c_size_t(cfg.batch * L.cout * F32)
+        # the normaliser's scalars are [n][cout] under instance norm, [cout] under batch norm (mode 0); the identity of
+        # the modulation stage fills the layer's whole scalar arrays ([n][cout]: the per-sample view)
+        nbytes = C.c_size_t((cfg.batch if nd.mode else 1) * L.cout * F32)
+        nbytes_id = C.c_size_t(L.norm["groups"] * L.cout * F32)
         for k in ("mean", "rstd", "scale", "shift"):       # the normaliser's own scalars move aside ...
             call("bsl_memcpy_d2d", qn[k], q[k], nbytes, s)
         ndn = _lib.NormDesc(nd.mode, nd.n, nd.hw, nd.c, nd.x_ld, L.cout, nd.eps, nd.decay, 0, nd.center, nd.scale)
@@ -263,7 +268,7 @@ class GUNetEngine(UNetEngine):
         call("bsl_dropout_bf16", C.byref(dd), C.c_longlong(cfg.batch * L.h * L.w), C.c_int(L.cout), T.p, C.c_int(L.cout),
              T.p, C.c_int(L.cout), s)
         for k, src in (("mean", self._zeros), ("rstd", self._ones), ("scale", self._ones), ("shift", self._zeros)):
-            call("bsl_memcpy_d2d", q[k], src.p, nbytes, s)     # ... and the modulation stage sees an identity normaliser
+            call("bsl_memcpy_d2d", q[k], src.p, nbytes_id, s)  # ... and the modulation stage sees an identity normaliser
         self._dropped = getattr(self, "_dropped", set()) | {L.scope}
         return T.p
 
@@ -349,22 +354,21 @@ class GUNetEngine(UNetEngine):
                           self._pp(self.W, f"{sc}/weights", off=L.sp_off).value, 2 * L.cout)
 
     def _modulate(self, L: ConvL, nd, q):
-        if L.mod_off is not None or L.sp_off is not None:
-            gm = C.c_void_p(self.ctx_params.ptr + L.mod_off * F32) if L.mod_off is not None else None
-            bsp = self._pp(self.W, f"GUNet/spatial/conv{L.level + 1}/biases", off=L.sp_off) if L.sp_off is not None else None
-            if self._bn_mod(L):
-                self.ctx.call("bsl_norm_modulate_bn", C.byref(self._apply_desc(L, nd)), gm,
-                              C.c_int(self.cfg.n_modulator_param), bsp, q["mean"], q["rstd"], q["scale"], q["shift"],
-                              self.stream)
-            else:
-                self.ctx.call("bsl_norm_modulate", C.byref(nd), gm, C.c_int(self.cfg.n_modulator_param), bsp, q["scale"],
-                              q["shift"], self.stream)
+        gm = C.c_void_p(self.ctx_params.ptr + L.mod_off * F32) if L.mod_off is not None else None
+        bsp = self._pp(self.W, f"GUNet/spatial/conv{L.level + 1}/biases", off=L.sp_off) if L.sp_off is not None else None
+        if self._bn_mod(L):      # (an un-modulated --dropout block: expansion to the per-sample view only)
+            self.ctx.call("bsl_norm_modulate_bn", C.byref(self._apply_desc(L, nd)), gm,
+                          C.c_int(self.cfg.n_modulator_param), bsp, q["mean"], q["rstd"], q["scale"], q["shift"],
+                          self.stream)
+        elif L.mod_off is not None or L.sp_off is not None:
+            self.ctx.call("bsl_norm_modulate", C.byref(nd), gm, C.c_int(self.cfg.n_modulator_param), bsp, q["scale"],
+                          q["shift"], self.stream)
         if L.affine:
             sp, hp, weff = self._aff_ptrs(L)
             g = self._guide_channels(L)
             wsp = self._pp(self.W, f"GUNet/spatial/conv{L.level + 1}/weights", off=L.sp_off) if g else None
-            self.ctx.call("bsl_norm_affine_fold", C.byref(nd), self._pp(self.W, f"{L.affine}/gamma"),
-                          self._pp(self.W, f"{L.affine}/beta"), q["scale"], q["shift"], sp, hp, wsp,
+            self.ctx.call("bsl_norm_affine_fold", C.byref(self._apply_desc(L, nd)),
+                          self._pp(self.W, f"{L.affine}/gamma"), self._pp(self.W, f"{L.affine}/beta"), q["scale"], q["shift"], sp, hp, wsp,
                           C.c_int(2 * L.cout), C.c_int(g), weff if g else None, self.stream)
         return self._guide_struct(L)
 
@@ -392,6 +396,15 @@ class GUNetEngine(UNetEngine):
         xin = self.drop[L.scope]["T"].p if dropped else L.y.p
         call("bsl_norm_bwd_reduce_mod", C.byref(nd), xin, cur.p, C.c_int(L.cout), q["mean"], q["rstd"], q["scale"],
              q["shift"], gp, q["sums"], s)
+        if dropped and L.affine:
+            # modulation stage over the dropped tensor with the folded affine: identity normaliser, no Jacobian
+            sp, hp, _ = self._aff_ptrs(L)
+            wsp = self._pp(self.W, f"{ssc}/weights", off=L.sp_off) if L.sp_off is not None else None
+            call("bsl_norm_bwd_finalize_affine_jac", C.byref(nd), C.c_int(JAC_NONE), q["sums"],
+                 C.c_int(self._guide_channels(L)), gm, C.c_int(nmod), None, None, self._pp(self.W, f"{L.affine}/gamma"),
+                 q["mean"], q["rstd"], sp, hp, wsp, C.c_int(2 * L.cout), q["c1"], q["c2"], None, None, dgm, dwg,
+                 C.c_int(2 * L.cout), dbg, self._pp(self.G, f"{L.affine}/gamma"), self._pp(self.G, f"{L.affine}/beta"), s)
+            return
         if dropped:
             # modulation stage over the dropped tensor: identity normaliser (no gamma / beta, no Jacobian: c1 = c2 = 0);
             # sum(dz * T) is the gradient of gamma_mod, the guide rows those of the 1x1 guide conv
@@ -402,10 +415,12 @@ class GUNetEngine(UNetEngine):
             call("bsl_memset", q["c2"], C.c_int(0), nbytes, s)
             return
         if L.affine:
+            # batch norm: modulated blocks on the per-sample view (pooled Jacobian), the others on their single group
             sp, hp, _ = self._aff_ptrs(L)
             wsp = self._pp(self.W, f"{ssc}/weights", off=L.sp_off) if L.sp_off is not None else None
-            call("bsl_norm_bwd_finalize_affine", C.byref(nd), q["sums"], C.c_int(self._guide_channels(L)), gm,
-                 C.c_int(nmod), self._pp(self.W, f"{L.scope}/{ns}/gamma"), self._pp(self.W, f"{L.scope}/{ns}/beta"),
+            call("bsl_norm_bwd_finalize_affine_jac", C.byref(nd), C.c_int(JAC_BATCH if self._bn_mod(L) else JAC_GROUP),
+                 q["sums"], C.c_int(self._guide_channels(L)), gm, C.c_int(nmod),
+                 self._pp(self.W, f"{L.scope}/{ns}/gamma"), self._pp(self.W, f"{L.scope}/{ns}/beta"),
                  self._pp(self.W, f"{L.affine}/gamma"), q["mean"], q["rstd"], sp, hp, wsp, C.c_int(2 * L.cout),
                  q["c1"], q["c2"], self._pp(self.G, f"{L.scope}/{ns}/gamma"), self._pp(self.G, f"{L.scope}/{ns}/beta"),
                  dgm, dwg, C.c_int(2 * L.cout), dbg, self._pp(self.G, f"{L.affine}/gamma"),
@@ -430,8 +445,8 @@ class GUNetEngine(UNetEngine):
             call, ns = self.ctx.call, self.norm_scope
             T, dT, qn = self.drop[L.scope]["T"], self.drop_grad, self._drop_ptrs(L)
             c = C.c_int(L.cout)
-            call("bsl_norm_bwd_apply_mod", C.byref(nd), T.p, cur.p, c, q["mean"], q["rstd"], q["scale"], q["shift"],
-                 q["c1"], q["c2"], C.byref(guide) if guide is not None else None, dT.p, c, stream)
+            call("bsl_norm_bwd_apply_mod", C.byref(self._apply_desc(L, nd)), T.p, cur.p, c, q["mean"], q["rstd"],
+                 q["scale"], q["shift"], q["c1"], q["c2"], C.byref(guide) if guide is not None else None, dT.p, c, stream)
             dd = self._drop_desc(L)
             call("bsl_dropout_bf16", C.byref(dd), C.c_longlong(self.cfg.batch * L.h * L.w), c, dT.p, c, dT.p, c, stream)
             ndn = _lib.NormDesc(nd.mode, nd.n, nd.hw, nd.c, nd.x_ld, nd.y_ld, nd.eps, nd.decay, 0, nd.center, nd.scale)

@@ -346,14 +346,36 @@ int bsl_norm_bwd_apply_bnmod(bsl_ctx* ctx, const bsl_norm_desc* d, const void* x
  * gamma_a * u + beta_a between the modulation and the ReLU of every encoder block. With u = y*scale + shift + guide.w
  * the affine folds into the same three quantities, so no pass changes: bsl_norm_affine_fold rewrites scale *= gamma_a,
  * shift = shift*gamma_a + beta_a in place (keeping the un-folded values in scale_pre / shift_pre for the backward
- * finaliser) and writes the gamma_a-scaled guide filter w_eff[g * c + ch] the *_mod passes then read. */
+ * finaliser) and writes the gamma_a-scaled guide filter w_eff[g * c + ch] the *_mod passes then read.
+ * Representation: scale / shift / mean / rstd are [groups][c] in the view the descriptor describes, groups = n in
+ * mode 1 and 1 in mode 0. An instance-norm layer and a modulated batch-norm layer (after bsl_norm_modulate_bn) pass the
+ * per-sample mode-1 view; an un-modulated batch-norm layer passes its mode-0 descriptor and folds its per-channel
+ * scale / shift (no guide there). scale_pre / shift_pre have the same [groups][c] shape. */
 int bsl_norm_affine_fold(bsl_ctx* ctx, const bsl_norm_desc* d, const float* gamma_a, const float* beta_a, float* scale,
                          float* shift, float* scale_pre, float* shift_pre, const float* w_guide /*nullable*/, int w_ld,
                          int guide_channels, float* w_eff /*[guide_channels][c], nullable*/, void* stream);
 /* bsl_norm_bwd_finalize_mod for a layer with the folded affine. `sums` were reduced with the FOLDED scale / shift /
- * w_eff (they are sums of dz, the gradient after the affine); scale_pre / shift_pre / w_guide are the un-folded ones.
- * Emits dgamma_a[c] = sum_n (scale_pre/rstd * S1 + (shift_pre + mean*scale_pre) * S0 + sum_g w_g * T_g) and
- * dbeta_a[c] = sum_n S0, and every other gradient with the sums scaled by gamma_a (du = gamma_a * dz). */
+ * w_eff (they are sums of dz, the gradient after the affine, one row per group of the descriptor's view); scale_pre /
+ * shift_pre / w_guide are the un-folded ones. Emits dgamma_a[c] = sum_groups (scale_pre/rstd * S1 +
+ * (shift_pre + mean*scale_pre) * S0 + sum_g w_g * T_g) (= sum dz * u, u the pre-affine value) and dbeta_a[c] = sum S0,
+ * and every other gradient with the sums scaled by gamma_a (du = gamma_a * dz). `jacobian` selects c1 / c2:
+ *   BSL_NORM_JAC_GROUP  c1 = S0/m, c2 = S1/m per group, m the values per group, for bsl_norm_bwd_apply[_mod]: instance
+ *                       norm (mode 1) and an un-modulated batch-norm layer (mode 0, one group);
+ *   BSL_NORM_JAC_BATCH  a modulated batch-norm layer on its per-sample view (mode 1): c1r / c2r of
+ *                       bsl_norm_bwd_finalize_bnmod with gamma_a in the chain, for bsl_norm_bwd_apply_bnmod;
+ *   BSL_NORM_JAC_NONE   identity normaliser (mean 0, rstd 1: the modulation stage of a GUNet --dropout layer, gamma /
+ *                       beta NULL): c1 = c2 = 0.
+ * bsl_norm_bwd_finalize_affine is the BSL_NORM_JAC_GROUP call. */
+#define BSL_NORM_JAC_GROUP 0
+#define BSL_NORM_JAC_BATCH 1
+#define BSL_NORM_JAC_NONE 2
+int bsl_norm_bwd_finalize_affine_jac(bsl_ctx* ctx, const bsl_norm_desc* d, int jacobian, const double* sums,
+                                     int guide_channels, const float* gamma_mod, int gm_ld, const float* gamma,
+                                     const float* beta, const float* gamma_a, const float* mean, const float* rstd,
+                                     const float* scale_pre, const float* shift_pre, const float* w_guide, int w_ld,
+                                     float* c1, float* c2, float* dgamma, float* dbeta, float* dgamma_mod,
+                                     float* dw_guide, int dw_ld, float* dbias_guide, float* dgamma_a, float* dbeta_a,
+                                     void* stream);
 int bsl_norm_bwd_finalize_affine(bsl_ctx* ctx, const bsl_norm_desc* d, const double* sums, int guide_channels,
                                  const float* gamma_mod, int gm_ld, const float* gamma, const float* beta,
                                  const float* gamma_a, const float* mean, const float* rstd, const float* scale_pre,
