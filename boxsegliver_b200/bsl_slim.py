@@ -11,6 +11,9 @@ then recognises the U-Net family the accelerated path covers --
     [conv3x3 + norm + ReLU] x 2 -> max_pool 2x2 (x depth) -> bridge -> [conv_transpose 2x2/2 + bias + ReLU ->
     concat(skip, up) -> [conv3x3 + norm + ReLU] x 2] (x depth) -> conv1x1 + bias
 
+with every 3x3 convolution either normalised (one normaliser throughout) or, with normalizer_fn=None, conv + bias + ReLU
+(engine --without_norm)
+
 -- and turns it into the layer table of `engine.UNetEngine`, i.e. into exactly the C-ABI launch sequence the engine
 issues (fused statistics epilogues, norm+pool in one pass, zero-copy concat, ...). Anything else raises
 NotImplementedError naming the node: a drop-in must never silently run something different.
@@ -320,6 +323,7 @@ def lower_to_layer_table(graph: Graph, logits: Tensor):
     convs_at_level = 0
     normalizer = None
     norm_params = None
+    norms_seen = set()     # normalizer attribute of every 3x3 conv (None: conv + bias + ReLU)
     regs = set()
     it = list(zip(order[1:], nodes[1:]))
     pos = 0
@@ -332,10 +336,11 @@ def lower_to_layer_table(graph: Graph, logits: Tensor):
             if a["kernel"] == (3, 3):
                 if a["stride"] != (1, 1) or a["rate"] != (1, 1):
                     _fail(nd, f"stride {a['stride']} / rate {a['rate']} (3x3 stride 1 rate 1 is covered)")
-                if a["normalizer"] is None or a["activation"] is not relu:
-                    _fail(nd, "3x3 convolutions are conv + batch/instance norm + ReLU")
-                if normalizer not in (None, a["normalizer"]):
-                    _fail(nd, "mixed normalisers")
+                if a["activation"] is not relu or (a["normalizer"] is None and not a["has_bias"]):
+                    _fail(nd, "3x3 convolutions are conv + batch/instance norm + ReLU, or conv + bias + ReLU")
+                norms_seen.add(a["normalizer"])
+                if len(norms_seen) > 1:
+                    _fail(nd, "mixed normalisers (normalised and plain 3x3 convolutions count as mixed)")
                 normalizer, norm_params = a["normalizer"], a["norm_params"]
                 convs_at_level += 1
                 if convs_at_level > 2:
@@ -396,7 +401,9 @@ def lower(graph: Graph, logits: Tensor, ctx, classes, **engine_kw):
     if len(classes) != info["num_classes"]:
         raise ValueError(f"{len(classes)} classes but the logits layer has {info['num_classes']} outputs")
     np_ = info["norm_params"] or {}
-    if info["normalizer"] == "batch_norm":
+    if info["normalizer"] is None:
+        engine_kw["without_norm"] = True
+    elif info["normalizer"] == "batch_norm":
         if not np_.get("scale", False):
             raise NotImplementedError("bsl_slim.lower: batch_norm without scale (the reference passes scale=True)")
         engine_kw.setdefault("bn_decay", np_.get("decay", 0.999))
@@ -406,7 +413,7 @@ def lower(graph: Graph, logits: Tensor, ctx, classes, **engine_kw):
     bias_reg = any(pair[1] for pair in info["regularizers"])
     cfg = EngineConfig(batch=info["batch"], height=info["height"], width=info["width"], channel=info["channel"],
                        classes=tuple(classes), init_channels=info["init_channels"],
-                       num_down_samples=info["num_down_samples"], normalizer=info["normalizer"],
+                       num_down_samples=info["num_down_samples"], normalizer=info["normalizer"] or "batch_norm",
                        weight_decay_rate=rate, bias_decay=bool(wd) and not bias_reg, **engine_kw)
 
     class GraphEngine(UNetEngine):

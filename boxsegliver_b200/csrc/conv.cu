@@ -212,10 +212,10 @@ int reduce_splits(bsl_ctx* ctx, const float* part, float* out, long long n, int 
 
 // ------------------------------------------------------------------ second-generation (halo-tile) kernels
 
-template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool TMA_ST = false>
+template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool TMA_ST = false, bool BR = false>
 int launch_halo_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, int grid,
                     cudaStream_t stream, const CUtensorMap* o = nullptr) {
-  auto kern = conv_halo_kernel<BN, NSUB, B_MN, STATS, SCATTER, false, TMA_ST>;
+  auto kern = conv_halo_kernel<BN, NSUB, B_MN, STATS, SCATTER, false, TMA_ST, false, BR>;
   constexpr int smem = ConvHaloCfg<BN, NSUB, TMA_ST>::SMEM_BYTES;
   static bool configured = false;
   if (!configured) {
@@ -232,10 +232,10 @@ struct HaloPlan {
   int pair;   // planned for CTA pairs (pair_replan): 128-wide tiles over sub-tile pairs, plain epilogue
 };
 
-template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER>
+template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool BR = false>
 int launch_halo_res_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, int grid,
                         int smem, cudaStream_t stream) {
-  auto kern = conv_halo_kernel<BN, NSUB, B_MN, STATS, SCATTER, true>;
+  auto kern = conv_halo_kernel<BN, NSUB, B_MN, STATS, SCATTER, true, false, false, BR>;
   static int configured = 0;
   if (configured < smem) {
     BSL_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -266,13 +266,13 @@ bool plan_resident(int bn, int ntaps, int cblocks, int* nsub, int* a_stages, int
   return true;
 }
 
-template <bool B_MN, bool STATS, bool SCATTER>
+template <bool B_MN, bool STATS, bool SCATTER, bool BR = false>
 int launch_halo_res(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args,
                     int grid, int smem, cudaStream_t stream) {
-  if (bn == 64 && nsub == 2) return launch_halo_res_one<64, 2, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 64 && nsub == 1) return launch_halo_res_one<64, 1, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 128 && nsub == 2) return launch_halo_res_one<128, 2, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 128 && nsub == 1) return launch_halo_res_one<128, 1, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 64 && nsub == 2) return launch_halo_res_one<64, 2, B_MN, STATS, SCATTER, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 64 && nsub == 1) return launch_halo_res_one<64, 1, B_MN, STATS, SCATTER, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 128 && nsub == 2) return launch_halo_res_one<128, 2, B_MN, STATS, SCATTER, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 128 && nsub == 1) return launch_halo_res_one<128, 1, B_MN, STATS, SCATTER, BR>(ctx, a, b, args, grid, smem, stream);
   return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv_halo (resident): tile %d x %d", bn, nsub);
 }
 
@@ -349,10 +349,10 @@ bool pair_eligible(bsl_ctx* ctx, const ConvHaloArgs& a, int bn, int nsub) {
   return max_pairs(ctx) >= 1 && (bn == 256 || bn == 128) && nsub == 2 && a.n_sub_total % 4 == 0 && a.ntaps == 9 && a.halo == 1 &&
          !a.tap_table && a.up_cpb == 0;
 }
-template <int BN, bool B_MN>
+template <int BN, bool B_MN, bool BR = false>
 int launch_halo_pair(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, cudaStream_t stream,
                      const CUtensorMap& o) {
-  auto kern = conv_halo_kernel<BN, 2, B_MN, false, false, false, true, true>;
+  auto kern = conv_halo_kernel<BN, 2, B_MN, false, false, false, true, true, BR>;
   constexpr int smem = ConvHaloCfg<BN, 2, true, true>::SMEM_BYTES;
   static bool configured = false;
   if (!configured) {
@@ -398,10 +398,10 @@ void replan_pair_units(bsl_ctx* ctx, HaloPlan& p) {   // one column tile; both C
   p.pair = 1;
 }
 
-template <int BN, int NSUB, bool STATS>
+template <int BN, int NSUB, bool STATS, bool BR = false>
 int launch_halo_res_pair_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args, int grid,
                              int smem, cudaStream_t stream) {
-  auto kern = conv_halo_kernel<BN, NSUB, false, STATS, false, true, false, true>;
+  auto kern = conv_halo_kernel<BN, NSUB, false, STATS, false, true, false, true, BR>;
   static int configured = 0;
   if (configured < smem) {
     BSL_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -411,13 +411,13 @@ int launch_halo_res_pair_one(bsl_ctx* ctx, const CUtensorMap& a, const CUtensorM
   BSL_LAUNCH_CHECK(ctx, "conv_halo_kernel (CTA pairs, resident filter) launch");
   return BSL_OK;
 }
-template <bool STATS>
+template <bool STATS, bool BR = false>
 int launch_halo_res_pair(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args,
                          int grid, int smem, cudaStream_t stream) {
-  if (bn == 64 && nsub == 2) return launch_halo_res_pair_one<64, 2, STATS>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 64 && nsub == 1) return launch_halo_res_pair_one<64, 1, STATS>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 128 && nsub == 2) return launch_halo_res_pair_one<128, 2, STATS>(ctx, a, b, args, grid, smem, stream);
-  if (bn == 128 && nsub == 1) return launch_halo_res_pair_one<128, 1, STATS>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 64 && nsub == 2) return launch_halo_res_pair_one<64, 2, STATS, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 64 && nsub == 1) return launch_halo_res_pair_one<64, 1, STATS, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 128 && nsub == 2) return launch_halo_res_pair_one<128, 2, STATS, BR>(ctx, a, b, args, grid, smem, stream);
+  if (bn == 128 && nsub == 1) return launch_halo_res_pair_one<128, 1, STATS, BR>(ctx, a, b, args, grid, smem, stream);
   return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv_halo (CTA pairs, resident): tile %d x %d", bn, nsub);
 }
 
@@ -432,31 +432,32 @@ __global__ void filter_kmajor_kernel(const __nv_bfloat16* __restrict__ w, __nv_b
   o[i] = w[((long long)tap * cin + ci) * cout + co];
 }
 
-template <bool B_MN, bool STATS, bool SCATTER>
+// BR: the bias + ReLU epilogue (args.bias, bsl_conv2d_fprop_bias_relu) on the same schedules as the plain one.
+template <bool B_MN, bool STATS, bool SCATTER, bool BR = false>
 int launch_halo(bsl_ctx* ctx, int bn, int nsub, const CUtensorMap& a, const CUtensorMap& b, const ConvHaloArgs& args,
                 int grid, cudaStream_t stream, const CUtensorMap* b_half = nullptr) {
   if constexpr (!STATS && !SCATTER) {
     if (pair_eligible(ctx, args, bn, nsub) && (B_MN || b_half != nullptr)) {
       CUtensorMap o;
       if (out_map(ctx, args, args.vw, args.vh, &o) == 0)
-        return bn == 256 ? launch_halo_pair<256, B_MN>(ctx, a, B_MN ? b : *b_half, args, stream, o)
-                         : launch_halo_pair<128, B_MN>(ctx, a, B_MN ? b : *b_half, args, stream, o);
+        return bn == 256 ? launch_halo_pair<256, B_MN, BR>(ctx, a, B_MN ? b : *b_half, args, stream, o)
+                         : launch_halo_pair<128, B_MN, BR>(ctx, a, B_MN ? b : *b_half, args, stream, o);
     }
     if (bn == 256) {   // TMA-store epilogue of the 256-wide tiles (DESIGN.md 3.6)
       CUtensorMap o;
       if (out_map(ctx, args, args.vw, args.vh, &o) == 0) {
-        if (nsub == 2) return launch_halo_one<256, 2, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
-        if (nsub == 1) return launch_halo_one<256, 1, B_MN, false, false, true>(ctx, a, b, args, grid, stream, &o);
+        if (nsub == 2) return launch_halo_one<256, 2, B_MN, false, false, true, BR>(ctx, a, b, args, grid, stream, &o);
+        if (nsub == 1) return launch_halo_one<256, 1, B_MN, false, false, true, BR>(ctx, a, b, args, grid, stream, &o);
       }
     }
   }
-  if (bn == 64 && nsub == 2) return launch_halo_one<64, 2, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, stream);
-  if (bn == 64 && nsub == 1) return launch_halo_one<64, 1, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, stream);
-  if (bn == 128 && nsub == 2) return launch_halo_one<128, 2, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, stream);
-  if (bn == 128 && nsub == 1) return launch_halo_one<128, 1, B_MN, STATS, SCATTER>(ctx, a, b, args, grid, stream);
+  if (bn == 64 && nsub == 2) return launch_halo_one<64, 2, B_MN, STATS, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
+  if (bn == 64 && nsub == 1) return launch_halo_one<64, 1, B_MN, STATS, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
+  if (bn == 128 && nsub == 2) return launch_halo_one<128, 2, B_MN, STATS, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
+  if (bn == 128 && nsub == 1) return launch_halo_one<128, 1, B_MN, STATS, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
   if (!STATS) {  // the widest tile has no spare TMEM for an overlapped epilogue: statistics stay a separate pass
-    if (bn == 256 && nsub == 2) return launch_halo_one<256, 2, B_MN, false, SCATTER>(ctx, a, b, args, grid, stream);
-    if (bn == 256 && nsub == 1) return launch_halo_one<256, 1, B_MN, false, SCATTER>(ctx, a, b, args, grid, stream);
+    if (bn == 256 && nsub == 2) return launch_halo_one<256, 2, B_MN, false, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
+    if (bn == 256 && nsub == 1) return launch_halo_one<256, 1, B_MN, false, SCATTER, false, BR>(ctx, a, b, args, grid, stream);
   }
   return bsl_fail(ctx, BSL_EUNSUPPORTED, "conv_halo: tile %d x %d", bn, nsub);
 }
@@ -742,8 +743,9 @@ static int launch_fprop_halo_stats(bsl_ctx* ctx, const HaloPlan& pl, bool res, i
 // fprop on the halo-tile kernel; `sums` (fp64 [2][cout], nullable) receives the per-channel sum and
 // sum of squares of the bf16 outputs, reduced deterministically from per-CTA partials.
 // group_imgs > 0: instance statistics, sums is [n / group_imgs][2][cout] (one group = group_imgs consecutive images).
+// bias != nullptr (no sums): the bias + ReLU epilogue, y = bf16(relu(conv + bias)), on the schedule the plain fprop takes.
 static int conv2d_fprop_halo(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
-                             double* sums, cudaStream_t stream, int group_imgs = 0) {
+                             double* sums, cudaStream_t stream, int group_imgs = 0, const float* bias = nullptr) {
   const int halo = d->kh == 3 ? 1 : 0;
   HaloPlan pl = plan_halo(ctx, d->w, d->h, d->n, d->cout);
   int res_stages = 0, res_smem = 0;
@@ -789,6 +791,13 @@ static int conv2d_fprop_halo(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void*
   a.a_stages = res_stages;
   a.b_rows_per_tap = d->cout;   // (K-major copy of a resident CTA pair; unused otherwise)
   a.status = ctx->d_status;
+  if (bias) {
+    a.bias = bias;
+    a.relu = 1;
+    if (res && pl.pair) return launch_halo_res_pair<false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, res_smem, stream);
+    if (res) return launch_halo_res<true, false, false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, res_smem, stream);
+    return launch_halo<true, false, false, true>(ctx, pl.bn, pl.nsub, ta, tb, a, pl.grid, stream);
+  }
   return launch_fprop_halo_stats(ctx, pl, res, res_smem, ta, tb, a, sums, group_imgs, d->n, d->h, d->w, d->cout, y,
                                  d->y_ld, stream);
 }
@@ -816,12 +825,11 @@ int bsl_conv2d_fprop_group_stats(bsl_ctx* ctx, const bsl_conv2d_desc* d, const v
                         as_stream(stream));
 }
 
-int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
-                     void* stream) {
-  int rc = check_conv(ctx, d, true);
-  if (rc) return rc;
-  if (!x || !w || !y) return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop: null buffer");
-  if (halo_eligible(d->w, d->h)) return conv2d_fprop_halo(ctx, d, x, w, y, nullptr, as_stream(stream));
+// fprop with the plain (bias == nullptr) or the bias + ReLU epilogue; both take the same schedule for a shape.
+static int conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, const float* bias, void* y,
+                        void* stream) {
+  int rc;
+  if (halo_eligible(d->w, d->h)) return conv2d_fprop_halo(ctx, d, x, w, y, nullptr, as_stream(stream), 0, bias);
   int box[4] = {0, 0, 0, 1};
   pick_box(128, d->w, d->h, d->n, &box[0], &box[1], &box[2]);
   const int bn = pick_bn(d->cout);
@@ -839,9 +847,27 @@ int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, cons
   a.ostride[2] = (long long)d->h * d->w * d->y_ld;
   a.n_group = d->cout;
   a.n_total = d->cout;
+  a.bias = bias;
+  a.relu = bias != nullptr;
   a.status = ctx->d_status;
   dim3 grid(a.ntile[0] * a.ntile[1] * a.ntile[2], d->cout / bn, 1);
   return launch_igemm<MODE_PIX_M, true>(ctx, bn, ta, tb, a, grid, as_stream(stream));
+}
+
+int bsl_conv2d_fprop(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, void* y,
+                     void* stream) {
+  int rc = check_conv(ctx, d, true);
+  if (rc) return rc;
+  if (!x || !w || !y) return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop: null buffer");
+  return conv2d_fprop(ctx, d, x, w, nullptr, y, stream);
+}
+
+int bsl_conv2d_fprop_bias_relu(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x, const void* w, const float* bias,
+                               void* y, void* stream) {
+  int rc = check_conv(ctx, d, true);
+  if (rc) return rc;
+  if (!x || !w || !bias || !y) return bsl_fail(ctx, BSL_EINVAL, "conv2d_fprop_bias_relu: null buffer");
+  return conv2d_fprop(ctx, d, x, w, bias, y, stream);
 }
 
 int bsl_conv2d_dgrad(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy, const void* w, void* dx,

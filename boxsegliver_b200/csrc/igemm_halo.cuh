@@ -537,7 +537,13 @@ constexpr int CH_MAX_A_STAGES = 4;
 // the time (`b_full`, tools/gpu_conv_bench.py --waits). Barriers: every TMA load of both CTAs counts its bytes on the
 // EVEN CTA's full barriers (cp.async.bulk.tensor.cta_group::2); the issuer's commits arrive on the empty / accumulator
 // barriers of both CTAs (multicast); the peer's epilogue warps arrive on the even CTA's acc_empty barrier through DSMEM.
-template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool B_RES = false, bool TMA_ST = false, bool PAIR = false>
+//
+// BIAS_RELU (plain epilogue of any schedule, no statistics, no scatter): y = bf16(relu(acc + bias[column])), slim.conv2d
+// without a normaliser. The bias of a warp's columns is staged in shared memory once per column tile, as for SCATTER;
+// with TMA_ST, whose 256-wide tiles leave no room for 8 KB of staged bias beside the rings, each warp stages the 64
+// columns of the chunk it is converting (loaded while the TMEM loads are in flight).
+template <int BN, int NSUB, bool B_MN, bool STATS, bool SCATTER, bool B_RES = false, bool TMA_ST = false, bool PAIR = false,
+          bool BIAS_RELU = false>
 // One CTA per SM: the shared-memory ring takes the SM anyway; with that bound ptxas keeps the epilogue's accumulator
 // values in registers instead of spilling them.
 __global__ void __launch_bounds__(CH_THREADS, 1)
@@ -545,6 +551,9 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                  const __grid_constant__ CUtensorMap tmO, const ConvHaloArgs p) {
   static_assert(!TMA_ST || (!STATS && !SCATTER && !B_RES), "TMA-store epilogue: plain streamed-filter variant only");
   static_assert(!PAIR || !SCATTER, "CTA pairs: no scatter epilogue");
+  static_assert(!BIAS_RELU || (!STATS && !SCATTER), "bias + ReLU epilogue: plain stores only");
+  constexpr bool EPI_BIAS = SCATTER || BIAS_RELU;
+  constexpr bool TILE_BIAS = SCATTER || (BIAS_RELU && !TMA_ST);   // bias staged per column tile (else per 64-column chunk)
   static_assert(!PAIR || !B_MN || BN >= 128, "CTA pairs: an MN-major filter splits in 64-column blocks");
   using Cfg = ConvHaloCfg<BN, NSUB, TMA_ST, PAIR>;
   constexpr int ACC_BUFS = Cfg::ACC_BUFS;
@@ -559,7 +568,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   __shared__ uint32_t tmem_slot;
   __shared__ int dead;
   __shared__ float s_stats[STATS ? CH_EPI_WARPS * 2 * BN : 1];
-  __shared__ __align__(16) float s_bias[SCATTER ? CH_EPI_WARPS * 256 : 1];   // per epilogue warp: bias of its columns
+  __shared__ __align__(16) float s_bias[TILE_BIAS ? CH_EPI_WARPS * 256 : (EPI_BIAS ? CH_EPI_WARPS * 64 : 1)];   // per epilogue warp: bias of its columns
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -890,7 +899,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     uint32_t pacc = 0;
     int bias_n0 = -1;
     uint32_t gphase = 0;
-    float* sb = s_bias + (SCATTER ? e * 256 : 0);
+    float* sb = s_bias + (TILE_BIAS ? e * 256 : (EPI_BIAS ? e * 64 : 0));
     // instance statistics: this warp's sums of statistics group `g` -> stats_part[g][slot * 4 + q][2][n_total]
     int cur_grp = -1, last_n0 = 0;
     auto flush_group = [&](int g, int n0) {
@@ -924,7 +933,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       const int n0 = (u % p.n_ntiles) * BN;
       int nsub = p.n_sub_total - pu * NSUB;
       nsub = nsub > NSUB ? NSUB : nsub;
-      if (SCATTER && p.bias != nullptr && n0 != bias_n0) {
+      if (TILE_BIAS && p.bias != nullptr && n0 != bias_n0) {
         // (re)stage the bias of this warp's columns: 32 scalar global loads per chunk in the store loop left the
         // epilogue waiting on the long scoreboard (ncu: 4.7 stalled warps per issue, tensor pipe 11 % active)
         __syncwarp();
@@ -950,9 +959,29 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 #pragma unroll 1
         for (int c = c_begin; c < c_begin + COLS; c += 64) {
           uint32_t v0[32], v1[32], pk[32];
+          float bl0 = 0.f, bl1 = 0.f;
+          if (BIAS_RELU) {
+            bl0 = __ldg(p.bias + n0 + c + lane);
+            bl1 = __ldg(p.bias + n0 + c + 32 + lane);
+          }
           tmem_ld_32x32(trow + c, v0);
           tmem_ld_32x32(trow + c + 32, v1);
           tmem_ld_wait();
+          if (BIAS_RELU) {
+            // (the previous chunk's reads of sb ended before the group barriers below)
+            sb[lane] = bl0;
+            sb[32 + lane] = bl1;
+            __syncwarp();
+            const float2* bb = reinterpret_cast<const float2*>(sb);
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const float2 b0 = bb[i], b1 = bb[16 + i];
+              v0[2 * i] = __float_as_uint(fmaxf(__uint_as_float(v0[2 * i]) + b0.x, 0.f));
+              v0[2 * i + 1] = __float_as_uint(fmaxf(__uint_as_float(v0[2 * i + 1]) + b0.y, 0.f));
+              v1[2 * i] = __float_as_uint(fmaxf(__uint_as_float(v1[2 * i]) + b1.x, 0.f));
+              v1[2 * i + 1] = __float_as_uint(fmaxf(__uint_as_float(v1[2 * i + 1]) + b1.y, 0.f));
+            }
+          }
 #pragma unroll
           for (int i = 0; i < 16; ++i) {
             __nv_bfloat162 h0 = __floats2bfloat162_rn(__uint_as_float(v0[2 * i]), __uint_as_float(v0[2 * i + 1]));
@@ -1013,8 +1042,9 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 bias = p.bias ? sb + (c - c_begin) + 32 * hc : nullptr;
               } else {
                 o = obase + col;
+                if (BIAS_RELU) bias = sb + (c - c_begin) + 32 * hc;
               }
-              if (inside) ch_store_chunk<SCATTER>(hc ? v1 : v0, o, bias, p.relu, packed);
+              if (inside) ch_store_chunk<EPI_BIAS>(hc ? v1 : v0, o, bias, BIAS_RELU ? 1 : p.relu, packed);
             }
           }
         }

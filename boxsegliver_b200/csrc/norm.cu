@@ -799,6 +799,38 @@ __global__ void maxpool_bwd_add_kernel(const __nv_bfloat16* __restrict__ act, in
   }
 }
 
+// y[n,i,j,:] = max of the 2x2 window x[n,2i..2i+1,2j..2j+1,:] (--without_norm encoder blocks: the pooled half of what
+// bsl_norm_apply_pool writes), 8 channels per thread; the comparison is the one maxpool_bwd_add_kernel makes.
+__global__ void maxpool2x2_bf16_kernel(const __nv_bfloat16* __restrict__ x, int x_ld, __nv_bfloat16* __restrict__ y, int y_ld,
+                                       int n, int h, int w, int c) {
+  bsl::pdl_wait();
+  const int cg = c / 8, ho = h / 2, wo = w / 2;
+  const long long total = (long long)n * ho * wo * cg;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
+       i += (long long)gridDim.x * blockDim.x) {
+    long long t = i;
+    const int ch0 = (int)(t % cg) * 8; t /= cg;
+    const int xo = (int)(t % wo); t /= wo;
+    const int yo = (int)(t % ho);
+    const int img = (int)(t / ho);
+    uint4 r[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      r[k] = ld16(x + (((long long)img * h + (2 * yo + (k >> 1))) * w + (2 * xo + (k & 1))) * x_ld + ch0);
+    float m[8];
+    unpack8(r[0], m);
+#pragma unroll
+    for (int k = 1; k < 4; ++k) {
+      float v[8];
+      unpack8(r[k], v);
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        if (v[j] > m[j]) m[j] = v[j];
+    }
+    st16(y + (((long long)img * ho + yo) * wo + xo) * y_ld + ch0, pack8(m));
+  }
+}
+
 __global__ void relu_bwd_kernel(const __nv_bfloat16* __restrict__ y, int y_ld, const __nv_bfloat16* __restrict__ dy,
                                 int dy_ld, __nv_bfloat16* __restrict__ out, int o_ld, long long pixels, int c) {
   bsl::pdl_wait();
@@ -1724,6 +1756,22 @@ int bsl_maxpool2x2_bwd_add(bsl_ctx* ctx, int n, int h, int w, int c, const void*
       reinterpret_cast<const __nv_bfloat16*>(dskip), dskip_ld, reinterpret_cast<__nv_bfloat16*>(dact), dact_ld, n, h,
       w, c);
   BSL_LAUNCH_CHECK(ctx, "maxpool_bwd_add_kernel");
+  return BSL_OK;
+}
+
+int bsl_maxpool2x2_bf16(bsl_ctx* ctx, int n, int h, int w, int c, const void* x, int x_ld, void* y, int y_ld,
+                        void* stream) {
+  if (!ctx) return BSL_EINVAL;
+  if (!x || !y) return bsl_fail(ctx, BSL_EINVAL, "maxpool2x2_bf16: null buffer");
+  if (n <= 0 || h <= 0 || w <= 0 || c <= 0) return bsl_fail(ctx, BSL_EINVAL, "maxpool2x2_bf16: non-positive size");
+  if ((h & 1) || (w & 1) || c % 8 || x_ld < c || y_ld < c || x_ld % 8 || y_ld % 8 ||
+      (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15))
+    return bsl_fail(ctx, BSL_EUNSUPPORTED, "maxpool2x2_bf16: h=%d w=%d even, c=%d, x_ld=%d, y_ld=%d multiples of 8 >= c, "
+                    "16-byte aligned buffers", h, w, c, x_ld, y_ld);
+  const long long items = (long long)n * (h / 2) * (w / 2) * (c / 8);
+  bsl_launch(maxpool2x2_bf16_kernel, dim3(ew_grid(ctx, items)), dim3(256), 0, as_stream(stream),
+             reinterpret_cast<const __nv_bfloat16*>(x), x_ld, reinterpret_cast<__nv_bfloat16*>(y), y_ld, n, h, w, c);
+  BSL_LAUNCH_CHECK(ctx, "maxpool2x2_bf16_kernel");
   return BSL_OK;
 }
 

@@ -6,7 +6,8 @@ module does explicitly: it plans every buffer once, then a step is a fixed seque
 on one compute stream (plus a side stream for the gradient all-reduce), replayable as a CUDA graph.
 
 Memory plan (all NHWC, bf16 unless noted):
-  * per conv layer: `y` (pre-norm conv output, kept for backward) and `a` (post norm+ReLU);
+  * per conv layer: `y` (pre-norm conv output, kept for backward) and `a` (post norm+ReLU); --without_norm keeps only
+    `a` = relu(conv + bias), out of the conv epilogue;
   * skip-concat is zero-copy: encoder level i writes `a` into channels [0,C) of cat_i, the
     transposed conv writes into [C,2C) (UNet.py:93 order: skip first, up second);
   * parameters live in flat fp32 arenas W / G / M / V with a bf16 shadow of W for the tensor-core
@@ -54,6 +55,7 @@ class EngineConfig:
     bn_decay: float = 0.999
     bn_eps: float = 1e-3
     in_eps: float = 1e-6
+    without_norm: bool = False         # --without_norm: slim.conv2d(normalizer_fn=None) -> weights + biases, bias + ReLU
     training: bool = True            # allocate backward / optimizer state
     world: int = 1                   # data-parallel replicas (gradient mean over `world`)
 
@@ -126,7 +128,7 @@ class ConvL:
     affine: str = None       # GUNet after_affine: scope of the ChannelWiseAffine variables of this encoder layer
     bn_decay: float = None   # batch-norm moving-average decay of this layer (None: cfg.bn_decay; GUNet encoder: 0.99)
     x: View = None
-    y: View = None           # pre-norm conv output (conv/stem), or output (convT)
+    y: View = None           # pre-norm conv output (conv/stem; None under --without_norm), or output (convT)
     a: View = None           # post-activation
     pooled: View = None
     params: dict = field(default_factory=dict)
@@ -397,6 +399,9 @@ class UNetEngine:
                 plist.append(Param(f"{L.scope}/weights", (3, 3, L.cin, L.cout),
                                    alloc=64 * L.cout if L.kind == "stem" else 0,
                                    dev_shape=(3, 3, L.cin_dev, L.cout) if L.cin_dev else None))
+                if cfg.without_norm:     # no normalizer_fn: slim keeps the conv's biases
+                    plist.append(Param(f"{L.scope}/biases", (L.cout,), region="B" if cfg.bias_decay else "A"))
+                    continue
                 if L.scale:
                     plist.append(Param(f"{L.scope}/{ns}/gamma", (L.cout,), region="B"))
                 if L.center:
@@ -478,7 +483,8 @@ class UNetEngine:
         small = 0  # floats for per-layer normalisation scalars
         for L in self.layers:
             if L.kind in ("stem", "conv"):
-                L.y = View(self._alloc(n * L.h * L.w * L.cout * BF16), n, L.h, L.w, L.cout)
+                if not cfg.without_norm:
+                    L.y = View(self._alloc(n * L.h * L.w * L.cout * BF16), n, L.h, L.w, L.cout)
                 is_enc2 = L.role == "enc2"
                 if is_enc2:
                     cbuf = View(self._alloc(n * L.h * L.w * 2 * L.cout * BF16), n, L.h, L.w, 2 * L.cout)
@@ -498,11 +504,13 @@ class UNetEngine:
                 prev_a = L.pooled if is_enc2 else L.a
                 if is_enc2 and L.pooled.ld != L.cout:
                     prev_a = View(L.pooled.buf, n, L.h // 2, L.w // 2, L.pooled.ld)
+                max_act = max(max_act, L.h * L.w * L.cout)
+                if cfg.without_norm:
+                    continue
                 g = self._norm_groups(L, groups_max)
                 k = 2 + self._guide_channels(L)
                 L.norm = dict(groups=g, off=small, k=k)
                 small += (2 * k + 6) * _align(g * L.cout, 16)  # sums (k x f64), mean, rstd, scale, shift, c1, c2
-                max_act = max(max_act, L.h * L.w * L.cout)
             elif L.kind == "convT":
                 L.x = prev_a
                 L.a = cat[L.level].slice(L.cout, L.cout)   # upper channel half of the concat buffer
@@ -573,7 +581,7 @@ class UNetEngine:
     def _conv_desc(self, L: ConvL):
         k = 1 if L.kind == "logits" else 3
         x_ld = L.x.ld if L.x is not None else L.cin
-        y_ld = L.y.ld if L.y is not None else L.cout
+        y_ld = L.y.ld if L.y is not None else (L.a.ld if L.a is not None else L.cout)   # --without_norm: y is a
         return _lib.Conv2dDesc(self.cfg.batch, L.h, L.w, L.cin_dev or L.cin, L.cout, k, k, x_ld, y_ld)
 
     def _convT_desc(self, L: ConvL):
@@ -716,7 +724,9 @@ class UNetEngine:
         self._head_done = False
         for idx, L in enumerate(self.layers):
             ctx.tag = L.scope
-            if L.kind in ("stem", "conv"):
+            if L.kind in ("stem", "conv") and self.cfg.without_norm:
+                self._forward_bias_relu(L)
+            elif L.kind in ("stem", "conv"):
                 d = self._conv_desc(L)
                 nd = self._norm_desc(L)
                 q = self._norm_ptrs(L)
@@ -770,6 +780,24 @@ class UNetEngine:
                 d = self._conv_desc(L)
                 call("bsl_conv2d_head_fprop", C.byref(d), L.x.p, self._pp(self.W, f"{L.scope}/weights"),
                      self._pp(self.W, f"{L.scope}/biases"), self.logits.p, s)
+
+    def _forward_bias_relu(self, L: ConvL):
+        """--without_norm: a = relu(conv + bias) out of the conv epilogue, then the 2x2 max-pool of an encoder block."""
+        ctx, s = self.ctx, self.stream
+        wbf = self._pp(self.Wbf, f"{L.scope}/weights", BF16)
+        b = self._pp(self.W, f"{L.scope}/biases")
+        if L.kind == "stem":
+            ctx.call("bsl_stem_im2col_ld", C.byref(self._conv_desc(L)), self.images.p, self.stem_col.p,
+                     C.c_int(self.stem_cols), s)
+            d1 = _lib.Conv2dDesc(self.cfg.batch, L.h, L.w, 64, L.cout, 1, 1, self.stem_cols, L.a.ld)
+            self._tc("fprop", self._flops(L), "bsl_conv2d_fprop_bias_relu", C.byref(d1), self.stem_col.p, wbf, b, L.a.p, s)
+        else:
+            self._tc("fprop", self._flops(L), "bsl_conv2d_fprop_bias_relu", C.byref(self._conv_desc(L)), L.x.p, wbf, b,
+                     L.a.p, s)
+        if L.pooled is not None:
+            ctx.call("bsl_maxpool2x2_bf16", C.c_int(self.cfg.batch), C.c_int(L.h), C.c_int(L.w), C.c_int(L.cout), L.a.p,
+                     C.c_int(L.a.ld), L.pooled.p, C.c_int(L.pooled.ld), s)
+            self._after_pool(L, s)
 
     def _modulate(self, L: ConvL, nd, q):
         """Hook between norm_finalize and norm_apply; returns the bsl_guide of the layer (or None)."""
@@ -860,7 +888,7 @@ class UNetEngine:
                 call("bsl_conv2d_head_wgrad", C.byref(d), L.x.p, self.dlogits.p, self._pp(self.G, f"{L.scope}/weights"),
                      self._pp(self.G, f"{L.scope}/biases"), ws)
                 prev = self.layers[idx - 1]
-                if (self._fuse_head_bwd and prev.kind == "conv" and prev.pooled is None
+                if (self._fuse_head_bwd and not cfg.without_norm and prev.kind == "conv" and prev.pooled is None
                         and not self._is_modulated(prev) and prev.a is L.x
                         and ctx.lib.bsl_norm_bwd_head_ok(ctx.h, C.byref(self._norm_desc(prev)), C.c_int(L.cout))):
                     # no Conv2DBackpropInput launch: the two normalisation-backward passes of `prev` recompute it
@@ -878,12 +906,19 @@ class UNetEngine:
                          C.c_int(L.a.ld), cur.p, C.c_int(L.pooled.ld), dc.p, C.c_int(dc.ld), alt.p, C.c_int(L.cout), s)
                     cur, alt = alt, cur
                 dyb = self.dyb[k]
-                nd = self._norm_desc(L)
-                q = self._norm_ptrs(L)
-                self._norm_backward_reduce(L, nd, q, cur)
-                if overlap and self._dy_busy[k] is not None:   # the wgrad that read this buffer two layers ago
-                    call("bsl_stream_wait_event", s, self._dy_busy[k])
-                self._norm_backward_apply(L, nd, q, cur, dyb, s)
+                if cfg.without_norm:
+                    if overlap and self._dy_busy[k] is not None:
+                        call("bsl_stream_wait_event", s, self._dy_busy[k])
+                    # ReluGrad into dY and BiasAddGrad from the same pass
+                    call("bsl_relu_bwd_bias", C.c_longlong(L.a.pixels), C.c_int(L.cout), L.a.p, C.c_int(L.a.ld), cur.p,
+                         C.c_int(L.cout), dyb.p, C.c_int(L.cout), self._pp(self.G, f"{L.scope}/biases"), s)
+                else:
+                    nd = self._norm_desc(L)
+                    q = self._norm_ptrs(L)
+                    self._norm_backward_reduce(L, nd, q, cur)
+                    if overlap and self._dy_busy[k] is not None:   # the wgrad that read this buffer two layers ago
+                        call("bsl_stream_wait_event", s, self._dy_busy[k])
+                    self._norm_backward_apply(L, nd, q, cur, dyb, s)
                 # dyb = dY (gradient w.r.t. the conv output), dense with ld = cout
                 d = self._conv_desc(L)
                 d.y_ld = L.cout
@@ -957,7 +992,7 @@ class UNetEngine:
     def train_step(self, lr: float, with_metrics: bool = False):
         """One `sess.run(train_op)` on device-resident inputs (/root/reference/core/estimator.py:756-757)."""
         self.forward(True)
-        if self.cfg.normalizer == "batch_norm":
+        if self.cfg.normalizer == "batch_norm" and not self.cfg.without_norm:
             self._allreduce_moving_stats()
         if with_metrics:
             self.predict_outputs(True)

@@ -56,7 +56,6 @@ class GUNetConfig(EngineConfig):
     dropout_seed: int = 0
     use_se: bool = False
     fix: bool = False
-    without_norm: bool = False
     dropout: float = None
     img_grad: bool = False                         # --img_grad: concat(images, dy, dx) of tf.image.image_gradients as input
 

@@ -43,8 +43,6 @@ class UNet(BaseNet):
     def _build_network(self, *args, **kwargs):
         if getattr(self.args, "img_grad", False):
             raise NotImplementedError("--img_grad (tf.image.image_gradients inputs) is outside the accelerated path")
-        if getattr(self.args, "without_norm", False):
-            raise NotImplementedError("--without_norm is outside the accelerated path")
         if self.ctx is None:
             from ..device import Context
             self.ctx = Context(0)
@@ -60,7 +58,8 @@ class UNet(BaseNet):
             loss_numeric_w=tuple(getattr(self.args, "loss_numeric_w", None) or ()),
             loss_proportion_decay=getattr(self.args, "loss_proportion_decay", 1000.0),
             **engine_optimizer_kwargs(self.args), weight_init=self._get_initializer(),
-            training=self.mode == ModeKeys.TRAIN, world=getattr(self, "world", 1))
+            training=self.mode == ModeKeys.TRAIN, world=getattr(self, "world", 1),
+            without_norm=bool(getattr(self.args, "without_norm", False)))
         if self.engine is None or self.engine.cfg != cfg:
             if self.engine is not None:
                 self.engine.close()

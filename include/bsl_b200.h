@@ -124,6 +124,11 @@ int bsl_conv2d_fprop_stats(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x
  * bsl_norm_stats in instance mode; the bf16 outputs are bit-identical. */
 int bsl_conv2d_fprop_group_stats(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x_bf16, const void* w_bf16,
                                  void* y_bf16, int imgs_per_group, double* sums, void* stream);
+/* slim.conv2d with normalizer_fn=None (--without_norm): y = bf16(relu(conv(x, w) + bias[c])), one rounding after the
+ * ReLU. bias is fp32 [cout] (the master copy of the `biases` variable). Same descriptor rules, strides and kernel
+ * schedules as bsl_conv2d_fprop; with a zero bias the output equals relu(bsl_conv2d_fprop) bit for bit. */
+int bsl_conv2d_fprop_bias_relu(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* x_bf16, const void* w_hwio_bf16,
+                               const float* bias_f32, void* y_bf16, void* stream);
 /* dx = dgrad(dy, w); dy has stride y_ld, dx has stride x_ld. */
 int bsl_conv2d_dgrad(bsl_ctx* ctx, const bsl_conv2d_desc* d, const void* dy_bf16,
                      const void* w_hwio_bf16, void* dx_bf16, void* stream);
@@ -425,6 +430,11 @@ int bsl_image_gradients_pack(bsl_ctx* ctx, int n, int h, int w, int c, const flo
 int bsl_maxpool2x2_f32_bf16(bsl_ctx* ctx, int n, int h, int w, int c, const float* x, void* y_bf16, int y_ld,
                             void* stream);
 
+/* slim.max_pool2d(x, 2) of a bf16 activation: y[n,i,j,ch] = max of x[n,2i..2i+1,2j..2j+1,ch]; h, w are the INPUT size
+ * (even), x and y are read / written with channel strides x_ld, y_ld (c, x_ld, y_ld multiples of 8). Exact (no rounding).
+ * The backward pass is bsl_maxpool2x2_bwd_add. */
+int bsl_maxpool2x2_bf16(bsl_ctx* ctx, int n, int h, int w, int c, const void* x_bf16, int x_ld, void* y_bf16, int y_ld,
+                        void* stream);
 /* MaxPoolGrad (first maximum in scan order wins ties) fused with the skip-connection add:
  * dact = dskip (nullable) + unpool(dpool). */
 int bsl_maxpool2x2_bwd_add(bsl_ctx* ctx, int n, int h, int w, int c, const void* act_bf16, int act_ld,
