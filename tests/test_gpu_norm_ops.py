@@ -35,13 +35,18 @@ GM_OFF = 8                      # the layer's slice of the context-MLP output st
 
 class Out:
     """Output operand of `rows` x `width` elements inside a buffer of `rows` x `ld` elements (lanes [off, off + width)
-    of each row) followed by GUARD elements; the whole buffer starts as a canary."""
+    of each row) followed by GUARD elements; the whole buffer starts as a canary, or the operand as `init` (values of
+    its element size, for kernels that work in place)."""
 
-    def __init__(self, ctx, rows, width, ld=None, off=0, esize=4):
+    def __init__(self, ctx, rows, width, ld=None, off=0, esize=4, init=None):
         self.rows, self.width, self.ld, self.off, self.esize = rows, width, ld or width, off, esize
         self.bits = _BITS[esize]
         self.total = rows * self.ld + GUARD
-        self.buf = ctx.from_numpy(np.full(self.total, _CANARY[esize], self.bits))
+        host = np.full(self.total, _CANARY[esize], self.bits)
+        if init is not None:
+            host[:rows * self.ld].reshape(rows, self.ld)[:, off:off + width] = \
+                np.asarray(init).view(self.bits).reshape(rows, width)
+        self.buf = ctx.from_numpy(host)
 
     @property
     def p(self):
