@@ -22,46 +22,18 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from .device import Context, DeviceBuffer, f32_to_bf16_bits
-
-F32 = 4
-BF16 = 2
+from .device import Context, DeviceBuffer
+from .engine_base import BF16, F32, EngineBase, Param, TrainConfig, _align
 
 
 @dataclass
-class EngineConfig:
-    batch: int
+class EngineConfig(TrainConfig):
     height: int = 256
     width: int = 256
     channel: int = 3
-    classes: tuple = ("Background", "Liver", "Tumor")
     init_channels: int = 64
     num_down_samples: int = 4
-    normalizer: str = "batch_norm"
-    weight_decay_rate: float = 1e-5
-    bias_decay: bool = False
-    loss_type: str = "xentropy"
-    loss_weight_type: str = "none"
-    loss_numeric_w: tuple = ()
-    loss_proportion_decay: float = 1000.0
-    optimizer: str = "adam"            # adam | momentum | adamw (core/solver.py:204-219)
-    adam_beta1: float = 0.9            # reference defaults {"beta1": 0.9, "beta2": 0.99} (solver.py:206)
-    adam_beta2: float = 0.99
-    adam_eps: float = 1e-8
-    momentum: float = 0.9              # solver.py:209
-    use_nesterov: bool = False
-    adamw_weight_decay: float = None   # AdamW decoupled decay; None -> weight_decay_rate (solver.py:212)
-    weight_init: str = "xavier"        # xavier | trunc_norm (base.py:137-151)
-    bn_decay: float = 0.999
-    bn_eps: float = 1e-3
-    in_eps: float = 1e-6
     without_norm: bool = False         # --without_norm: slim.conv2d(normalizer_fn=None) -> weights + biases, bias + ReLU
-    training: bool = True            # allocate backward / optimizer state
-    world: int = 1                   # data-parallel replicas (gradient mean over `world`)
-
-    @property
-    def num_classes(self):
-        return len(self.classes)
 
 
 class View:
@@ -86,31 +58,6 @@ class View:
 
 
 @dataclass
-class Param:
-    name: str
-    shape: tuple
-    offset: int = 0          # element offset in the arena
-    size: int = 0
-    alloc: int = 0           # elements reserved in the arena (>= size; the stem filter is padded to 64 x 64)
-    region: str = "A"        # "A" regularised, "B" not, "S" moving statistics (not trained)
-    dev_shape: tuple = None  # stored shape when the input-channel axis is zero-padded to a 64-channel block (else `shape`)
-
-    def to_dev(self, a: np.ndarray) -> np.ndarray:
-        """TF-shaped variable -> flat stored layout (zero rows for the padded input channels)."""
-        if self.dev_shape is None:
-            return a.ravel()
-        out = np.zeros(self.dev_shape, np.float32)
-        out[:, :, :self.shape[2], :] = a
-        return out.ravel()
-
-    def from_dev(self, flat: np.ndarray) -> np.ndarray:
-        a = flat[self.offset:self.offset + self.size]
-        if self.dev_shape is None:
-            return a.reshape(self.shape).copy()
-        return a.reshape(self.dev_shape)[:, :, :self.shape[2], :].copy()
-
-
-@dataclass
 class ConvL:
     kind: str                # "stem" | "conv" | "convT" | "logits"
     scope: str
@@ -119,7 +66,6 @@ class ConvL:
     h: int
     w: int                   # INPUT spatial size
     level: int
-    cin_dev: int = 0         # stored input channels when cin is not a multiple of 64 (UNetInter --mid_cat: 66 -> 128); 0 = cin
     role: str = ""           # enc1 | enc2 (pooled afterwards) | bridge1 | bridge2 | dec1 (reads the concat) | dec2
     center: bool = True      # normaliser has beta / gamma (GUNet's modulated blocks take them from the YAML)
     scale: bool = True
@@ -135,53 +81,10 @@ class ConvL:
     norm: dict = field(default_factory=dict)
 
 
-def _align(n, a=64):
-    return (n + a - 1) // a * a
-
-
-def truncated_normal(rng, shape, stddev: float, mean: float = 0.0) -> np.ndarray:
-    """tf.truncated_normal semantics: N(mean, stddev) samples, values beyond 2 stddev are dropped and re-drawn."""
-    out = rng.standard_normal(shape)
-    bad = np.abs(out) > 2.0
-    while bad.any():
-        out[bad] = rng.standard_normal(int(bad.sum()))
-        bad = np.abs(out) > 2.0
-    return (mean + stddev * out).astype(np.float32)
-
-
-OPTIMIZERS = ("adam", "momentum", "adamw")
-
-
-def enqueue_optimizer(eng, lr: float):
-    """One fused update over the flat arenas of `eng` (2-D and 3-D engines share the layout: region A = L2-regularised
-    [0, n_reg), region B = the rest). Hyper-parameters come from the config (core/solver.py:86-97,204-219)."""
-    ctx, s, cfg = eng.ctx, eng.stream, eng.cfg
-    l2 = cfg.weight_decay_rate if cfg.weight_decay_rate > 0 else 0.0
-    regions = [(0, eng.n_reg, l2, eng.sumsq.p), (eng.n_reg, eng.n_train - eng.n_reg, 0.0, None)]
-    if cfg.optimizer not in OPTIMIZERS:
-        raise ValueError("Not supported optimizer: " + cfg.optimizer)
-    decay = 0.0
-    if cfg.optimizer == "adamw":       # DecoupledWeightDecayExtension decays EVERY variable (decay_var_list=None)
-        decay = cfg.weight_decay_rate if cfg.adamw_weight_decay is None else cfg.adamw_weight_decay
-    for off, n, rate, sq in regions:
-        if n <= 0:
-            continue
-        w = C.c_void_p(eng.W.ptr + off * F32)
-        g = C.c_void_p(eng.G.ptr + off * F32)
-        m = C.c_void_p(eng.M.ptr + off * F32)
-        wb = C.c_void_p(eng.Wbf.ptr + off * BF16)
-        if cfg.optimizer in ("adam", "adamw"):
-            v = C.c_void_p(eng.V.ptr + off * F32)
-            d = _lib.AdamDesc(lr, cfg.adam_beta1, cfg.adam_beta2, cfg.adam_eps, rate, 1.0, eng.step_count, decay)
-            ctx.call("bsl_adam_step", C.byref(d), w, g, m, v, wb, C.c_size_t(n), sq, s)
-        else:
-            ctx.call("bsl_momentum_step", C.c_float(lr), C.c_float(cfg.momentum), C.c_int(int(cfg.use_nesterov)),
-                     C.c_float(rate), C.c_float(1.0), w, g, m, wb, C.c_size_t(n), sq, s)
-
-
-class UNetEngine:
+class UNetEngine(EngineBase):
     def __init__(self, ctx: Context, cfg: EngineConfig):
         self.ctx, self.cfg = ctx, cfg
+        self.pixels_per_sample = cfg.height * cfg.width
         if 9 * cfg.channel > 64:
             raise ValueError("im_channel must be <= 7 (the stem's im2col row holds 9 * channels <= 64 columns)")
         if cfg.init_channels % 64:
@@ -189,31 +92,16 @@ class UNetEngine:
         ds = 2 ** cfg.num_down_samples
         if cfg.height % ds or cfg.width % ds:
             raise ValueError(f"height/width must be multiples of {ds}")
-        if not self._loss_terms():
-            raise ValueError("Not supported loss_type: {}".format(cfg.loss_type))  # UNet.py:132
-        if cfg.loss_weight_type not in ("none", "numerical", "proportion"):
-            raise ValueError("Not supported weight type: " + cfg.loss_weight_type)
-        if cfg.loss_weight_type == "numerical" and len(cfg.loss_numeric_w) != cfg.num_classes:
-            raise KeyError("w_type `numerical` need keyword argument `numeric_w` (one value per class)")
-        if cfg.optimizer not in OPTIMIZERS:
-            raise ValueError("Not supported optimizer: " + cfg.optimizer)       # solver.py:217
-        if cfg.weight_init not in ("xavier", "trunc_norm"):
-            raise ValueError("Not supported weight initializer: " + cfg.weight_init)   # base.py:147
-        self.step_count = 0
-        self._bufs = []
+        self._check_train_config()
+        self._init_plumbing()
         self._skip_exchange = False   # bench.py's data-parallel check runs one backward without the gradient exchange
         self._plan_params()
         self._plan_activations()
-        self.stream = ctx.stream
         self.comm_stream = None
         self._graph = None
         self._grad_stream = self.stream
         self._overlap_wgrad = cfg.training
-        self._ev_ring, self._ev_ring_i = [ctx.new_event() for _ in range(160)], 0
-        if cfg.training:
-            self.wg_stream = ctx.new_stream()
-            self._dy_events = [ctx.new_event(), ctx.new_event()]
-            self._dy_busy = [None, None]
+        self._dy_busy = [None, None]
         # logits out of the last normalised layer's apply pass (bsl_norm_apply_head) instead of a 1x1 conv over the stored
         # activation; bit-identical (tests/test_gpu_unet.py compares both ways)
         self._fuse_head = True
@@ -229,12 +117,6 @@ class UNetEngine:
         self._timed = []          # (name, flops, ev0, ev1) in launch order for the current step(s)
         self._ev_pool = getattr(self, "_ev_pool", [])
         self._ev_next = 0
-
-    def _next_event(self):
-        """Round-robin pool for fork / join events (a step records far fewer than the ring holds)."""
-        e = self._ev_ring[self._ev_ring_i]
-        self._ev_ring_i = (self._ev_ring_i + 1) % len(self._ev_ring)
-        return e
 
     def _ev(self):
         if self._ev_next == len(self._ev_pool):
@@ -287,7 +169,6 @@ class UNetEngine:
         self.comm_stream = self.ctx.new_stream()
         self._ev_ready = [self.ctx.new_event() for _ in range(16)]
         self._ev_done = self.ctx.new_event()
-        self._ev_stats = self.ctx.new_event()
         self._bucket_at = {}          # scope of the layer that closes a bucket -> (offset, count)
         # parameters outside the conv trunk (GUNet guide convs) sit after the last layer in region A and get their
         # gradients late in backward: they travel with the tail
@@ -341,24 +222,12 @@ class UNetEngine:
         self._bucket_i = 0
 
     def _allreduce_moving_stats(self):
-        # MirroredStrategy aggregates the moving-average updates with MEAN across replicas
-        # (/root/reference/core/estimator.py:570-613); batch statistics themselves stay per replica. Nothing reads the
-        # moving statistics before the next step's forward, so the exchange rides the side stream (ahead of the
-        # gradient buckets) and is ordered before the optimizer by the same join as the gradients.
-        if self.cfg.world > 1 and self.n_stats > 0 and not self._skip_exchange:
-            st = self.comm_stream if self.comm_stream is not None else self.stream
-            if st is not self.stream:
-                self.ctx.record(self._ev_stats, self.stream)
-                self.ctx.call("bsl_stream_wait_event", st, self._ev_stats)
-            self.ctx.call("bsl_allreduce_sum_f32", self.S.p, C.c_size_t(self.n_stats), st)
-            self.ctx.call("bsl_scale_f32", self.S.p, C.c_size_t(self.n_stats), C.c_float(1.0 / self.cfg.world), st)
+        # Nothing reads the moving statistics before the next step's forward, so the exchange rides the side stream
+        # (ahead of the gradient buckets) and is ordered before the optimizer by the same join as the gradients.
+        if not self._skip_exchange:
+            super()._allreduce_moving_stats(self.comm_stream)
 
     # ------------------------------------------------------------------ planning
-    def _alloc(self, nbytes) -> DeviceBuffer:
-        b = self.ctx.alloc(max(int(nbytes), 16))
-        self._bufs.append(b)
-        return b
-
     def _layer_specs(self):
         cfg = self.cfg
         specs = []
@@ -396,9 +265,11 @@ class UNetEngine:
         plist = []
         for L in self.layers:
             if L.kind in ("stem", "conv"):
-                plist.append(Param(f"{L.scope}/weights", (3, 3, L.cin, L.cout),
-                                   alloc=64 * L.cout if L.kind == "stem" else 0,
-                                   dev_shape=(3, 3, L.cin_dev, L.cout) if L.cin_dev else None))
+                # the convs reduce over whole 64-channel blocks: a conv's input channels beyond cin (UNetInter --mid_cat
+                # 66 -> 128, GUNet --img_grad 9 -> 64) are stored as zero rows; the im2col stem reserves 64 rows instead
+                cin = L.cin if L.kind == "stem" else _align(L.cin, 64)
+                plist.append(Param(f"{L.scope}/weights", (3, 3, L.cin, L.cout), (3, 3, cin, L.cout),
+                                   (slice(None), slice(None), slice(L.cin)), alloc=64 * L.cout if L.kind == "stem" else 0))
                 if cfg.without_norm:     # no normalizer_fn: slim keeps the conv's biases
                     plist.append(Param(f"{L.scope}/biases", (L.cout,), region="B" if cfg.bias_decay else "A"))
                     continue
@@ -415,33 +286,7 @@ class UNetEngine:
             else:
                 plist.append(Param(f"{L.scope}/weights", (1, 1, L.cin, L.cout)))
                 plist.append(Param(f"{L.scope}/biases", (L.cout,), region="B" if cfg.bias_decay else "A"))
-        plist += self._extra_params()
-        off = 0
-        for region in ("A", "B"):
-            for p in plist:
-                if p.region == region:
-                    p.size = int(np.prod(p.dev_shape or p.shape))
-                    p.offset = off
-                    off += _align(max(p.size, p.alloc))
-            if region == "A":
-                self.n_reg = off
-        self.n_train = off
-        soff = 0
-        for p in plist:
-            if p.region == "S":
-                p.size = int(np.prod(p.shape))
-                p.offset = soff
-                soff += _align(p.size)
-        self.n_stats = soff
-        self.params = {p.name: p for p in plist}
-        self.W = self._alloc(self.n_train * F32)
-        self.Wbf = self._alloc(self.n_train * BF16)
-        self.S = self._alloc(max(self.n_stats, 1) * F32)
-        if cfg.training:
-            self.G = self._alloc(self.n_train * F32).zero()
-            self.M = self._alloc(self.n_train * F32).zero()
-            self.V = self._alloc(self.n_train * F32).zero() if cfg.optimizer in ("adam", "adamw") else None
-        self.sumsq = self._alloc(16)
+        self._layout(plist + self._extra_params())
 
     def _extra_params(self):
         """Parameters outside the conv trunk (GUNet: context MLP, guide convs)."""
@@ -510,7 +355,7 @@ class UNetEngine:
                 g = self._norm_groups(L, groups_max)
                 k = 2 + self._guide_channels(L)
                 L.norm = dict(groups=g, off=small, k=k)
-                small += (2 * k + 6) * _align(g * L.cout, 16)  # sums (k x f64), mean, rstd, scale, shift, c1, c2
+                small += self._norm_scalar_floats(g * L.cout, k)
             elif L.kind == "convT":
                 L.x = prev_a
                 L.a = cat[L.level].slice(L.cout, L.cout)   # upper channel half of the concat buffer
@@ -582,7 +427,8 @@ class UNetEngine:
         k = 1 if L.kind == "logits" else 3
         x_ld = L.x.ld if L.x is not None else L.cin
         y_ld = L.y.ld if L.y is not None else (L.a.ld if L.a is not None else L.cout)   # --without_norm: y is a
-        return _lib.Conv2dDesc(self.cfg.batch, L.h, L.w, L.cin_dev or L.cin, L.cout, k, k, x_ld, y_ld)
+        cin = self.params[f"{L.scope}/weights"].stored[2]       # zero-padded input channels
+        return _lib.Conv2dDesc(self.cfg.batch, L.h, L.w, cin, L.cout, k, k, x_ld, y_ld)
 
     def _convT_desc(self, L: ConvL):
         return _lib.ConvT2dDesc(self.cfg.batch, L.h, L.w, L.cin, L.cout, L.x.ld, L.a.ld, 1)
@@ -594,48 +440,10 @@ class UNetEngine:
                              cfg.bn_eps if bn else cfg.in_eps, L.bn_decay if L.bn_decay is not None else cfg.bn_decay, 1,
                              int(L.center), int(L.scale))
 
-    def _loss_desc(self):
-        cfg = self.cfg
-        wt = {"none": 0, "numerical": 1, "proportion": 2}[cfg.loss_weight_type]
-        nw = (C.c_float * 8)(*([float(x) for x in cfg.loss_numeric_w] + [0.0] * (8 - len(cfg.loss_numeric_w))))
-        return _lib.LossDesc(cfg.batch, cfg.height * cfg.width, cfg.num_classes, wt, nw,
-                             float(cfg.loss_proportion_decay), 1.0 / cfg.world)
-
     def _norm_ptrs(self, L: ConvL):
-        """sums (f64 x 2), mean, rstd, scale, shift, c1, c2 carved from the small-scalar arena."""
-        g = L.norm["groups"]
-        n = _align(g * L.cout, 16)
-        base = self.small.ptr + L.norm["off"] * F32
-        k2 = 2 * L.norm["k"]
-        names = ["mean", "rstd", "scale", "shift", "c1", "c2"]
-        out = {nm: C.c_void_p(base + (k2 + i) * n * F32) for i, nm in enumerate(names)}
-        out["sums"] = C.c_void_p(base)
-        return out
+        return self._norm_scalars(self.small.ptr + L.norm["off"] * F32, L.norm["groups"] * L.cout, L.norm["k"])
 
-    # ------------------------------------------------------------------ weights
-    def set_weights(self, weights: dict):
-        """Load a {tf variable name: numpy array} map (TF layouts: HWIO, [k,k,Cout,Cin], vectors)."""
-        hostW = np.zeros(self.n_train, np.float32)
-        hostS = np.zeros(max(self.n_stats, 1), np.float32)
-        for name, p in self.params.items():
-            if name not in weights:
-                raise KeyError(f"missing variable {name}")
-            a = np.asarray(weights[name], np.float32)
-            if tuple(a.shape) != tuple(p.shape):
-                raise ValueError(f"{name}: shape {a.shape} != {p.shape}")
-            (hostS if p.region == "S" else hostW)[p.offset:p.offset + p.size] = p.to_dev(a)
-        self.W.upload(hostW)
-        self.Wbf.upload(f32_to_bf16_bits(hostW))
-        self.S.upload(hostS)
-
-    def get_weights(self) -> dict:
-        hostW = self.W.download(np.float32, (self.n_train,))
-        hostS = self.S.download(np.float32, (max(self.n_stats, 1),))
-        out = {}
-        for name, p in self.params.items():
-            out[name] = p.from_dev(hostS if p.region == "S" else hostW)
-        return out
-
+    # ------------------------------------------------------------------ stored activations
     def get_stored_forward(self) -> dict:
         """{scope: {"y": pre-norm conv output, "a": activation}} as fp32 numpy (what backward will read)."""
         out = {}
@@ -650,63 +458,6 @@ class UNetEngine:
                 d[key] = full[..., v.c0:v.c0 + v.c].copy()
             out[L.scope] = d
         return out
-
-    def get_grads(self) -> dict:
-        hostG = self.G.download(np.float32, (self.n_train,))
-        return {name: p.from_dev(hostG) for name, p in self.params.items() if p.region != "S"}
-
-    def get_slots(self) -> dict:
-        """Optimizer slots in TF variable shapes: {variable name: (m, v)} for Adam / AdamW, {name: (acc,)} for Momentum."""
-        m = self.M.download(np.float32, (self.n_train,))
-        v = self.V.download(np.float32, (self.n_train,)) if self.V is not None else None
-        out = {}
-        for name, p in self.params.items():
-            if p.region == "S":
-                continue
-            out[name] = tuple(p.from_dev(a) for a in ((m, v) if v is not None else (m,)))
-        return out
-
-    def set_slots(self, slots: dict):
-        """Inverse of get_slots (every trainable variable must be present)."""
-        m = np.zeros(self.n_train, np.float32)
-        v = np.zeros(self.n_train, np.float32) if self.V is not None else None
-        for name, p in self.params.items():
-            if p.region == "S":
-                continue
-            if name not in slots:
-                raise KeyError(f"missing optimizer slots of {name}")
-            for dst, a in zip((m, v), slots[name]):
-                a = np.asarray(a, np.float32)
-                if tuple(a.shape) != tuple(p.shape):
-                    raise ValueError(f"{name}: slot shape {a.shape} != {p.shape}")
-                dst[p.offset:p.offset + p.size] = p.to_dev(a)
-        self.M.upload(m)
-        if v is not None:
-            self.V.upload(v)
-
-    def _draw_weight(self, rng, shp, fan_in, fan_out):
-        """--weight_init (/root/reference/NetworksV2/base.py:137-151): slim.xavier_initializer() (uniform) or
-        tf.truncated_normal_initializer(stddev=0.01) -- normal samples re-drawn while |x| > 2 sigma."""
-        if getattr(self.cfg, "weight_init", "xavier") == "trunc_norm":
-            return truncated_normal(rng, shp, 0.01)
-        lim = np.sqrt(6.0 / (fan_in + fan_out))
-        return rng.uniform(-lim, lim, size=shp).astype(np.float32)
-
-    def init_weights(self, seed: int = 0):
-        """--weight_init weights (seeded numpy stream), zero biases, gamma 1, beta 0, moving 0 / 1."""
-        rng = np.random.default_rng(seed)
-        w = {}
-        for name, p in self.params.items():
-            if name.endswith("/weights"):
-                shp = p.shape
-                rf = shp[0] * shp[1]
-                w[name] = self._draw_weight(rng, shp, rf * shp[2], rf * shp[3])
-            elif name.endswith(("gamma", "moving_variance")):
-                w[name] = np.ones(p.shape, np.float32)
-            else:
-                w[name] = np.zeros(p.shape, np.float32)
-        self.set_weights(w)
-        return w
 
     # ------------------------------------------------------------------ inputs
     def set_inputs(self, images: np.ndarray, labels: np.ndarray | None = None, stream=None):
@@ -840,12 +591,6 @@ class UNetEngine:
         self._norm_backward_reduce(L, nd, q, cur)
         self._norm_backward_apply(L, nd, q, cur, oth, self.stream)
 
-    def predict_outputs(self, with_counts: bool):
-        """softmax, `<Cls>Pred` masks, argmax and (optionally) the integer Dice sums, one pass over the logits."""
-        ld = self._loss_desc()
-        self.ctx.call("bsl_softmax_threshold", C.byref(ld), self.logits.p, self.labels.p if with_counts else None,
-                      self.prob.p, self.masks.p, self.argmax.p, self.ilr.p if with_counts else None, self.stream)
-
     # ------------------------------------------------------------------ loss + backward
     def loss_backward(self):
         ctx, s, cfg = self.ctx, self.stream, self.cfg
@@ -875,9 +620,7 @@ class UNetEngine:
         def fork():
             """side stream waits for everything enqueued on the main stream so far"""
             if overlap:
-                ev = self._next_event()
-                ctx.record(ev, s)
-                call("bsl_stream_wait_event", ws, ev)
+                self._stream_wait(ws, s)
 
         for idx in range(len(self.layers) - 1, -1, -1):
             L = self.layers[idx]
@@ -935,7 +678,7 @@ class UNetEngine:
                         dd.x_ld = dc.ld
                         self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad", C.byref(dd), dyb.p, wbf, dc.p, s)
                     else:
-                        dd.x_ld = L.cin_dev or L.cin
+                        dd.x_ld = dd.cin
                         self._tc("dgrad", self._flops(L), "bsl_conv2d_dgrad", C.byref(dd), dyb.p, wbf, cur.p, s)
                 if L.kind == "stem":
                     d1 = _lib.Conv2dDesc(n, L.h, L.w, 64, L.cout, 1, 1, self.stem_cols, L.cout)
@@ -968,26 +711,8 @@ class UNetEngine:
                          self.wgrad_ws.p, wsb, ws, stream=ws)
                 self._after_grad(L)
         if overlap:     # join: everything downstream (optimizer, host reads of G) is ordered after the filter gradients
-            ev = self._next_event()
-            ctx.record(ev, ws)
-            call("bsl_stream_wait_event", s, ev)
+            self._stream_wait(s, ws)
             self._dy_busy = [None, None]
-
-    # ------------------------------------------------------------------ optimizer
-    def optimizer_step(self, lr: float):
-        self.step_count += 1
-        enqueue_optimizer(self, lr)
-
-    # ------------------------------------------------------------------ results
-    def read_loss(self):
-        """(data loss, L2 regularisation loss) of the step just run; the only D2H read of a train step."""
-        data = float(self.loss_dev.download(np.float32, (len(self._loss_terms()),)).sum())
-        sq = self.sumsq.download(np.float64, (1,))[0]
-        return float(data), float(self.cfg.weight_decay_rate * 0.5 * sq) if self.cfg.weight_decay_rate > 0 else 0.0
-
-    def read_counts(self):
-        k = self.cfg.num_classes - 1
-        return self.ilr.download(np.uint32, (self.cfg.batch, k, 3))
 
     def train_step(self, lr: float, with_metrics: bool = False):
         """One `sess.run(train_op)` on device-resident inputs (/root/reference/core/estimator.py:756-757)."""
@@ -1088,8 +813,3 @@ class UNetEngine:
     def h2d_bytes_per_step(self):
         cfg = self.cfg
         return cfg.batch * cfg.height * cfg.width * (cfg.channel * 4 + 4)
-
-    def close(self):
-        for b in self._bufs:
-            b.free()
-        self._bufs = []

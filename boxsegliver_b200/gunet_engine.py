@@ -107,8 +107,6 @@ class GUNetEngine(UNetEngine):
                 L = ConvL(kind, f"{self.prefix}/Encode/down_conv{i + 1}/mod_conv{j}/Conv", cin, c, h, w, i, role=role,
                           center=(cfg.norm_with_center and not aa) if mod else True,
                           scale=(cfg.norm_with_scale and not aa) if mod else True)
-                if cin % 64 and kind == "conv":      # UNetInter --mid_cat: 64 + guide_channel inputs, stored as 128 lanes
-                    L.cin_dev = _align(cin, 64)
                 if aa:
                     L.affine = f"{self.prefix}/Encode/down_conv{i + 1}/mod_conv{j}/ChannelWiseAffine"
                 # batch norm: the encoder arg scope's decay 0.99 reaches GUNet's modulated blocks (the un-modulated ones
@@ -175,8 +173,8 @@ class GUNetEngine(UNetEngine):
     def _first_input(self, L: ConvL):
         """--img_grad: the bf16 tensor [n, h, w, 64] that bsl_image_gradients_pack fills with (images, dy, dx)."""
         cfg = self.cfg
-        self.input_packed = View(self._alloc(cfg.batch * L.h * L.w * L.cin_dev * BF16).zero(), cfg.batch, L.h, L.w,
-                                 L.cin_dev)
+        lanes = self.params[f"{L.scope}/weights"].stored[2]
+        self.input_packed = View(self._alloc(cfg.batch * L.h * L.w * lanes * BF16).zero(), cfg.batch, L.h, L.w, lanes)
         return self.input_packed
 
     def _bn_mod(self, L: ConvL) -> bool:
@@ -235,16 +233,13 @@ class GUNetEngine(UNetEngine):
         self._ones.upload(ones)
         self._zeros = self._alloc(ones.nbytes).zero()
         for L in layers:
-            m = _align(n * L.cout, 16)
-            self.drop[L.scope] = dict(T=self._alloc(n * L.h * L.w * L.cout * BF16), small=self._alloc(10 * m * F32), m=m)
+            self.drop[L.scope] = dict(T=self._alloc(n * L.h * L.w * L.cout * BF16),
+                                      small=self._alloc(self._norm_scalar_floats(n * L.cout) * F32))
         if cfg.training:
             self.drop_grad = self._alloc(n * max(L.h * L.w * L.cout for L in layers) * BF16)
 
     def _drop_ptrs(self, L: ConvL):
-        d = self.drop[L.scope]
-        base, m = d["small"].ptr, d["m"]
-        names = ["sums", "_s1", "_s2", "_s3", "mean", "rstd", "scale", "shift", "c1", "c2"]
-        return {nm: C.c_void_p(base + i * m * F32) for i, nm in enumerate(names)}
+        return self._norm_scalars(self.drop[L.scope]["small"].ptr, self.cfg.batch * L.cout)
 
     def _drop_desc(self, L: ConvL):
         return _lib.DropoutDesc(1.0 - self.cfg.dropout, self.cfg.dropout_seed, (self.step_count + 1) * 16 + 8 + L.level)

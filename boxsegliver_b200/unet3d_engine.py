@@ -40,15 +40,14 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from .device import Context, DeviceBuffer, f32_to_bf16_bits
-from .engine import BF16, F32, OPTIMIZERS, _align, enqueue_optimizer, truncated_normal
+from .device import Context, DeviceBuffer
+from .engine_base import BF16, F32, EngineBase, Param, TrainConfig, _align
 
 CPAD = 64
 
 
 @dataclass
-class UNet3DConfig:
-    batch: int
+class UNet3DConfig(TrainConfig):
     depth: int = 64
     height: int = 128
     width: int = 128
@@ -61,28 +60,8 @@ class UNet3DConfig:
     guide_channel: int = 2
     normalizer: str = "instance_norm"
     weight_decay_rate: float = 3e-5
-    bias_decay: bool = False
-    loss_type: str = "xentropy"
     loss_weight_type: str = "numerical"
     loss_numeric_w: tuple = (1.0, 1.0)
-    loss_proportion_decay: float = 1000.0
-    optimizer: str = "adam"            # adam | momentum | adamw; hyper-parameters as in engine.EngineConfig
-    adam_beta1: float = 0.9
-    adam_beta2: float = 0.99
-    adam_eps: float = 1e-8
-    momentum: float = 0.9
-    use_nesterov: bool = False
-    adamw_weight_decay: float = None
-    weight_init: str = "xavier"
-    in_eps: float = 1e-6
-    bn_eps: float = 1e-3               # slim.batch_norm defaults (BaseNet._get_normalization)
-    bn_decay: float = 0.999
-    training: bool = True
-    world: int = 1
-
-    @property
-    def num_classes(self):
-        return len(self.classes)
 
     @property
     def in_channels(self):
@@ -147,17 +126,6 @@ class Layer3:
     params: dict = field(default_factory=dict)
 
 
-@dataclass
-class Param3:
-    name: str
-    shape: tuple              # TF variable shape
-    pshape: tuple             # stored (padded) shape
-    layer: Layer3 = None
-    offset: int = 0
-    size: int = 0             # stored elements
-    region: str = "A"         # "A" regularised, "B" not, "S" moving statistics (not trained)
-
-
 def _cp(c):
     return _align(c, CPAD)
 
@@ -179,47 +147,28 @@ def _model_config(pools: int):
     return out
 
 
-class UNet3DEngine:
+class UNet3DEngine(EngineBase):
     def __init__(self, ctx: Context, cfg: UNet3DConfig):
         self.ctx, self.cfg = ctx, cfg
+        self.pixels_per_sample = cfg.depth * cfg.height * cfg.width
         if cfg.normalizer not in ("batch_norm", "instance_norm"):
             raise ValueError("Not supported normalization function: " + cfg.normalizer)
         self.bn = cfg.normalizer == "batch_norm"
         self.norm_scope = "BatchNorm" if self.bn else "InstanceNorm"
-        if "xentropy" not in cfg.loss_type:
-            raise ValueError("Not supported loss_type: {}".format(cfg.loss_type))   # UNet3D.py:198-199
-        if cfg.loss_weight_type not in ("none", "numerical", "proportion"):
-            raise ValueError("Not supported weight type: " + cfg.loss_weight_type)
-        if cfg.loss_weight_type == "numerical" and len(cfg.loss_numeric_w) != cfg.num_classes:
-            raise KeyError("w_type `numerical` need keyword argument `numeric_w` (one value per class)")
-        if cfg.optimizer not in OPTIMIZERS:
-            raise ValueError("Not supported optimizer: " + cfg.optimizer)
-        if cfg.weight_init not in ("xavier", "trunc_norm"):
-            raise ValueError("Not supported weight initializer: " + cfg.weight_init)
+        self._check_train_config()
         if 9 * cfg.in_channels > 64:
             raise ValueError("input channels must be <= 7 (the stem's im2col row holds 9 * channels <= 64 columns)")
         ds = 2 ** cfg.num_pool_layers
         if cfg.height % ds or cfg.width % ds or cfg.depth % 2:
             raise ValueError(f"height/width must be multiples of {ds} and depth even")
-        self.step_count = 0
-        self._bufs = []
-        self.stream = ctx.stream
+        self._init_plumbing()
         self._pair = (cfg.init_channels <= 32 and cfg.width % 16 == 0 and cfg.height % 32 == 0
                       and 9 * cfg.in_channels <= 32 and os.environ.get("BSL_UNET3D_PAIR", "1") != "0")
         # filter gradients on a side stream, as in engine.UNetEngine.loss_backward
         self._overlap_wgrad = cfg.training
-        if cfg.training:
-            self.wg_stream = ctx.new_stream()
-            self._dy_events = [ctx.new_event(), ctx.new_event()]
-            self._ev_ring, self._ev_ring_i = [ctx.new_event() for _ in range(96)], 0
         self._plan_layers()
         self._plan_params()
         self._plan_activations()
-
-    def _alloc(self, nbytes) -> DeviceBuffer:
-        b = self.ctx.alloc(max(int(nbytes), 16))
-        self._bufs.append(b)
-        return b
 
     # ------------------------------------------------------------------ planning
     def _plan_layers(self):
@@ -287,49 +236,29 @@ class UNet3DEngine:
         self.layers = layers
 
     def _plan_params(self):
+        """TF-shaped variables inside their padded stored layouts (concat inputs split as [encoder | up] by cin_map)."""
         cfg = self.cfg
         plist = []
+        every = (slice(None),) * 3
         for L in self.layers:
             if L.kind in ("stem", "conv"):
-                ps = (L.cinp, L.coutp) if L.kind == "stem" else L.k + (L.cinp, L.coutp)
-                plist.append(Param3(f"{L.scope}/weights", L.k + (L.cin, L.cout), ps, L))
+                name, shape = f"{L.scope}/weights", L.k + (L.cin, L.cout)
+                if L.kind == "stem":     # im2col rows (kh, kw, cin) of the 1x1 conv over the stem's im2col matrix
+                    plist.append(Param(name, shape, (L.cinp, L.coutp), (slice(int(np.prod(shape[:4]))), slice(L.cout))))
+                else:
+                    plist.append(Param(name, shape, L.k + (L.cinp, L.coutp), every + (L.cin_map, slice(L.cout))))
                 ns = f"{L.scope}/{self.norm_scope}"
-                plist.append(Param3(f"{ns}/gamma", (L.cout,), (L.coutp,), L, region="B"))
-                plist.append(Param3(f"{ns}/beta", (L.cout,), (L.coutp,), L, region="B"))
-                if self.bn:
-                    plist.append(Param3(f"{ns}/moving_mean", (L.cout,), (L.coutp,), L, region="S"))
-                    plist.append(Param3(f"{ns}/moving_variance", (L.cout,), (L.coutp,), L, region="S"))
+                for v, region in (("gamma", "B"), ("beta", "B")) + ((("moving_mean", "S"), ("moving_variance", "S"))
+                                                                     if self.bn else ()):
+                    plist.append(Param(f"{ns}/{v}", (L.cout,), (L.coutp,), (slice(L.cout),), region=region))
             elif L.kind == "convT":
-                plist.append(Param3(f"{L.scope}/weights", L.k + (L.cout, L.cin), L.k + (L.coutp, L.cinp), L))
+                plist.append(Param(f"{L.scope}/weights", L.k + (L.cout, L.cin), L.k + (L.coutp, L.cinp),
+                                   every + (slice(L.cout), slice(L.cin))))
             else:
-                plist.append(Param3(f"{L.scope}/weights", (1, 1, 1, L.cin, L.cout), (L.cinp, L.cout), L))
-                plist.append(Param3(f"{L.scope}/biases", (L.cout,), (L.cout,), L, region="B" if cfg.bias_decay else "A"))
-        off = 0
-        for region in ("A", "B"):
-            for p in plist:
-                if p.region == region:
-                    p.size = int(np.prod(p.pshape))
-                    p.offset = off
-                    off += _align(p.size)
-            if region == "A":
-                self.n_reg = off
-        self.n_train = off
-        soff = 0
-        for p in plist:
-            if p.region == "S":
-                p.size = int(np.prod(p.pshape))
-                p.offset = soff
-                soff += _align(p.size)
-        self.n_stats = soff
-        self.params = {p.name: p for p in plist}
-        self.W = self._alloc(self.n_train * F32)
-        self.Wbf = self._alloc(self.n_train * BF16)
-        self.S = self._alloc(max(self.n_stats, 1) * F32)
-        if cfg.training:
-            self.G = self._alloc(self.n_train * F32).zero()
-            self.M = self._alloc(self.n_train * F32).zero()
-            self.V = self._alloc(self.n_train * F32).zero() if cfg.optimizer in ("adam", "adamw") else None
-        self.sumsq = self._alloc(16)
+                plist.append(Param(f"{L.scope}/weights", (1, 1, 1, L.cin, L.cout), (L.cinp, L.cout),
+                                   (L.cin_map, slice(None))))
+                plist.append(Param(f"{L.scope}/biases", (L.cout,), region="B" if cfg.bias_decay else "A"))
+        self._layout(plist)
         self._plan_super_filters()
 
     # ------------------------------------------------------------------ pixel-pair packing: super filters
@@ -440,7 +369,7 @@ class UNet3DEngine:
                 L.x = cat[L.block.replace("d", "e")] if is_dec1 else prev
                 prev = L.a
                 L.norm_off = small
-                small += 10 * _align(n * L.coutp, 16)
+                small += self._norm_scalar_floats(n * L.coutp)
                 max_act = max(max_act, vox * L.coutp)
                 if L.kind == "conv" and not is_dec1:      # its dgrad writes in-voxels x cinp lanes into a ping-pong buffer
                     max_grad = max(max_grad, int(np.prod(L.dhw)) * L.cinp)
@@ -545,17 +474,10 @@ class UNet3DEngine:
                              cfg.bn_eps if self.bn else cfg.in_eps, cfg.bn_decay if self.bn else 0.0, 1, 1, 1)
 
     def _norm_ptrs(self, L: Layer3):
-        n = _align(self.cfg.batch * L.coutp, 16)
-        base = self.small.ptr + L.norm_off * F32
-        names = ["sums", "_s1", "_s2", "_s3", "mean", "rstd", "scale", "shift", "c1", "c2"]
-        return {nm: C.c_void_p(base + i * n * F32) for i, nm in enumerate(names)}
+        return self._norm_scalars(self.small.ptr + L.norm_off * F32, self.cfg.batch * L.coutp)
 
-    def _loss_desc(self):
-        cfg = self.cfg
-        wt = {"none": 0, "numerical": 1, "proportion": 2}[cfg.loss_weight_type]
-        nw = (C.c_float * 8)(*([float(x) for x in cfg.loss_numeric_w] + [0.0] * (8 - len(cfg.loss_numeric_w))))
-        return _lib.LossDesc(cfg.batch, cfg.depth * cfg.height * cfg.width, cfg.num_classes, wt, nw,
-                             float(cfg.loss_proportion_decay), 1.0 / cfg.world)
+    def _loss_terms(self):
+        return ["xentropy"] if "xentropy" in self.cfg.loss_type else []     # UNet3D.py:198-199
 
     def _flops(self, L: Layer3) -> float:
         n = self.cfg.batch
@@ -567,102 +489,7 @@ class UNet3DEngine:
         bwd = sum(self._flops(L) * (1 if L.kind == "stem" else 2) for L in self.layers)
         return {"fwd": fwd, "bwd": bwd, "total": fwd + bwd}
 
-    # ------------------------------------------------------------------ weights (pack / unpack)
-    def _pack(self, p: Param3, a: np.ndarray) -> np.ndarray:
-        L = p.layer
-        out = np.zeros(p.pshape, np.float32)
-        if p.name.endswith("/weights"):
-            if L.kind == "stem":
-                out[:a.shape[1] * a.shape[2] * a.shape[3], :L.cout] = a.reshape(-1, L.cout)
-            elif L.kind == "conv":
-                out[:, :, :, L.cin_map, :L.cout] = a
-            elif L.kind == "convT":
-                out[:, :, :, :L.cout, :L.cin] = a
-            else:
-                out[L.cin_map, :] = a.reshape(L.cin, L.cout)
-        else:
-            out[:a.shape[0]] = a
-        return out
-
-    def _unpack(self, p: Param3, flat: np.ndarray) -> np.ndarray:
-        L = p.layer
-        a = flat[p.offset:p.offset + p.size].reshape(p.pshape)
-        if p.name.endswith("/weights"):
-            if L.kind == "stem":
-                return a[:int(np.prod(p.shape[:4])), :L.cout].reshape(p.shape).copy()
-            if L.kind == "conv":
-                return a[:, :, :, L.cin_map, :L.cout].copy()
-            if L.kind == "convT":
-                return a[:, :, :, :L.cout, :L.cin].copy()
-            return a[L.cin_map, :].reshape(p.shape).copy()
-        return a[:p.shape[0]].copy()
-
-    def set_weights(self, weights: dict):
-        """Trainable variables and (batch norm) moving statistics, TF-shaped."""
-        host = np.zeros(self.n_train, np.float32)
-        hostS = np.zeros(max(self.n_stats, 1), np.float32)
-        for name, p in self.params.items():
-            if name not in weights:
-                raise KeyError(f"missing variable {name}")
-            a = np.asarray(weights[name], np.float32)
-            if tuple(a.shape) != tuple(p.shape):
-                raise ValueError(f"{name}: shape {a.shape} != {p.shape}")
-            (hostS if p.region == "S" else host)[p.offset:p.offset + p.size] = self._pack(p, a).ravel()
-        self.W.upload(host)
-        self.Wbf.upload(f32_to_bf16_bits(host))
-        self.S.upload(hostS)
-
-    def get_weights(self) -> dict:
-        host = self.W.download(np.float32, (self.n_train,))
-        hostS = self.S.download(np.float32, (max(self.n_stats, 1),))
-        return {name: self._unpack(p, hostS if p.region == "S" else host) for name, p in self.params.items()}
-
-    def get_grads(self) -> dict:
-        host = self.G.download(np.float32, (self.n_train,))
-        return {name: self._unpack(p, host) for name, p in self.params.items() if p.region != "S"}
-
-    def get_slots(self) -> dict:
-        """Optimizer slots in TF variable shapes (un-padded, [encoder | up] channel order): {name: (m, v)} / {name: (acc,)}."""
-        arenas = [self.M.download(np.float32, (self.n_train,))]
-        if self.V is not None:
-            arenas.append(self.V.download(np.float32, (self.n_train,)))
-        return {name: tuple(self._unpack(p, a) for a in arenas) for name, p in self.params.items() if p.region != "S"}
-
-    def set_slots(self, slots: dict):
-        arenas = [np.zeros(self.n_train, np.float32) for _ in range(2 if self.V is not None else 1)]
-        for name, p in self.params.items():
-            if p.region == "S":
-                continue
-            if name not in slots:
-                raise KeyError(f"missing optimizer slots of {name}")
-            for dst, a in zip(arenas, slots[name]):
-                a = np.asarray(a, np.float32)
-                if tuple(a.shape) != tuple(p.shape):
-                    raise ValueError(f"{name}: slot shape {a.shape} != {p.shape}")
-                dst[p.offset:p.offset + p.size] = self._pack(p, a).ravel()
-        self.M.upload(arenas[0])
-        if self.V is not None:
-            self.V.upload(arenas[1])
-
-    def init_weights(self, seed: int = 0):
-        rng = np.random.default_rng(seed)
-        w = {}
-        for name, p in self.params.items():
-            shp = p.shape
-            if name.endswith("/weights"):
-                rf = int(np.prod(shp[:3]))
-                if self.cfg.weight_init == "trunc_norm":        # base.py:138-139
-                    w[name] = truncated_normal(rng, shp, 0.01)
-                else:
-                    lim = np.sqrt(6.0 / (rf * shp[3] + rf * shp[4]))
-                    w[name] = rng.uniform(-lim, lim, size=shp).astype(np.float32)
-            elif name.endswith(("gamma", "moving_variance")):
-                w[name] = np.ones(shp, np.float32)
-            else:
-                w[name] = np.zeros(shp, np.float32)
-        self.set_weights(w)
-        return w
-
+    # ------------------------------------------------------------------ inputs
     def set_inputs(self, images: np.ndarray, labels: np.ndarray | None = None, sp_guide: np.ndarray | None = None):
         cfg = self.cfg
         shp = (cfg.batch, cfg.depth, cfg.height, cfg.width)
@@ -760,11 +587,6 @@ class UNet3DEngine:
                 call("bsl_conv2d_head_fprop", C.byref(dh), L.x.p, self._pp(self.W, f"{L.scope}/weights"),
                      self._pp(self.W, f"{L.scope}/biases"), self.logits.p, s)
 
-    def predict_outputs(self, with_counts: bool):
-        ld = self._loss_desc()
-        self.ctx.call("bsl_softmax_threshold", C.byref(ld), self.logits.p, self.labels.p if with_counts else None,
-                      self.prob.p, self.masks.p, self.argmax.p, self.ilr.p if with_counts else None, self.stream)
-
     # ------------------------------------------------------------------ loss + backward
     def loss_backward(self):
         ctx, s, cfg = self.ctx, self.stream, self.cfg
@@ -784,10 +606,7 @@ class UNet3DEngine:
 
         def fork():
             if overlap:
-                ev = self._ev_ring[self._ev_ring_i]
-                self._ev_ring_i = (self._ev_ring_i + 1) % len(self._ev_ring)
-                ctx.record(ev, s)
-                call("bsl_stream_wait_event", ws, ev)
+                self._stream_wait(ws, s)
 
         for L in reversed(self.layers):
             ctx.tag = L.scope
@@ -883,27 +702,12 @@ class UNet3DEngine:
                 call("bsl_convT2d_bwd_data" if two_d else "bsl_convT3d_bwd_data", C.byref(dd), dup.p, wbf, cur.p, s)
                 cur_ld = L.cinp
         if overlap:
-            ev = self._ev_ring[self._ev_ring_i]
-            self._ev_ring_i = (self._ev_ring_i + 1) % len(self._ev_ring)
-            ctx.record(ev, ws)
-            call("bsl_stream_wait_event", s, ev)
+            self._stream_wait(s, ws)
 
     # ------------------------------------------------------------------ optimizer / step
     def attach_comm(self, rank: int, world: int, unique_id: bytes):
         assert world == self.cfg.world
         self.ctx.attach_comm(rank, world, unique_id)
-
-    def optimizer_step(self, lr: float):
-        self.step_count += 1
-        enqueue_optimizer(self, lr)
-
-    def _allreduce_moving_stats(self):
-        # MirroredStrategy aggregates the moving-average updates with MEAN across replicas
-        # (/root/reference/core/estimator.py:570-613); batch statistics themselves stay per replica (no sync-BN)
-        if self.cfg.world > 1 and self.n_stats > 0:
-            self.ctx.call("bsl_allreduce_sum_f32", self.S.p, C.c_size_t(self.n_stats), self.stream)
-            self.ctx.call("bsl_scale_f32", self.S.p, C.c_size_t(self.n_stats), C.c_float(1.0 / self.cfg.world),
-                          self.stream)
 
     def train_step(self, lr: float, with_metrics: bool = False):
         self.forward(True)
@@ -914,16 +718,3 @@ class UNet3DEngine:
         if self.cfg.world > 1:
             self.ctx.call("bsl_allreduce_sum_f32", self.G.p, C.c_size_t(self.n_train), self.stream)
         self.optimizer_step(lr)
-
-    def read_loss(self):
-        data = self.loss_dev.download(np.float32, (1,))[0]
-        sq = self.sumsq.download(np.float64, (1,))[0]
-        return float(data), float(self.cfg.weight_decay_rate * 0.5 * sq) if self.cfg.weight_decay_rate > 0 else 0.0
-
-    def read_counts(self):
-        return self.ilr.download(np.uint32, (self.cfg.batch, self.cfg.num_classes - 1, 3))
-
-    def close(self):
-        for b in self._bufs:
-            b.free()
-        self._bufs = []

@@ -4,9 +4,6 @@ such a graph by bsl_slim to the engine config and the C-ABI call sequence of eng
 
 Without a normaliser, slim.conv2d keeps its `biases` variable (zeros initializer), adds it and applies ReLU
 (tf.contrib.layers.convolution2d with normalizer_fn=None)."""
-import ctypes as C
-import types
-
 import numpy as np
 import pytest
 import torch
@@ -14,6 +11,7 @@ import torch
 from boxsegliver_b200 import bsl_slim as slim
 from boxsegliver_b200 import synthetic
 from tests import unet_without_norm_ref as R
+from tests.fake_ctx import FakeContext
 from tests import unet_without_norm_torch as T
 
 tf = slim.tf
@@ -142,58 +140,8 @@ def test_variable_inventory_follows_slim(bias_decay):
 
 
 # ------------------------------------------------------------------ bsl_slim lowering, traced without a device
-class _TraceBuf:
-    def __init__(self, ptr, nbytes):
-        self.ptr, self.nbytes = ptr, nbytes
-
-    @property
-    def p(self):
-        return C.c_void_p(self.ptr)
-
-    def at(self, off):
-        return C.c_void_p(self.ptr + off)
-
-    def zero(self, stream=None):
-        return self
-
-    def free(self):
-        pass
-
-
-class _TraceCtx:
-    """Stands in for device.Context: hands out fake addresses and records the C-ABI entry points called."""
-
-    def __init__(self):
-        self.trace = []
-        self._next = 1 << 20
-        self.h = None
-        self.tag = ""
-        self._prof = None
-        self.stream = C.c_void_p(1)
-        self.lib = types.SimpleNamespace(bsl_loss_workspace=lambda *a: 256, bsl_conv2d_wgrad_workspace=lambda *a: 256,
-                                         bsl_convT2d_bwd_filter_workspace=lambda *a: 256)
-
-    def alloc(self, nbytes):
-        b = _TraceBuf(self._next, nbytes)
-        self._next += (int(nbytes) + 255) // 256 * 256
-        return b
-
-    def call(self, name, *args):
-        self.trace.append(name)
-        return 0
-
-    def new_event(self):
-        return C.c_void_p(2)
-
-    def new_stream(self):
-        return C.c_void_p(3)
-
-    def record(self, ev, stream=None):
-        pass
-
-
 def _engine(cls, cfg):
-    return cls(_TraceCtx(), cfg)
+    return cls(FakeContext(), cfg)
 
 
 def build_unet(images, num_classes, norm_fn=None, norm_params=None, plain_scope=None, weight_decay_rate=1e-5,
@@ -244,7 +192,7 @@ def test_lowered_graph_gives_the_engine_config_and_call_sequence(bias_decay):
     with slim.graph_as_default() as g:
         logits = build_unet(slim.placeholder((n, hw, hw, 3)), 3, bias_decay=bias_decay, num_down_samples=depth)
         table, info = slim.lower_to_layer_table(g, logits)
-        geng = slim.lower(g, logits, _TraceCtx(), classes)
+        geng = slim.lower(g, logits, FakeContext(), classes)
     assert info["normalizer"] is None and info["num_down_samples"] == depth
     names = set()
     for L in table:
@@ -307,6 +255,6 @@ def test_plain_conv_without_bias_is_rejected():
 def test_gunet_and_unetinter_engines_still_raise():
     from boxsegliver_b200.gunet_engine import GUNetConfig, GUNetEngine, UNetInterConfig, UNetInterEngine
     with pytest.raises(NotImplementedError, match="without_norm"):
-        GUNetEngine(_TraceCtx(), GUNetConfig(batch=1, height=64, width=64, without_norm=True))
+        GUNetEngine(FakeContext(), GUNetConfig(batch=1, height=64, width=64, without_norm=True))
     with pytest.raises(NotImplementedError, match="without_norm"):
-        UNetInterEngine(_TraceCtx(), UNetInterConfig(batch=1, height=64, width=64, without_norm=True))
+        UNetInterEngine(FakeContext(), UNetInterConfig(batch=1, height=64, width=64, without_norm=True))
